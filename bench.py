@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — det-head images/sec (assign + loss + NMS), BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg1] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic head outputs per GPU:
 CIoU top-9 assignment + the four loss reductions (train chain) and dense decode + class-aware
@@ -27,6 +27,10 @@ Prints ONE JSON line (rank 0):
                          mode) and ``workload_stats`` (positives / candidates / detections per image) describe this arm
 
 ``--impl reference``: only that CPU arm (rank 0), same metric/unit/config.
+
+``--steps K`` is the number of timed steps of ``value`` (after ``--warmup`` untimed ones).  ``--dump-outputs DIR``: the
+StepOutputs of the last of them (rank 0) as ``DIR/<field>.npy``, a few MB at every workload.  The inputs come from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -77,15 +81,23 @@ def parse_args():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-gpu-eager", action="store_true")
-    ap.add_argument("--regions", type=int, default=5,
-                    help="timed regions of --steps steps each; the line reports the median region (SURVEY.md §8d), min/max "
-                         "and per-rank times beside it")
+    ap.add_argument("--regions", type=int, default=1,
+                    help="split the --steps timed steps into this many regions; the line reports the median region's time "
+                         "per step (SURVEY.md §8d), min/max and per-rank times beside it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy "
+                         "(float32, or float64 for the fp64 sums)")
     ap.add_argument("--skip-half-maps", action="store_true", help="do not also time the step on bf16 head outputs")
     ap.add_argument("--skip-mlp", action="store_true", help="do not also time the MLP towers in front of the path (row N4)")
     ap.add_argument("--skip-train-tail", action="store_true", help="do not time the drop-in head's training tail with backward")
     ap.add_argument("--e2e-steps", type=int, default=60)
     ap.add_argument("--e2e-lanes", type=int, default=3, help="end-to-end steps in flight (own stream + buffers each)")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def measured_peaks():
@@ -285,6 +297,20 @@ def bind_rank_to_gpu_numa(local_rank, world):
 
 
 # ----------------------------------------------------------------------------- our arm
+def dump_outputs(directory, out):
+    """One ``<field>.npy`` per field of ``out`` (a StepOutputs): float64 for the fp64 loss sums, float32 for the rest; the
+    integer fields (gt indices, counts, class ids) are exact in float32."""
+    import dataclasses
+
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for f in dataclasses.fields(out):
+        t = getattr(out, f.name).cpu()
+        t = t if t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(directory, f.name + ".npy"), t.numpy())
+
+
 def run_ours(args, w, world, rank, local_rank):
     import torch
     import torch.distributed as dist
@@ -363,8 +389,8 @@ def run_ours(args, w, world, rank, local_rank):
         torch.cuda.synchronize()
 
     def timed_steps(mode, steps, warmup, n_regions, in_sets=None):
-        """Build the lanes for one decode mode, replay `warmup` steps and `n_regions` regions of `steps` steps, return
-        (median region ms, pipes, outs, graphs, timing)."""
+        """Build the lanes for one decode mode, replay `warmup` steps and then `steps` timed steps split into `n_regions`
+        regions, return (median region ms per step, pipes, outs, graphs, timing, outputs of the last timed step)."""
         pipes = attach([DetectionHeadPipeline(levels, W, H, B, C, B * G, dev, TOPK, K, SCORE_THR, IOU_THR, decode_mode=mode)
                         for _ in range(n_lanes)])
         # every (lane, input set) pair owns its outputs: steps in flight on different lanes never share a buffer
@@ -401,6 +427,7 @@ def run_ours(args, w, world, rank, local_rank):
                         g = torch.cuda.CUDAGraph()
                         with torch.cuda.graph(g, stream=lane_streams[ln]):
                             full_step(ln, i)                   # NCCL all-reduce is captured as a graph node
+                        g.replay()                             # a graph's first launch is slower: keep it out of the timing
                         lane_graphs.append(g)
                     graphs.append(lane_graphs)
             torch.cuda.synchronize()
@@ -434,13 +461,16 @@ def run_ours(args, w, world, rank, local_rank):
             run_step(s)
         issue_done()
         drain()
-        # R timed regions of exactly n_steps steps each.  Every region: host barrier + synchronize on both sides (the
-        # contract), and — with the fused exchange — a DEVICE-side barrier enqueued in front of the start event, so that
+        # n_steps timed steps in R regions (sizes differ by at most one).  Every region: host barrier + synchronize on
+        # both sides, and — with the fused exchange — a DEVICE-side barrier enqueued in front of the start event, so that
         # all GPUs enter the region within an NVLink round trip of each other and the host barrier's rank skew stays
-        # outside it.  Reported: the median region of the max-over-ranks times, min / max, and every rank's median.
+        # outside it.  Reported per step: the median region of the max-over-ranks times, min / max, and every
+        # rank's median.
         start_barrier = getattr(pipes[0], "start_barrier", None) if fused else None
+        R = max(1, min(n_regions, n_steps))
+        sizes = [n_steps // R + (r < n_steps % R) for r in range(R)]
         per_region, step_no, host_issue = [], n_warmup, []
-        for _ in range(max(1, n_regions)):
+        for n in sizes:
             barrier()
             if sampler: sampler.mark()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -450,16 +480,16 @@ def run_ours(args, w, world, rank, local_rank):
             for st in lane_streams:                        # the lanes start behind the start event itself (same-box A/B
                 st.wait_event(e0)                          # against fork(): no difference, 40.54 vs 40.56 us at 20 steps)
             h0 = time.perf_counter()
-            for s in range(step_no, step_no + n_steps):
+            for s in range(step_no, step_no + n):
                 run_step(s)
-            host_issue.append((time.perf_counter() - h0) * 1e3 / n_steps)
+            host_issue.append((time.perf_counter() - h0) * 1e3 / n)
             issue_done()
-            step_no += n_steps
+            step_no += n
             drain()
             e1.record(main)
             barrier()
             if sampler: sampler.mark()
-            per_region.append(e0.elapsed_time(e1))
+            per_region.append(e0.elapsed_time(e1) / n)
         mine = torch.tensor(per_region, dtype=torch.float64, device=dev)
         if multi:
             allr = [torch.empty_like(mine) for _ in range(world)]
@@ -469,20 +499,23 @@ def run_ours(args, w, world, rank, local_rank):
             allr = mine.view(1, -1)
         region_max = allr.max(dim=0).values                 # max over ranks, per region
         ms = float(region_max.median().item())
-        timing = {"regions": len(per_region), "steps_per_region": n_steps, "ms_per_step_median": ms / n_steps,
-                  "ms_per_step_min": float(region_max.min().item()) / n_steps,
-                  "ms_per_step_max": float(region_max.max().item()) / n_steps,
-                  "per_rank_ms_per_step_median": [float(v) / n_steps for v in allr.median(dim=1).values.tolist()],
+        timing = {"regions": len(per_region), "steps_per_region": sizes, "ms_per_step_median": ms,
+                  "ms_per_step_min": float(region_max.min().item()),
+                  "ms_per_step_max": float(region_max.max().item()),
+                  "per_rank_ms_per_step_median": allr.median(dim=1).values.tolist(),
                   "start": "device-side barrier over NVLink peer memory" if start_barrier is not None else "host barrier",
                   # host wall time to ENQUEUE one step (rank 0, median region): the step is device-bound while this is
                   # well below ms_per_step
                   "host_issue_ms_per_step": sorted(host_issue)[len(host_issue) // 2]}
-        return ms, pipes, outs, graphs, timing
+        last = step_no - 1
+        return ms, pipes, outs, graphs, timing, outs[last % n_lanes][last % n_sets]
 
-    ms, pipes, outs, graphs, timing = timed_steps(args.decode_mode, args.steps, max(args.warmup, 3), args.regions)
+    ms, pipes, outs, graphs, timing, last_out = timed_steps(args.decode_mode, args.steps, max(args.warmup, 3), args.regions)
     pipe = pipes[0]
-    value = B * world * args.steps / (ms * 1e-3)
+    value = B * world / (ms * 1e-3)
     outs0 = outs[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out)
 
     # ---- sanity of what was timed (not timed): losses finite, detections present
     losses = outs0[0].losses.cpu().tolist()
@@ -508,12 +541,12 @@ def run_ours(args, w, world, rank, local_rank):
     if not args.skip_candidate_first:
         other_mode = "candidate_first" if args.decode_mode == "dense" else "dense"
         o_steps = max(3, min(args.steps, 1000))
-        o_ms, o_pipes, o_outs, _, _ = timed_steps(other_mode, o_steps, max(min(args.warmup, 100), 3), min(args.regions, 3))
+        o_ms, o_pipes, o_outs, _, _, _ = timed_steps(other_mode, o_steps, max(min(args.warmup, 100), 3), min(args.regions, 3))
         same = all(torch.equal(a, b) for a, b in zip(
             (outs0[0].num_instances, outs0[0].scores, outs0[0].classes, outs0[0].boxes, outs0[0].assignment),
             (o_outs[0][0].num_instances, o_outs[0][0].scores, o_outs[0][0].classes, o_outs[0][0].boxes, o_outs[0][0].assignment)))
-        other = {"decode_mode": other_mode, "value": B * world * o_steps / (o_ms * 1e-3), "unit": UNIT, "steps": o_steps,
-                 "ms_per_step": o_ms / o_steps, "outputs_equal_to_timed_mode": bool(same)}
+        other = {"decode_mode": other_mode, "value": B * world / (o_ms * 1e-3), "unit": UNIT, "steps": o_steps,
+                 "ms_per_step": o_ms, "outputs_equal_to_timed_mode": bool(same)}
         del o_pipes, o_outs
 
     def both_e2e(smp, rows):
@@ -638,10 +671,10 @@ def run_ours(args, w, world, rank, local_rank):
     # the raw boxes of the locations that are not candidates (never read); the survey's own figure is reported beside it
     step_bytes_survey = 20 * A + 24 * G + (16 + 4 * C) * P_bar + 4 * A * (C + 5) + 28 * K + 8
     step_bytes_per_image = step_bytes_survey - 16 * (A - cand_mean)
-    step_gbs = step_bytes_per_image * B * args.steps / (ms * 1e-3) / 1e9          # per GPU
+    step_gbs = step_bytes_per_image * B / (ms * 1e-3) / 1e9          # per GPU
     roofline_step = {"bytes_per_image": step_bytes_per_image, "achieved": step_gbs, "peak": peak, "unit": "GB/s",
                      "frac": step_gbs / peak, "per_gpu": True, "bytes_per_image_survey_8d": step_bytes_survey,
-                     "frac_survey_8d_bytes": step_bytes_survey * B * args.steps / (ms * 1e-3) / 1e9 / peak}
+                     "frac_survey_8d_bytes": step_bytes_survey * B / (ms * 1e-3) / 1e9 / peak}
 
     # ---- end to end: host (pinned) inputs -> H2D -> step -> D2H of losses + detections, every step
     e2e = e2e_full = None
@@ -665,8 +698,9 @@ def run_ours(args, w, world, rank, local_rank):
                                                    "half-precision operator semantics (tests/test_gpu_half_maps.py)"}
         for mode in ("dense", "candidate_first"):
             h_steps = max(3, min(args.steps, 1000))
-            h_ms, h_pipes, h_outs, _, _ = timed_steps(mode, h_steps, max(min(args.warmup, 100), 3), min(args.regions, 3), hsets)
-            half_maps[mode] = {"value": B * h_steps / (h_ms * 1e-3), "unit": UNIT, "ms_per_step": h_ms / h_steps,
+            h_ms, h_pipes, h_outs, _, _, _ = timed_steps(mode, h_steps, max(min(args.warmup, 100), 3), min(args.regions, 3),
+                                                         hsets)
+            half_maps[mode] = {"value": B / (h_ms * 1e-3), "unit": UNIT, "ms_per_step": h_ms,
                                "losses": h_outs[0][0].losses.cpu().tolist()}
             del h_pipes, h_outs
         del hsets
@@ -692,7 +726,7 @@ def run_ours(args, w, world, rank, local_rank):
     clocks = sampler.stop() if sampler else None
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
-        "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
         # `config` names the WORKLOAD only and is the same object in both arms (`--impl reference` prints it too); how this
         # arm executes it, and what the synthetic inputs turned out to contain, sit beside it

@@ -1,44 +1,44 @@
-"""oracle/torch_restatement.py against the REAL reference functions (container only: needs /root/reference).
-This is the link that lets the gpu tests use the restatement as "the reference on the same device"."""
+"""oracle/torch_restatement.py against outputs of the REAL reference functions, stored under tests/golden/ by
+oracle/make_golden.py (same seeded inputs, torch CPU).  This is the link that lets the gpu tests use the restatement as
+"the reference on the same device"."""
+import numpy as np
 import pytest
 import torch
 
 from oracle import golden_cases as gc
 from oracle import ref_loader
 from oracle import torch_restatement as tr
-from sihl_b200 import synth
-
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the authoring container")
 
 
 @pytest.mark.parametrize("name", sorted(gc.GEOMETRIES))
 def test_offsets_scales_anchors(name):
     g = gc.GEOMETRIES[name]
     levels = gc.geom_levels(g)
-    Ref = ref_loader.ObjectDetection()
-    head = Ref(in_channels=[3] + [4] * g["top"], num_classes=1, bottom_level=g["bottom"], top_level=g["top"],
-               num_channels=4, num_layers=0)
-    inputs = [torch.zeros(1, 1, g["height"], g["width"])] + [None] * (g["bottom"] - 1) + [torch.zeros(1, 1, h, w) for h, w in levels]
-    off, sc = head.get_offsets_and_scales(inputs)
-    off_t, sc_t = tr.offsets_and_scales(levels, "cpu")
-    assert torch.equal(off, off_t) and torch.equal(sc, sc_t)
     gold = gc.load("geom_" + name)
+    off_t, sc_t = tr.offsets_and_scales(levels, "cpu")
+    assert torch.equal(off_t, torch.from_numpy(gold["offsets"])) and torch.equal(sc_t, torch.from_numpy(gold["scales"]))
     assert torch.equal(tr.anchors_px(levels, g["width"], g["height"], "cpu"), torch.from_numpy(gold["anchors"]))
 
 
-@pytest.mark.parametrize("seed", range(6))
+@pytest.mark.parametrize("name", sorted(gc.ASSIGN_CASES))
 @pytest.mark.parametrize("relative", [True, False])
-def test_match_one_is_the_reference_bbox_matching(seed, relative):
-    Ref = ref_loader.ObjectDetection()
-    H, W = (640, 640) if seed % 2 == 0 else (384, 512)
-    levels = synth.level_sizes(H, W)
-    anchors = tr.anchors_px(levels, W, H, "cpu")
-    gt = synth.gt_batch_np(1000 + seed, 3, H, W, 80, 60)
-    for bx, _ in gt.per_image():
-        t = torch.from_numpy(bx)
-        ra, rv = Ref.bbox_matching(anchors, t, 9, relative=relative)
-        a, v = tr.match_one(anchors, t, 9, relative)
-        assert torch.equal(ra, a) and torch.equal(rv, v)
+def test_match_one_is_the_reference_bbox_matching(name, relative):
+    """tr.match_one == ObjectDetection.bbox_matching (ref :252-284) in the stored form: positives (flat index, value,
+    assignment) bit-equal, and the number of anchors the raw output assigns per image."""
+    case = gc.ASSIGN_CASES[name]
+    gold, tag = gc.load(name), "rel" if relative else "abs"
+    anchors = torch.from_numpy(gc.load("geom_" + case["geom"])["anchors"])
+    flat, vals, asg, n_valid_raw = [], [], [], []
+    for b, (bx, _) in enumerate(gc.case_gt(case).per_image()):
+        a, v = tr.match_one(anchors, torch.from_numpy(bx), 9, relative)
+        a, v = a.numpy(), v.numpy()
+        n_valid_raw.append(int((a >= 0).sum()))
+        pos = np.nonzero(v > 0)[0]
+        flat.append(pos + b * len(a)); vals.append(v[pos]); asg.append(a[pos])
+    np.testing.assert_array_equal(np.concatenate(flat), gold[f"{tag}_pos_flat"])
+    np.testing.assert_array_equal(np.concatenate(vals), gold[f"{tag}_pos_val"])
+    np.testing.assert_array_equal(np.concatenate(asg), gold[f"{tag}_pos_assign"])
+    np.testing.assert_array_equal(n_valid_raw, gold[f"{tag}_n_valid_raw"])
 
 
 @pytest.mark.parametrize("name", ["train_cfg0", "train_test128", "train_cfg1", "train_empty"])
@@ -78,23 +78,23 @@ def test_forward_tail_equals_the_reference_forward(name):
 
 @pytest.mark.parametrize("name", sorted(gc.QUAD_CASES))
 def test_quad_match_one_is_the_reference_quad_bbox_matching(name):
-    """N1: tr.quad_match_one == QuadrilateralDetection.bbox_matching (ref quadrilateral_detection.py:266-294), raw
-    outputs, and the sihl_b200 anchor helper == the reference's inline anchor construction (ref :156-161)."""
-    Q = ref_loader.QuadrilateralDetection()
+    """N1: tr.quad_match_one == QuadrilateralDetection.bbox_matching (ref quadrilateral_detection.py:266-294) in the
+    stored canonical form, bit-equal, and the sihl_b200 anchor helper == the reference's inline anchor construction
+    (ref :156-161)."""
     case, gold = gc.QUAD_CASES[name], gc.load(name)
     anchors = torch.from_numpy(gold["anchors"])
-    for bx, _ in gc.quad_gt(case).per_image():
+    for b, (bx, _) in enumerate(gc.quad_gt(case).per_image()):
         t = torch.from_numpy(bx).reshape(-1, 4)
-        want = Q.bbox_matching(anchors, t, 9)
-        got = tr.quad_match_one(anchors, t, 9)
-        for w, g in zip(want, got):
-            assert torch.equal(w, g)
+        got = tr.quad_canonical(*tr.quad_match_one(anchors, t, int(gold["topk"])))
+        for key, g in zip(("assignment", "o2o", "iou", "rel"), got):
+            np.testing.assert_array_equal(g.numpy(), gold[key][b], err_msg=key)
     from sihl_b200.heads.quadrilateral_detection import quad_anchors
     sizes = [tuple(int(v) for v in s) for s in gold["level_sizes"]]
     mine = quad_anchors(sizes, range(case["bottom"], case["top"] + 1), case["top"], case["width"], case["height"], "cpu")
     assert torch.equal(mine, anchors)
 
 
+@pytest.mark.skipif(not ref_loader.available(), reason="needs the reference's source (SIHL_REFERENCE_ROOT); no stored outputs")
 def test_quads_to_boxes_equals_the_reference():
     """sihl_b200.heads.quadrilateral_detection.quads_to_boxes == QuadrilateralDetection.quads_to_boxes (ref :318-324)."""
     from sihl_b200.heads.quadrilateral_detection import quads_to_boxes
