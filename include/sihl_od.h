@@ -118,9 +118,9 @@ SIHL_OD_API int sihl_od_assign_select(const float *anchors, const float *anchor_
  * Positive lists (ref :182-184 order = row-major (b,a)): if tile_pos_count !=
  * NULL the kernel writes, per (image, tile), the number of positives and their
  * flat indices b*A+a in ascending order into tile_pos_rows [B * n_tiles * tile];
- * query the geometry with sihl_od_resolve_tiles().  sihl_od_pos_compact() turns
- * the lists into one pos_index (compact rows for the reference's gathered-row
- * MLPs); sihl_od_pos_loss_tiles() consumes them directly for dense maps.
+ * query the geometry with sihl_od_resolve_tiles().  sihl_od_pos_loss_tiles()
+ * consumes the lists directly for dense maps (sihl_od_train_assign compacts them
+ * into one pos_index for the reference's gathered-row MLPs).
  * prefetch_box_raw / prefetch_cls_logits (optional dense maps [B*A,4] / [B*A,C]):
  * the rows of the positives are prefetched into L2 for that next kernel.
  * pos_chunks (optional, int32 [B * n_tiles * tile / 32]): work list of 32-row chunks
@@ -166,38 +166,13 @@ SIHL_OD_API int sihl_od_quad_matching(const float *anchors, int64_t num_anchors,
                           int64_t *assignment, uint8_t *o2o_mask, float *o2m_iou, float *rel_iou,
                           int32_t *sel_anchor, float *sel_val, float *anchor_terms, void *stream);
 
-/* pos_index int32 [capacity] (flat b*A+a, ascending), pos_total int32 [1],
- * pos_image_offsets int32 [B+1] (may be NULL).  Entries beyond capacity are
- * dropped (pos_total still reports the true count). */
-SIHL_OD_API int sihl_od_pos_compact(const int32_t *tile_pos_count, const int32_t *tile_pos_rows, int batch,
-                        int64_t num_anchors, int32_t *pos_index, int64_t capacity, int32_t *pos_total,
-                        int32_t *pos_image_offsets, void *stream);
-
 /* ---- a5-a10: losses ---------------------------------------------------------
- * Dense losses alone (ref :157-163, :175-180) for callers that already hold
- * rel_iou.  iou_preds may be NULL (early-out path).  Accumulates into sums. */
-SIHL_OD_API int sihl_od_dense_loss(const float *loc_logits, const float *iou_preds, const float *rel_iou,
-                       int64_t n, double *sums, void *stream);
-
-/* Positive-row losses (ref :187-208; CIoU loss from torchvision
- * ops/ciou_loss.py:47-64, diou_loss.py:64-91, _utils.py:87-106).
- * pos_index int32 [P] flat b*A+a; n_pos_dev int32 [1] on the device (the true
- * count, clamped to capacity) or NULL to use `capacity` rows.
- * dense_rows != 0: box_raw [B*A,4], cls_logits [B*A,C] addressed by b*A+a;
- * dense_rows == 0: compact rows [P,4] / [P,C] in pos_index order (what the
- * reference's box_head / cls_head produce from flat_feats[o2m_mask]).
- * Either of box_raw / cls_logits may be NULL.  Accumulates sums[4], sums[5]. */
-SIHL_OD_API int sihl_od_pos_loss(const int32_t *pos_index, const int32_t *n_pos_dev, int64_t capacity,
-                     int64_t num_anchors, const float *rel_iou, const int64_t *assignment,
-                     const float *offsets, const float *scales, int img_w, int img_h,
-                     const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
-                     const float *box_raw, const float *cls_logits, int num_classes, int dense_rows,
-                     double *sums, void *stream);
-
-/* The same positive-row losses over DENSE maps (box_raw [B*A,4], cls_logits
- * [B*A,C]) taken straight from the per-tile lists of sihl_od_assign_resolve: no
- * compaction pass, no host round trip.  pos_chunks / tile_pos_rows / tile_pos_aux
- * are what sihl_od_assign_resolve published (the chunk count lives in sums[7]).
+ * Positive-row losses (ref :187-208; CIoU loss from torchvision
+ * ops/ciou_loss.py:47-64, diou_loss.py:64-91, _utils.py:87-106) over DENSE maps
+ * (box_raw [B*A,4], cls_logits [B*A,C]) taken straight from the per-tile lists of
+ * sihl_od_assign_resolve: no compaction pass, no host round trip.  pos_chunks /
+ * tile_pos_rows / tile_pos_aux are what sihl_od_assign_resolve published (the
+ * chunk count lives in sums[7]).
  * Accumulates sums[4], sums[5].  If losses != NULL (with done_counter, a
  * zero-initialised uint32 the kernel resets itself) the last CTA also performs
  * sihl_od_loss_finalize — one launch less on a single GPU. */
@@ -268,29 +243,6 @@ SIHL_OD_API int sihl_od_exchange_status(const void *region, int world, uint64_t 
  * [location, box, class, iou, total]; early-out when sums[6] == 0. */
 SIHL_OD_API int sihl_od_loss_finalize(const double *sums, float *losses, void *stream);
 
-/* Backward of the four loss terms w.r.t. the head outputs (SURVEY.md §7.4).
- * grad_terms: device fp32 [4] = upstream gradient of [location, box, class, iou]
- * loss; NULL means the total loss of ref :210, i.e. {1, 10, 1, 1}.
- *   dloc[i]  = g0 * (sigmoid(loc) - [rel==1]) / sums[1]
- *   diou[i]  = g3 * 2 (iou_pred - rel) / sums[3]         (0 if sums[6] == 0)
- * dbox [P,4] / dcls [P,C] (compact rows) or dense [B*A,..] scattered rows
- * (dense_rows != 0; non-positive rows are NOT written — zero them first):
- *   dcls = g2 * w/sums[3] * (softmax - onehot)
- *   dbox = g1 * w/sums[3] * dCIoU/dpred * scales * exp(raw), alpha constant
- * (the reference's early-out, ref :165-172, leaves box/class/iou heads without
- * gradient; callers skip sihl_od_pos_loss_bwd when there are no positives). */
-SIHL_OD_API int sihl_od_dense_loss_bwd(const float *loc_logits, const float *iou_preds, const float *rel_iou, int64_t n,
-                           const double *sums, const float *grad_terms,
-                           float *dloc, float *diou, void *stream);
-
-SIHL_OD_API int sihl_od_pos_loss_bwd(const int32_t *pos_index, const int32_t *n_pos_dev, int64_t capacity,
-                         int64_t num_anchors, const float *rel_iou, const int64_t *assignment,
-                         const float *offsets, const float *scales, int img_w, int img_h,
-                         const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
-                         const float *box_raw, const float *cls_logits, int num_classes, int dense_rows,
-                         const double *sums, const float *grad_terms,
-                         float *dbox, float *dcls, void *stream);
-
 /* ---- the training step of the drop-in head, three calls (SURVEY.md §8f N2) ------------------
  * What ObjectDetection.training_step (ref :124-217) does around its MLPs, with no host
  * synchronisation, no allocation and a fixed launch sequence (CUDA-graph capturable):
@@ -345,13 +297,19 @@ SIHL_OD_API int sihl_od_train_loss(const void *loc_logits, const void *iou_preds
                        const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
                        double *sums, float *losses, void *stream);
 
-/* sihl_od_train_loss_bwd: ONE launch for all four gradients, written in map_dtype.
- * grad_losses: device fp32 [5] = upstream gradient of [location, box, class, iou, total]
- * (NULL: d total = 1); the effective weights are g_i + g_total * {1,10,1,1}[i] (ref :210),
- * times grad_scale (1, or the world size when the sums were all-reduced and DDP will average
- * the gradients).  dloc / diou [B*A]; dbox_rows [pos_capacity,4] / dcls_rows [pos_capacity,C]:
- * rows >= P are zeroed.  Any output may be NULL.  With no positives (sums[6] == 0) everything
- * but dloc is zero (the reference's early-out returns before those heads run). */
+/* sihl_od_train_loss_bwd: ONE launch for all four gradients, written in map_dtype
+ * (SURVEY.md §7.4).  grad_losses: device fp32 [5] = upstream gradient of [location, box,
+ * class, iou, total] (NULL: d total = 1); the effective weights are
+ * g_i = grad_losses[i] + grad_losses[4] * {1,10,1,1}[i] (ref :210), times grad_scale (1, or the
+ * world size when the sums were all-reduced and DDP will average the gradients).  With
+ * w = rel_iou of row r's location pos_index[r]:
+ *   dloc[i]  = g0 * (sigmoid(loc) - [rel==1]) / sums[1]
+ *   diou[i]  = g3 * 2 (iou_pred - rel) / sums[3]
+ *   dcls_rows[r] = g2 * w/sums[3] * (softmax - onehot)   (NaN for a gt class outside [0, C))
+ *   dbox_rows[r] = g1 * w/sums[3] * dCIoU/dpred * scales * exp(raw), the CIoU alpha held constant
+ * dloc / diou [B*A]; dbox_rows [pos_capacity,4] / dcls_rows [pos_capacity,C]: rows >= P are
+ * zeroed.  Any output may be NULL.  With no positives (sums[6] == 0) everything but dloc is zero
+ * (the reference's early-out, ref :165-172, returns before the box / class / iou heads run). */
 SIHL_OD_API int sihl_od_train_loss_bwd(const void *loc_logits, const void *iou_preds, const void *box_rows, const void *cls_rows,
                            int map_dtype, int batch, int64_t num_anchors, int num_classes,
                            const float *rel_iou, const int64_t *assignment,

@@ -40,12 +40,7 @@ _SIGNATURES = {
     "sihl_od_exchange_barrier": (I, [P, I, I, P]),
     "sihl_od_exchange_set_timeout": (I, [P, I, C.c_uint64]),
     "sihl_od_exchange_status": (I, [P, I, P, P]),
-    "sihl_od_pos_compact": (I, [P, P, I, I64, P, I64, P, P, P]),
-    "sihl_od_dense_loss": (I, [P, P, P, I64, P, P]),
-    "sihl_od_pos_loss": (I, [P, P, I64, I64, P, P, P, P, I, I, P, P, P, P, P, I, I, P, P]),
     "sihl_od_loss_finalize": (I, [P, P, P]),
-    "sihl_od_dense_loss_bwd": (I, [P, P, P, I64, P, P, P, P, P]),
-    "sihl_od_pos_loss_bwd": (I, [P, P, I64, I64, P, P, P, P, I, I, P, P, P, P, P, I, I, P, P, P, P, P]),
     "sihl_od_train_workspace_bytes": (C.c_size_t, [I, I64, I, I]),
     "sihl_od_train_assign": (I, [P, P, I64, P, I, I, I, P, P, P, I, I, I, P, P, P, I64, P, P, P, C.c_size_t, P]),
     "sihl_od_train_loss": (I, [P, P, P, P, I, I, I64, I, P, P, P, I64, P, P, P, I, I, P, P, P, P, P, P]),

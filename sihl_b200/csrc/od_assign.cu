@@ -518,9 +518,8 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
 // Tile lists -> one ascending pos_index (ref :182-184 row order)
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-k_pos_compact(const int32_t *__restrict__ tile_pos_count, const int32_t *__restrict__ tile_pos_rows, int n_tiles,
-              int n_slots, int32_t *__restrict__ pos_index, int64_t capacity, int32_t *__restrict__ pos_total,
-              int32_t *__restrict__ pos_image_offsets, int pad_tail)
+k_pos_compact(const int32_t *__restrict__ tile_pos_count, const int32_t *__restrict__ tile_pos_rows, int n_slots,
+              int32_t *__restrict__ pos_index, int64_t capacity, int32_t *__restrict__ pos_total)
 {
     __shared__ int s_red[32];
     const int slot = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -536,19 +535,13 @@ k_pos_compact(const int32_t *__restrict__ tile_pos_count, const int32_t *__restr
     __syncthreads();
     before = 0; total = 0;
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { before += s_red[w]; total += s_red[16 + w]; }
-    if (tid == 0) {
-        if (slot == 0 && pos_total) *pos_total = total;
-        if (pos_image_offsets) {
-            if (slot % n_tiles == 0) pos_image_offsets[slot / n_tiles] = before;
-            if (slot == n_slots - 1) pos_image_offsets[n_slots / n_tiles] = total;
-        }
-    }
+    if (tid == 0 && slot == 0) *pos_total = total;
     const int n = __ldg(tile_pos_count + slot);
     for (int r = tid; r < n; r += blockDim.x)
         if ((int64_t)before + r < capacity) pos_index[before + r] = __ldg(tile_pos_rows + (int64_t)slot * kTile + r);
-    if (pad_tail)           // rows [total, capacity) are gathered by the static-size MLP batch: any valid row will do
-        for (int64_t r = (int64_t)total + (int64_t)slot * blockDim.x + tid; r < capacity; r += (int64_t)n_slots * blockDim.x)
-            pos_index[r] = 0;
+    // rows [total, capacity) are gathered by the static-size MLP batch: any valid row will do
+    for (int64_t r = (int64_t)total + (int64_t)slot * blockDim.x + tid; r < capacity; r += (int64_t)n_slots * blockDim.x)
+        pos_index[r] = 0;
 }
 
 }  // namespace sihl
@@ -699,8 +692,7 @@ extern "C" int sihl_od_train_assign(const float *anchors, const float *anchor_te
     if (rc) return rc;
     const int n_tiles = (int)((num_anchors + kTile - 1) / kTile);
     const int n_slots = batch * n_tiles;
-    k_pos_compact<<<n_slots, 256, 0, st>>>(w.tile_pos_count, w.tile_pos_rows, n_tiles, n_slots, pos_index, pos_capacity,
-                                           pos_total, nullptr, 1);
+    k_pos_compact<<<n_slots, 256, 0, st>>>(w.tile_pos_count, w.tile_pos_rows, n_slots, pos_index, pos_capacity, pos_total);
     SIHL_CHECK_LAUNCH("k_pos_compact");
     return SIHL_OD_OK;
 }
@@ -754,21 +746,6 @@ extern "C" int sihl_od_assign_resolve_t(const int32_t *sel_anchor, const float *
     SIHL_CHECK_ARG(batch <= 65535, "batch=%d > 65535", batch);
     SIHL_DISPATCH_DTYPE(map_dtype, (k_assign_resolve<T><<<grid, kResThreads, 0, (cudaStream_t)stream>>>(p)));
     SIHL_CHECK_LAUNCH("k_assign_resolve");
-    return SIHL_OD_OK;
-}
-
-extern "C" int sihl_od_pos_compact(const int32_t *tile_pos_count, const int32_t *tile_pos_rows, int batch,
-                                   int64_t num_anchors, int32_t *pos_index, int64_t capacity, int32_t *pos_total,
-                                   int32_t *pos_image_offsets, void *stream)
-{
-    SIHL_CHECK_ARG(tile_pos_count && tile_pos_rows && pos_index, "NULL argument");
-    SIHL_CHECK_ARG(batch >= 0 && num_anchors >= 0 && capacity >= 0, "bad sizes");
-    const int n_tiles = (int)((num_anchors + kTile - 1) / kTile);
-    const int n_slots = batch * n_tiles;
-    if (n_slots == 0) return SIHL_OD_OK;
-    k_pos_compact<<<n_slots, 256, 0, (cudaStream_t)stream>>>(tile_pos_count, tile_pos_rows, n_tiles, n_slots, pos_index,
-                                                              capacity, pos_total, pos_image_offsets, 0);
-    SIHL_CHECK_LAUNCH("k_pos_compact");
     return SIHL_OD_OK;
 }
 

@@ -47,8 +47,6 @@ struct LevelTable {                   // passed by value as a kernel parameter
     int base[SIHL_OD_MAX_LEVELS + 1]; // first anchor index of each level
 };
 
-__device__ __forceinline__ float4 ldg4(const float *p) { return __ldg(reinterpret_cast<const float4 *>(p)); }
-
 // Head-output maps may arrive in half precision (the reference trains with precision="16-mixed",
 // ref examples/object_detection.py:294, and upcasts inside its autocast-off blocks, ref :178,:195,:206):
 // kernels templated on the map type load T and upcast in registers — no fp32 copy of the map is ever made.
@@ -181,7 +179,7 @@ __device__ __forceinline__ float warp_max(float v)
 // kernel's instructions: log1p(e^-|x|) with y = e^-|x| from ex2.approx and, for y < 0.223 (|x| > 1.5: all but a
 // handful of the locations of a detection head whose location logits sit around -5), the alternating series
 // y - y^2/2 + ... - y^8/8 (truncation <= y^8/9 = 7e-7 relative) in 8 FMAs; the exact libdevice path otherwise.
-// The location loss is held to 1e-5 relative (north_star), not to bit equality; sihl_od_dense_loss keeps the
+// The location loss is held to 1e-5 relative (north_star), not to bit equality; sihl_od_train_loss keeps the
 // libdevice form.
 __device__ __forceinline__ float bce_logits_fast(float x, float t)
 {

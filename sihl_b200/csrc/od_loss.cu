@@ -1,11 +1,10 @@
-// od_loss.cu — loss reductions of the detection head and their backward
-// (SURVEY.md §8 a5-a10, §7.4).
+
+// od_loss.cu — positive-row losses of the detection head over dense maps, and the loss finalize
+// (SURVEY.md §8 a5-a10).  The compact-row forward and backward of the drop-in head's training
+// step are in od_train.cu.
 //
-//   k_dense_loss      ref object_detection.py:157-163, :175-180   HBM-bound, 12 B / anchor
-//   k_pos_loss        ref :187-208 (+ torchvision ciou_loss.py)   gather-bound, (16+4C) B / positive
+//   k_pos_loss_tiles  ref :187-208 (+ torchvision ciou_loss.py)   gather-bound, (16+4C) B / positive
 //   k_loss_finalize   ref :163-172, :180, :197, :208, :210        5 scalars
-//   k_dense_loss_bwd  d/d loc_logits, d/d iou_preds               HBM-bound, 20 B / anchor
-//   k_pos_loss_bwd    d/d box_raw, d/d class_logits               (32+8C) B / positive
 //
 // Sums are accumulated per thread in fp32 over a handful of elements, then in fp64
 // through warp shuffles, one shared-memory hop and one atomicAdd per CTA and term.
@@ -15,95 +14,6 @@
 #include "od_pos.cuh"
 
 namespace sihl {
-
-constexpr int kLossThreads = 256;
-
-__global__ void __launch_bounds__(kLossThreads)
-k_dense_loss(const float *__restrict__ loc, const float *__restrict__ iou_pred, const float *__restrict__ rel,
-             int64_t n, double *__restrict__ sums)
-{
-    __shared__ double s_red[5 * 32];
-    double v[5] = {0, 0, 0, 0, 0};
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t base = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; base < n; base += 4 * stride) {
-        float bce = 0.f, one = 0.f, mse = 0.f, rs = 0.f, np = 0.f;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int64_t i = base + u * stride;
-            if (i < n) {
-                const float r = __ldg(rel + i);
-                const float t = (r == 1.0f) ? 1.f : 0.f;
-                bce += bce_logits(__ldg(loc + i), t);
-                one += t;
-                if (iou_pred != nullptr) { const float d = __ldg(iou_pred + i) - r; mse += d * d; }
-                rs += r;
-                np += (r > 0.f) ? 1.f : 0.f;
-            }
-        }
-        v[0] += bce; v[1] += one; v[2] += mse; v[3] += rs; v[4] += np;
-    }
-    const int slot[5] = {0, 1, 2, 3, 6};
-    block_accumulate<5>(v, s_red, sums, slot);
-}
-
-struct PosParams {
-    const int32_t *pos_index; const int32_t *n_pos_dev; int64_t capacity; int num_anchors;
-    const float *rel; const int64_t *assignment;
-    const float4 *offsets; const float4 *scales; float img_w, img_h;
-    const float4 *gt_boxes; const int64_t *gt_classes; const int32_t *gt_offsets;
-    const float *box_raw; const float *cls; int num_classes; int dense_rows;
-    double *sums;                   // fwd: accumulated into; bwd: read
-    const float *grad_terms;        // bwd
-    float *dbox; float *dcls;       // bwd
-};
-
-__device__ __forceinline__ int64_t pos_count(const PosParams &p)
-{
-    int64_t n = p.capacity;
-    if (p.n_pos_dev != nullptr) { const int64_t m = __ldg(p.n_pos_dev); n = m < n ? m : n; }
-    return n;
-}
-
-__global__ void __launch_bounds__(kLossThreads) k_pos_loss(PosParams p)
-{
-    __shared__ double s_red[2 * 32];
-    const int64_t n = pos_count(p);
-    const int A = p.num_anchors;
-    float acc_box = 0.f, acc_cls = 0.f;
-    if (p.box_raw != nullptr) {                                   // thread per positive row
-        for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
-            const int64_t flat = __ldg(p.pos_index + r);
-            const int b = (int)(flat / A), a = (int)(flat - (int64_t)b * A);
-            const int g = __ldg(p.gt_offsets + b) + (int)__ldg(p.assignment + flat);
-            const int64_t row = p.dense_rows ? flat : r;
-            const float l = pos_box_loss(ldg4(p.box_raw + 4 * row), __ldg(p.offsets + a), __ldg(p.scales + a),
-                                         __ldg(p.gt_boxes + g), p.img_w, p.img_h);
-            acc_box += __ldg(p.rel + flat) * l;                   // ref :197
-        }
-    }
-    if (p.cls != nullptr) {                                       // 8 lanes per positive row
-        const int gl = threadIdx.x & 7;
-        const int64_t ngrp = ((int64_t)gridDim.x * blockDim.x) >> 3;
-        const int64_t grp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
-        const int64_t rounds = (n + ngrp - 1) / ngrp;
-        for (int64_t it = 0; it < rounds; ++it) {
-            const int64_t r = it * ngrp + grp;
-            const bool ok = r < n;
-            const int64_t flat = __ldg(p.pos_index + (ok ? r : 0));
-            const int b = (int)(flat / A);
-            const int g = __ldg(p.gt_offsets + b) + (int)__ldg(p.assignment + flat);
-            const int64_t row = p.dense_rows ? flat : (ok ? r : 0);
-            // a label outside [0, C) would read foreign memory (torch raises a device assert there): NaN loss instead
-            const int64_t tgt64 = __ldg(p.gt_classes + g);
-            const bool tgt_ok = tgt64 >= 0 && tgt64 < p.num_classes;
-            const float ce = ce_row_group8(p.cls + row * p.num_classes, p.num_classes, tgt_ok ? (int)tgt64 : 0, gl);
-            if (ok && gl == 0) acc_cls += __ldg(p.rel + flat) * (tgt_ok ? ce : CUDART_NAN_F);   // ref :208
-        }
-    }
-    double v[2] = {acc_box, acc_cls};
-    const int slot[2] = {4, 5};
-    block_accumulate<2>(v, s_red, p.sums, slot);
-}
 
 // Positive-row losses straight from the per-tile lists k_assign_resolve leaves behind (dense
 // maps only).  Work items are 32-row chunks of those lists, published by k_assign_resolve in
@@ -120,8 +30,6 @@ __device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; a
 #else
 #define SIHL_PT(i) do { } while (0)
 #endif
-
-__device__ __forceinline__ void finalize_losses(const double *sums, float *losses);
 
 struct PosTileParams {
     const int32_t *pos_chunks; const int32_t *tile_pos_rows; const int2 *tile_pos_aux; int n_tiles; int num_anchors;
@@ -497,197 +405,20 @@ __global__ void __launch_bounds__(kPosTileThreads, 8) k_pos_loss_tiles(PosTilePa
     SIHL_PT(3);
 }
 
-__device__ __forceinline__ void finalize_losses(const double *sums, float *losses)
-{
-    const double loc = sums[0] / sums[1];                         // ref :163 (0/0 and x/0 as in the reference)
-    if (sums[6] == 0.0) {                                         // ref :165-172, rel_iou.max() == 0
-        losses[0] = (float)loc; losses[1] = 0.f; losses[2] = 0.f; losses[3] = 0.f; losses[4] = (float)loc;
-        return;
-    }
-    const double iou = sums[2] / sums[3], box = sums[4] / sums[3], cls = sums[5] / sums[3];
-    losses[0] = (float)loc; losses[1] = (float)box; losses[2] = (float)cls; losses[3] = (float)iou;
-    losses[4] = (float)(loc + 10.0 * box + cls + iou);           // ref :210
-}
-
 __global__ void k_loss_finalize(const double *__restrict__ sums, float *__restrict__ losses)
 {
     if (threadIdx.x == 0 && blockIdx.x == 0) finalize_losses(sums, losses);
-}
-
-__global__ void __launch_bounds__(kLossThreads)
-k_dense_loss_bwd(const float *__restrict__ loc, const float *__restrict__ iou_pred, const float *__restrict__ rel,
-                 int64_t n, const double *__restrict__ sums, const float *__restrict__ grad_terms,
-                 float *__restrict__ dloc, float *__restrict__ diou)
-{
-    const float g_loc = grad_terms ? __ldg(grad_terms + 0) : 1.f;
-    const float g_iou = grad_terms ? __ldg(grad_terms + 3) : 1.f;
-    const float inv_one = (float)((double)g_loc / sums[1]);
-    const bool early = sums[6] == 0.0;
-    const float inv_rel2 = early ? 0.f : (float)(2.0 * (double)g_iou / sums[3]);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const float r = __ldg(rel + i);
-        if (dloc != nullptr) dloc[i] = (sigmoid_f(__ldg(loc + i)) - ((r == 1.0f) ? 1.f : 0.f)) * inv_one;
-        if (diou != nullptr) diou[i] = early ? 0.f : (__ldg(iou_pred + i) - r) * inv_rel2;
-    }
-}
-
-__global__ void __launch_bounds__(kLossThreads) k_pos_loss_bwd(PosParams p)
-{
-    const int64_t n = pos_count(p);
-    const int A = p.num_anchors;
-    const float g_box = p.grad_terms ? __ldg(p.grad_terms + 1) : 10.f;   // total = loc + 10*box + cls + iou (ref :210)
-    const float g_cls = p.grad_terms ? __ldg(p.grad_terms + 2) : 1.f;
-    const float inv_w = (float)(1.0 / p.sums[3]);
-    if (p.dbox != nullptr) {
-        for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
-            const int64_t flat = __ldg(p.pos_index + r);
-            const int b = (int)(flat / A), a = (int)(flat - (int64_t)b * A);
-            const int g = __ldg(p.gt_offsets + b) + (int)__ldg(p.assignment + flat);
-            const int64_t row = p.dense_rows ? flat : r;
-            const float4 raw = ldg4(p.box_raw + 4 * row), off = __ldg(p.offsets + a), sc = __ldg(p.scales + a);
-            Box4 pred, tgt;
-            pos_boxes(raw, off, sc, __ldg(p.gt_boxes + g), p.img_w, p.img_h, &pred, &tgt);
-            float gr[4];
-            ciou_loss_row(pred, tgt, gr);
-            const float k = g_box * __ldg(p.rel + flat) * inv_w;      // ref :197, :210
-            // d pred_j / d raw_j = scales_j * exp(raw_j) = pred_j - offsets_j
-            const float4 out = make_float4(k * gr[0] * (pred.x1 - off.x), k * gr[1] * (pred.y1 - off.y),
-                                           k * gr[2] * (pred.x2 - off.z), k * gr[3] * (pred.y2 - off.w));
-            *reinterpret_cast<float4 *>(p.dbox + 4 * row) = out;
-        }
-    }
-    if (p.dcls != nullptr) {
-        const int gl = threadIdx.x & 7, C = p.num_classes;
-        const int64_t ngrp = ((int64_t)gridDim.x * blockDim.x) >> 3;
-        const int64_t grp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
-        const int64_t rounds = (n + ngrp - 1) / ngrp;
-        for (int64_t it = 0; it < rounds; ++it) {
-            const int64_t r = it * ngrp + grp;
-            const bool ok = r < n;
-            const int64_t flat = __ldg(p.pos_index + (ok ? r : 0));
-            const int b = (int)(flat / A);
-            const int g = __ldg(p.gt_offsets + b) + (int)__ldg(p.assignment + flat);
-            const int64_t row = p.dense_rows ? flat : (ok ? r : 0);
-            const float *z = p.cls + row * C;
-            float m, s;
-            row_softmax_stats8(z, C, gl, &m, &s);
-            if (ok) {
-                const int64_t tgt64 = __ldg(p.gt_classes + g);
-                const int target = (tgt64 >= 0 && tgt64 < C) ? (int)tgt64 : -1;
-                const float k = target >= 0 ? g_cls * __ldg(p.rel + flat) * inv_w : CUDART_NAN_F;  // ref :208
-                const float inv_s = 1.f / s;
-                float *out = p.dcls + row * C;
-                for (int c = gl; c < C; c += 8)
-                    out[c] = k * (expf(__ldg(z + c) - m) * inv_s - (c == target ? 1.f : 0.f));
-            }
-        }
-    }
-}
-
-static int grid_for(int64_t n, int per_thread)
-{
-    int64_t blocks = (n + (int64_t)kLossThreads * per_thread - 1) / ((int64_t)kLossThreads * per_thread);
-    const int64_t cap = (int64_t)kNumSMs * 8;
-    if (blocks > cap) blocks = cap;
-    return blocks < 1 ? 1 : (int)blocks;
-}
-
-static int fill_pos(PosParams *p, const int32_t *pos_index, const int32_t *n_pos_dev, int64_t capacity,
-                    int64_t num_anchors, const float *rel_iou, const int64_t *assignment, const float *offsets,
-                    const float *scales, int img_w, int img_h, const float *gt_boxes, const int64_t *gt_classes,
-                    const int32_t *gt_offsets, const float *box_raw, const float *cls_logits, int num_classes,
-                    int dense_rows)
-{
-    SIHL_CHECK_ARG(pos_index && rel_iou && assignment && gt_offsets, "NULL argument");
-    SIHL_CHECK_ARG(capacity >= 0 && num_anchors > 0 && num_anchors < (1ll << 30), "bad sizes");
-    // gt_boxes / gt_classes may be NULL when the batch holds no ground truth at all (then no row is positive)
-    SIHL_CHECK_ARG(box_raw == nullptr || (offsets && scales && img_w > 0 && img_h > 0),
-                   "box loss needs offsets, scales and the image size");
-    SIHL_CHECK_ARG(cls_logits == nullptr || num_classes > 0, "class loss needs num_classes");
-    p->pos_index = pos_index; p->n_pos_dev = n_pos_dev; p->capacity = capacity; p->num_anchors = (int)num_anchors;
-    p->rel = rel_iou; p->assignment = assignment;
-    p->offsets = reinterpret_cast<const float4 *>(offsets); p->scales = reinterpret_cast<const float4 *>(scales);
-    p->img_w = (float)img_w; p->img_h = (float)img_h;
-    p->gt_boxes = reinterpret_cast<const float4 *>(gt_boxes); p->gt_classes = gt_classes; p->gt_offsets = gt_offsets;
-    p->box_raw = box_raw; p->cls = cls_logits; p->num_classes = num_classes; p->dense_rows = dense_rows;
-    p->sums = nullptr; p->grad_terms = nullptr; p->dbox = nullptr; p->dcls = nullptr;
-    return SIHL_OD_OK;
 }
 
 }  // namespace sihl
 
 using namespace sihl;
 
-extern "C" int sihl_od_dense_loss(const float *loc_logits, const float *iou_preds, const float *rel_iou, int64_t n,
-                                  double *sums, void *stream)
-{
-    SIHL_CHECK_ARG(loc_logits && rel_iou && sums && n >= 0, "NULL argument");
-    if (n == 0) return SIHL_OD_OK;
-    k_dense_loss<<<grid_for(n, 4), kLossThreads, 0, (cudaStream_t)stream>>>(loc_logits, iou_preds, rel_iou, n, sums);
-    SIHL_CHECK_LAUNCH("k_dense_loss");
-    return SIHL_OD_OK;
-}
-
-extern "C" int sihl_od_pos_loss(const int32_t *pos_index, const int32_t *n_pos_dev, int64_t capacity,
-                                int64_t num_anchors, const float *rel_iou, const int64_t *assignment,
-                                const float *offsets, const float *scales, int img_w, int img_h,
-                                const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
-                                const float *box_raw, const float *cls_logits, int num_classes, int dense_rows,
-                                double *sums, void *stream)
-{
-    PosParams p;
-    int rc = fill_pos(&p, pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w,
-                      img_h, gt_boxes, gt_classes, gt_offsets, box_raw, cls_logits, num_classes, dense_rows);
-    if (rc) return rc;
-    SIHL_CHECK_ARG(sums != nullptr, "sums is NULL");
-    if (capacity == 0 || (box_raw == nullptr && cls_logits == nullptr)) return SIHL_OD_OK;
-    p.sums = sums;
-    k_pos_loss<<<grid_for(capacity, 1) * (cls_logits ? 4 : 1), kLossThreads, 0, (cudaStream_t)stream>>>(p);
-    SIHL_CHECK_LAUNCH("k_pos_loss");
-    return SIHL_OD_OK;
-}
-
 extern "C" int sihl_od_loss_finalize(const double *sums, float *losses, void *stream)
 {
     SIHL_CHECK_ARG(sums && losses, "NULL argument");
     k_loss_finalize<<<1, 32, 0, (cudaStream_t)stream>>>(sums, losses);
     SIHL_CHECK_LAUNCH("k_loss_finalize");
-    return SIHL_OD_OK;
-}
-
-extern "C" int sihl_od_dense_loss_bwd(const float *loc_logits, const float *iou_preds, const float *rel_iou,
-                                      int64_t n, const double *sums, const float *grad_terms, float *dloc,
-                                      float *diou, void *stream)
-{
-    SIHL_CHECK_ARG(rel_iou && sums && n >= 0, "NULL argument");
-    SIHL_CHECK_ARG(dloc == nullptr || loc_logits != nullptr, "dloc needs loc_logits");
-    SIHL_CHECK_ARG(diou == nullptr || iou_preds != nullptr, "diou needs iou_preds");
-    if (n == 0 || (dloc == nullptr && diou == nullptr)) return SIHL_OD_OK;
-    k_dense_loss_bwd<<<grid_for(n, 4), kLossThreads, 0, (cudaStream_t)stream>>>(loc_logits, iou_preds, rel_iou, n, sums,
-                                                                                 grad_terms, dloc, diou);
-    SIHL_CHECK_LAUNCH("k_dense_loss_bwd");
-    return SIHL_OD_OK;
-}
-
-extern "C" int sihl_od_pos_loss_bwd(const int32_t *pos_index, const int32_t *n_pos_dev, int64_t capacity,
-                                    int64_t num_anchors, const float *rel_iou, const int64_t *assignment,
-                                    const float *offsets, const float *scales, int img_w, int img_h,
-                                    const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
-                                    const float *box_raw, const float *cls_logits, int num_classes, int dense_rows,
-                                    const double *sums, const float *grad_terms, float *dbox, float *dcls,
-                                    void *stream)
-{
-    PosParams p;
-    int rc = fill_pos(&p, pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w,
-                      img_h, gt_boxes, gt_classes, gt_offsets, box_raw, cls_logits, num_classes, dense_rows);
-    if (rc) return rc;
-    SIHL_CHECK_ARG(sums != nullptr, "sums is NULL");
-    SIHL_CHECK_ARG(dbox == nullptr || box_raw != nullptr, "dbox needs box_raw");
-    SIHL_CHECK_ARG(dcls == nullptr || cls_logits != nullptr, "dcls needs cls_logits");
-    if (capacity == 0 || (dbox == nullptr && dcls == nullptr)) return SIHL_OD_OK;
-    p.sums = const_cast<double *>(sums); p.grad_terms = grad_terms; p.dbox = dbox; p.dcls = dcls;
-    k_pos_loss_bwd<<<grid_for(capacity, 1) * (dcls ? 4 : 1), kLossThreads, 0, (cudaStream_t)stream>>>(p);
-    SIHL_CHECK_LAUNCH("k_pos_loss_bwd");
     return SIHL_OD_OK;
 }
 

@@ -1,5 +1,5 @@
-// od_pos.cuh — device pieces of the positive-row losses (SURVEY.md §8 a8/a9), shared by the
-// fused resolve kernel (od_assign.cu) and the stand-alone forward/backward kernels (od_loss.cu).
+// od_pos.cuh — device pieces of the losses (SURVEY.md §8 a5-a10) shared by the positive-row loss over
+// dense maps (od_loss.cu) and the compact-row forward / backward of the training step (od_train.cu).
 #pragma once
 
 #include "od_common.cuh"
@@ -51,14 +51,6 @@ __device__ __forceinline__ void row_softmax_stats8(const float *__restrict__ z, 
     *s_out = s;
 }
 
-// Cross-entropy of one row (ref :205-207): logsumexp(z) - z[target].
-__device__ __forceinline__ float ce_row_group8(const float *__restrict__ z, int C, int target, int gl)
-{
-    float m, s;
-    row_softmax_stats8(z, C, gl, &m, &s);
-    return (logf(s) + m) - __ldg(z + target);
-}
-
 // Same with 4 lanes per row and 16-byte loads (C % 4 == 0, 16-byte aligned rows): 8 rows per warp.
 template <bool FAST = false>
 __device__ __forceinline__ void row_softmax_stats4v(const float *__restrict__ z, int C, int gl, float *m_out, float *s_out)
@@ -83,11 +75,17 @@ __device__ __forceinline__ void row_softmax_stats4v(const float *__restrict__ z,
     *s_out = s;
 }
 
-__device__ __forceinline__ float ce_row_group4v(const float *__restrict__ z, int C, int target, int gl)
+// The five losses [location, box, class, iou, total] from the 8 sums (layout in sihl_od.h).
+__device__ __forceinline__ void finalize_losses(const double *sums, float *losses)
 {
-    float m, s;
-    row_softmax_stats4v(z, C, gl, &m, &s);
-    return (logf(s) + m) - __ldg(z + target);
+    const double loc = sums[0] / sums[1];                         // ref :163 (0/0 and x/0 as in the reference)
+    if (sums[6] == 0.0) {                                         // ref :165-172, rel_iou.max() == 0
+        losses[0] = (float)loc; losses[1] = 0.f; losses[2] = 0.f; losses[3] = 0.f; losses[4] = (float)loc;
+        return;
+    }
+    const double iou = sums[2] / sums[3], box = sums[4] / sums[3], cls = sums[5] / sums[3];
+    losses[0] = (float)loc; losses[1] = (float)box; losses[2] = (float)cls; losses[3] = (float)iou;
+    losses[4] = (float)(loc + 10.0 * box + cls + iou);           // ref :210
 }
 
 }  // namespace sihl

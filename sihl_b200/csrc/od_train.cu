@@ -8,7 +8,8 @@
 // Both kernels split their grid by role: the first `dense_blocks` CTAs stream the dense maps
 // (loc_logits / iou_preds / rel_iou: HBM-bound, 12 B per anchor forward, 20 B backward), the others take
 // the compact positive rows (gather-bound, (16+4C) B per positive).  The roles share nothing but the 8
-// fp64 sums, so one launch replaces dense-loss + positive-loss + finalize (and, backward, two launches).
+// fp64 sums, so one launch does the dense losses, the positive-row losses and the finalize (and, backward,
+// both gradient halves).
 // Compact rows: row r of box_rows / cls_rows belongs to location pos_index[r]; only the first
 // P = min(*pos_total, pos_capacity) rows are real (see sihl_od.h).
 #include "od_common.cuh"
@@ -48,18 +49,6 @@ template <typename T> __device__ __forceinline__ float bce_term(float x, float t
     return (1.f - t) * x - round_to<T>(ls);
 }
 template <> __device__ __forceinline__ float bce_term<float>(float x, float t) { return bce_logits(x, t); }
-
-__device__ __forceinline__ void finalize5(const double *sums, float *losses)
-{
-    const double loc = sums[0] / sums[1];                         // ref :163 (0/0 and x/0 as in the reference)
-    if (sums[6] == 0.0) {                                         // ref :165-172, rel_iou.max() == 0
-        losses[0] = (float)loc; losses[1] = 0.f; losses[2] = 0.f; losses[3] = 0.f; losses[4] = (float)loc;
-        return;
-    }
-    const double iou = sums[2] / sums[3], box = sums[4] / sums[3], cls = sums[5] / sums[3];
-    losses[0] = (float)loc; losses[1] = (float)box; losses[2] = (float)cls; losses[3] = (float)iou;
-    losses[4] = (float)(loc + 10.0 * box + cls + iou);           // ref :210
-}
 
 // Class target of positive row r (ref :201-203), or -1 if the label is outside [0, C).
 __device__ __forceinline__ int pos_target(const TrainLossParams &p, int64_t flat, int b)
@@ -176,7 +165,7 @@ __global__ void __launch_bounds__(kTrainThreads) k_train_loss(TrainLossParams p)
         __syncthreads();
         if (s_last && tid == 0) {
             __threadfence();
-            finalize5(const_cast<const double *>(reinterpret_cast<volatile double *>(p.sums)), p.losses);
+            finalize_losses(const_cast<const double *>(reinterpret_cast<volatile double *>(p.sums)), p.losses);
         }
     }
 }

@@ -215,8 +215,7 @@ def resolve_tiles(num_anchors: int) -> Tuple[int, int]:
 
 def assign_resolve(sel, gt: GtBatch, num_anchors: int, topk: int = 9, relative: bool = True,
                    loc_logits: Optional[Tensor] = None, iou_preds: Optional[Tensor] = None,
-                   sums: Optional[Tensor] = None, want_positives: bool = False,
-                   fused: Optional[dict] = None):
+                   sums: Optional[Tensor] = None, fused: Optional[dict] = None):
     """Stage 2 (ref :270-282) with the dense losses (ref :157-163, :175-180) fused when
     ``loc_logits`` is given.  ``fused`` = dict(box_raw, cls_logits, offsets, scales, img_w, img_h)
     additionally runs the positive-row losses over dense maps from the per-tile lists.
@@ -226,18 +225,12 @@ def assign_resolve(sel, gt: GtBatch, num_anchors: int, topk: int = 9, relative: 
     B, A = gt.batch_size, int(num_anchors)
     assignment = torch.empty((B, A), dtype=torch.int64, device=dev)
     out_iou = torch.empty((B, A), dtype=torch.float32, device=dev)
-    tpc = tpr = None
-    if want_positives:
-        n_tiles, tile = resolve_tiles(A)
-        tpc = torch.empty((B * n_tiles,), dtype=torch.int32, device=dev)
-        tpr = torch.empty((B * n_tiles * tile,), dtype=torch.int32, device=dev)
     f = fused or {}
-    chunks = aux = None
+    tpc = tpr = chunks = aux = None
     if f:
         n_tiles, tile = resolve_tiles(A)
-        if tpc is None:
-            tpc = torch.empty((B * n_tiles,), dtype=torch.int32, device=dev)
-            tpr = torch.zeros((B * n_tiles * tile,), dtype=torch.int32, device=dev)
+        tpc = torch.empty((B * n_tiles,), dtype=torch.int32, device=dev)
+        tpr = torch.zeros((B * n_tiles * tile,), dtype=torch.int32, device=dev)
         chunks = torch.zeros((B * n_tiles * (tile // 32),), dtype=torch.int32, device=dev)
         aux = torch.zeros((B * n_tiles * tile, 2), dtype=torch.int32, device=dev)
     with _on(dev):
@@ -252,22 +245,6 @@ def assign_resolve(sel, gt: GtBatch, num_anchors: int, topk: int = 9, relative: 
             pos_loss_tiles(chunks, tpr, aux, B, A, f["offsets"], f["scales"], f["img_w"], f["img_h"], gt,
                            f.get("box_raw"), f.get("cls_logits"), sums)
     return dict(assignment=assignment, iou=out_iou, tile_pos_count=tpc, tile_pos_rows=tpr)
-
-
-def pos_compact(tile_pos_count: Tensor, tile_pos_rows: Tensor, batch: int, num_anchors: int,
-                capacity: Optional[int] = None):
-    """Tile lists -> ``pos_index`` in the row order of ``flat_feats[o2m_mask]`` (ref :182-184).
-    Returns ``(pos_index [capacity] i32, pos_total [1] i32, pos_image_offsets [B+1] i32)``."""
-    dev = tile_pos_count.device
-    cap = int(capacity if capacity is not None else tile_pos_rows.numel())
-    pos_index = torch.empty((max(cap, 1),), dtype=torch.int32, device=dev)
-    total = torch.zeros((1,), dtype=torch.int32, device=dev)
-    img_off = torch.zeros((batch + 1,), dtype=torch.int32, device=dev)
-    with _on(dev):
-        rc = _lib().sihl_od_pos_compact(_p(tile_pos_count), _p(tile_pos_rows), int(batch), int(num_anchors),
-                                        _p(pos_index), cap, _p(total), _p(img_off), _stream(dev))
-    _native.check(rc, "sihl_od_pos_compact")
-    return pos_index, total, img_off
 
 
 def bbox_matching(anchors: Tensor, gt_boxes: Tensor, topk: int, relative: bool = False,
@@ -320,41 +297,6 @@ def new_sums(device) -> Tensor:
     return torch.zeros((NUM_SUMS,), dtype=torch.float64, device=device)
 
 
-def dense_loss(loc_logits: Tensor, iou_preds: Optional[Tensor], rel_iou: Tensor, sums: Tensor) -> Tensor:
-    """ref :157-163, :175-180 — accumulates into ``sums`` (fp64 [8])."""
-    loc = _req(loc_logits, torch.float32, "loc_logits")
-    rel = _req(rel_iou, torch.float32, "rel_iou")
-    iou = None if iou_preds is None else _req(iou_preds, torch.float32, "iou_preds")
-    sums = _req(sums, torch.float64, "sums")
-    dev = rel.device
-    with _on(dev):
-        rc = _lib().sihl_od_dense_loss(_p(loc), _p(iou), _p(rel), rel.numel(), _p(sums), _stream(dev))
-    _native.check(rc, "sihl_od_dense_loss")
-    return sums
-
-
-def _pos_args(pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w, img_h,
-              gt: GtBatch, box_raw, cls_logits, dense_rows):
-    return [_p(pos_index), _p(n_pos_dev), int(capacity), int(num_anchors), _p(rel_iou), _p(assignment), _p(offsets),
-            _p(scales), int(img_w), int(img_h), _p(gt.boxes), _p(gt.classes), _p(gt.offsets),
-            _p(None if box_raw is None else _req(box_raw, torch.float32, "box_raw")),
-            _p(None if cls_logits is None else _req(cls_logits, torch.float32, "cls_logits")),
-            0 if cls_logits is None else int(cls_logits.shape[-1]), int(bool(dense_rows))]
-
-
-def pos_loss(pos_index: Tensor, n_pos_dev: Optional[Tensor], capacity: int, num_anchors: int, rel_iou: Tensor,
-             assignment: Tensor, offsets: Tensor, scales: Tensor, img_w: int, img_h: int, gt: GtBatch,
-             box_raw: Optional[Tensor], cls_logits: Optional[Tensor], dense_rows: bool, sums: Tensor) -> Tensor:
-    """ref :187-208 — weighted CIoU loss and cross-entropy over the positive rows."""
-    dev = rel_iou.device
-    args = _pos_args(pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w, img_h,
-                     gt, box_raw, cls_logits, dense_rows)
-    with _on(dev):
-        rc = _lib().sihl_od_pos_loss(*args, _p(sums), _stream(dev))
-    _native.check(rc, "sihl_od_pos_loss")
-    return sums
-
-
 def pos_loss_tiles(pos_chunks: Tensor, tile_pos_rows: Tensor, tile_pos_aux: Tensor, batch: int, num_anchors: int,
                    offsets: Tensor, scales: Tensor, img_w: int, img_h: int, gt: GtBatch,
                    box_raw: Optional[Tensor], cls_logits: Optional[Tensor], sums: Tensor,
@@ -380,33 +322,6 @@ def loss_finalize(sums: Tensor) -> Tensor:
         rc = _lib().sihl_od_loss_finalize(_p(sums), _p(out), _stream(sums.device))
     _native.check(rc, "sihl_od_loss_finalize")
     return out
-
-
-def dense_loss_bwd(loc_logits: Tensor, iou_preds: Optional[Tensor], rel_iou: Tensor, sums: Tensor,
-                   grad_terms: Optional[Tensor], want_dloc: bool = True, want_diou: bool = True):
-    dev = rel_iou.device
-    dloc = torch.empty_like(loc_logits, dtype=torch.float32) if want_dloc else None
-    diou = torch.empty_like(iou_preds, dtype=torch.float32) if (want_diou and iou_preds is not None) else None
-    with _on(dev):
-        rc = _lib().sihl_od_dense_loss_bwd(_p(loc_logits), _p(iou_preds), _p(rel_iou), rel_iou.numel(), _p(sums),
-                                           _p(grad_terms), _p(dloc), _p(diou), _stream(dev))
-    _native.check(rc, "sihl_od_dense_loss_bwd")
-    return dloc, diou
-
-
-def pos_loss_bwd(pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w, img_h,
-                 gt: GtBatch, box_raw, cls_logits, dense_rows, sums, grad_terms, dbox=None, dcls=None):
-    dev = rel_iou.device
-    if dbox is None and box_raw is not None:
-        dbox = torch.zeros_like(box_raw) if dense_rows else torch.empty_like(box_raw)
-    if dcls is None and cls_logits is not None:
-        dcls = torch.zeros_like(cls_logits) if dense_rows else torch.empty_like(cls_logits)
-    args = _pos_args(pos_index, n_pos_dev, capacity, num_anchors, rel_iou, assignment, offsets, scales, img_w, img_h,
-                     gt, box_raw, cls_logits, dense_rows)
-    with _on(dev):
-        rc = _lib().sihl_od_pos_loss_bwd(*args, _p(sums), _p(grad_terms), _p(dbox), _p(dcls), _stream(dev))
-    _native.check(rc, "sihl_od_pos_loss_bwd")
-    return dbox, dcls
 
 
 # --------------------------------------------------------------------------- the drop-in head's training step (N2)

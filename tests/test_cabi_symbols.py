@@ -55,7 +55,7 @@ def test_sm100a_only_and_blackwell_bulk_copy_in_sass():
     assert "UBLKCP" in sass and "SYNCS" in sass      # cp.async.bulk + mbarrier (TMA-class bulk copies)
 
 
-def test_ops_reject_cpu_tensors():
+def test_topk_and_nms_reject_cpu_tensors():
     import pytest
     import torch
 
@@ -63,7 +63,7 @@ def test_ops_reject_cpu_tensors():
     with pytest.raises(RuntimeError, match="CUDA tensors only"):
         ops.topk_locations(torch.zeros(2, 300), 100)
     with pytest.raises(RuntimeError, match="CUDA tensors only"):
-        ops.dense_loss(torch.zeros(10), None, torch.zeros(10), torch.zeros(8, dtype=torch.float64))
+        ops.batched_nms(torch.zeros(10, 4), torch.zeros(10), torch.zeros(10, dtype=torch.int64), 0.5)
 
 
 def test_exchange_and_split_helpers_without_a_gpu():

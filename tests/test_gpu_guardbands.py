@@ -136,7 +136,7 @@ def test_batched_nms_stays_inside_its_buffers(guarded, n, n_cls, segments):
     guarded.check()
 
 
-def test_training_entry_points_stay_inside_their_buffers(guarded):
+def test_training_and_assignment_entries_stay_inside_their_buffers(guarded):
     size, B, C, G = 320, 3, 10, 20
     levels = synth.level_sizes(size, size)
     A = synth.num_anchors(levels)
@@ -161,9 +161,8 @@ def test_training_entry_points_stay_inside_their_buffers(guarded):
     g = ops.GtBatch(gt_boxes, gt_classes, _t(gt.offsets), [20, 0, 7])
     sums = ops.new_sums(DEV)
     sel = ops.assign_select(anchors, levels, size, size, g, 9, sums=sums)
-    res = ops.assign_resolve(sel, g, A, 9, True, loc, iou, sums, want_positives=True,
-                             fused=dict(box_raw=box, cls_logits=cls, offsets=off, scales=sc, img_w=size, img_h=size))
-    ops.pos_compact(res["tile_pos_count"], res["tile_pos_rows"], B, A, capacity=17)      # fewer slots than positives
+    ops.assign_resolve(sel, g, A, 9, True, loc, iou, sums,
+                       fused=dict(box_raw=box, cls_logits=cls, offsets=off, scales=sc, img_w=size, img_h=size))
     ops.loss_finalize(sums)
     ops.bbox_matching(anchors, gt_boxes[:20], 9, True)
     ops.quad_bbox_matching(anchors, g, 9)

@@ -138,43 +138,65 @@ def test_assign_errors_mirror_reference():
 
 
 # --------------------------------------------------------------------------- a5-a10
-def _train(case, g, levels, W, H, fused):
-    gt_np = gc.case_gt(case)
+def _train_inputs(case):
+    gt_np, maps = gc.case_gt(case), gc.train_maps(case)
+    return gt_np, maps, [_t(m) for m in (maps.loc_logits, maps.iou_preds, maps.box_raw, maps.cls_logits)]
+
+
+def _pipeline_losses(case, g, levels, W, H):
+    """assign_select + assign_resolve with the fused dense and positive-row losses + loss_finalize, on the golden tables."""
+    gt_np, maps, (loc, iou, box, cls) = _train_inputs(case)
     gt = _gt_dev(gt_np)
-    maps = gc.train_maps(case)
-    B, A = maps.loc_logits.shape
+    A = maps.loc_logits.shape[1]
     off, sc, anchors = _t(g["offsets"]), _t(g["scales"]), _t(g["anchors"])
-    loc, iou, box, cls = _t(maps.loc_logits), _t(maps.iou_preds), _t(maps.box_raw), _t(maps.cls_logits)
     sums = ops.new_sums(DEV)
     sums.fill_(123.0)                                  # select must zero it
     sel = ops.assign_select(anchors, levels, W, H, gt, 9, sums=sums)
-    fd = dict(box_raw=box, cls_logits=cls, offsets=off, scales=sc, img_w=W, img_h=H) if fused else None
-    res = ops.assign_resolve(sel, gt, A, 9, True, loc, iou, sums, want_positives=True, fused=fd)
-    pos_index, total, img_off = ops.pos_compact(res["tile_pos_count"], res["tile_pos_rows"], B, A)
-    P = int(total.item())
-    if not fused:
-        ops.pos_loss(pos_index, total, pos_index.numel(), A, res["iou"], res["assignment"], off, sc, W, H, gt, box, cls,
-                     True, sums)
+    res = ops.assign_resolve(sel, gt, A, 9, True, loc, iou, sums,
+                             fused=dict(box_raw=box, cls_logits=cls, offsets=off, scales=sc, img_w=W, img_h=H))
     losses = ops.loss_finalize(sums)
-    return dict(gt_np=gt_np, gt=gt, maps=maps, res=res, pos_index=pos_index[:P], P=P, img_off=img_off, sums=sums,
-                losses=losses, dev=(off, sc, anchors, loc, iou, box, cls))
+    # the per-tile positive lists, concatenated in tile order, are the compact positive index
+    _, tile = ops.resolve_tiles(A)
+    counts = res["tile_pos_count"].cpu().numpy()
+    lists = res["tile_pos_rows"].cpu().numpy().reshape(-1, tile)
+    pos_index = np.concatenate([np.zeros(0, np.int32)] + [lists[s, :n] for s, n in enumerate(counts)])
+    return dict(tables=(g["anchors"], g["offsets"], g["scales"]), assignment=res["assignment"], pos_index=pos_index,
+                sums=sums, losses=losses)
+
+
+def _train_losses(case, levels, W, H):
+    """train_assign + train_loss on the compact rows gathered by pos_index (what the drop-in head runs).  train_assign
+    builds its own anchor tables on the device; they are returned for the oracle."""
+    gt_np, maps, (loc, iou, box, cls) = _train_inputs(case)
+    B, A = maps.loc_logits.shape
+    st = ops.train_assign(levels, W, H, _t(gt_np.boxes).reshape(-1, 4), _t(gt_np.classes), np.diff(gt_np.offsets).tolist(),
+                          B, 9)
+    rows = st.pos_index.long()
+    losses, maps_used = ops.train_loss(st, loc, iou, box.reshape(B * A, 4)[rows], cls.reshape(B * A, -1)[rows])
+    P = int(st.pos_total.item())
+    off, sc, anchors = ops.anchor_tables(levels, W, H, DEV)
+    return dict(tables=(anchors.cpu().numpy(), off.cpu().numpy(), sc.cpu().numpy()), assignment=st.assignment,
+                pos_index=st.pos_index[:P].cpu().numpy(), sums=st.sums, losses=losses, st=st, maps=maps_used)
 
 
 @pytest.mark.parametrize("name", sorted(gc.TRAIN_CASES))
-@pytest.mark.parametrize("fused", [False, True])
-def test_train_losses(name, fused):
+@pytest.mark.parametrize("path", ["pipeline", "train"])
+def test_train_losses(name, path):
     case = gc.TRAIN_CASES[name]
     g, levels, W, H = _geom(case["geom"])
     gold = gc.load(name)
-    r = _train(case, g, levels, W, H, fused)
-    gt_np, maps = r["gt_np"], r["maps"]
-    want = orc.train_losses(g["anchors"], g["offsets"], g["scales"], W, H, gt_np.boxes, gt_np.classes, gt_np.offsets,
+    r = _pipeline_losses(case, g, levels, W, H) if path == "pipeline" else _train_losses(case, levels, W, H)
+    gt_np, maps = gc.case_gt(case), gc.train_maps(case)
+    B, A = maps.loc_logits.shape
+    anchors, off, sc = r["tables"]
+    want = orc.train_losses(anchors, off, sc, W, H, gt_np.boxes, gt_np.classes, gt_np.offsets,
                             maps.loc_logits, maps.iou_preds, maps.box_raw, maps.cls_logits, dense_rows=True)
-    np.testing.assert_array_equal(r["res"]["assignment"].cpu().numpy(), want["assignment"])
-    np.testing.assert_array_equal(r["pos_index"].cpu().numpy(), want["pos_index"])     # row order of flat_feats[o2m_mask]
+    np.testing.assert_array_equal(r["assignment"].cpu().numpy(), want["assignment"])
+    pos_index = r["pos_index"]
+    np.testing.assert_array_equal(pos_index, want["pos_index"])     # row order of flat_feats[o2m_mask]
     got_sums = r["sums"].cpu().numpy()
     np.testing.assert_allclose(got_sums[:7], want["sums"][:7], rtol=1e-5, atol=1e-9)
-    assert got_sums[6] == r["P"]
+    assert got_sums[6] == len(pos_index)
     got = r["losses"].cpu().numpy()
     gold_l = [gold["location_loss"], gold["box_loss"], gold["class_loss"], gold["iou_loss"], gold["loss"]]
     for gv, wv, ov in zip(got, gold_l, want["losses"]):
@@ -183,52 +205,28 @@ def test_train_losses(name, fused):
             assert gv == pytest.approx(float(ov), rel=1e-5)
         else:
             assert not np.isfinite(gv)
-    offs = r["img_off"].cpu().numpy()
     per_img = (want["rel_iou"] > 0).sum(1)
-    np.testing.assert_array_equal(np.diff(offs), per_img)
+    np.testing.assert_array_equal(np.bincount(pos_index // A, minlength=B), per_img)
 
 
 @pytest.mark.parametrize("name", ["train_cfg0", "train_test128", "train_cfg1"])
-@pytest.mark.parametrize("dense_rows", [True, False])
-def test_loss_backward_vs_reference_autograd(name, dense_rows):
+def test_loss_backward_vs_reference_autograd(name):
     case = gc.TRAIN_CASES[name]
     g, levels, W, H = _geom(case["geom"])
     gold = gc.load(name)
     if not np.isfinite(gold["loss"]) or "dloc" not in gold:
         pytest.skip("reference loss is not finite for this fixture (no anchor with rel==1)")
-    r = _train(case, g, levels, W, H, fused=False)
-    off, sc, anchors, loc, iou, box, cls = r["dev"]
-    B, A = loc.shape
-    res, P, pos_index = r["res"], r["P"], r["pos_index"]
-    dloc, diou = ops.dense_loss_bwd(loc, iou, res["iou"], r["sums"], None)
-    np.testing.assert_allclose(dloc.cpu().numpy().reshape(-1), gold["dloc"].reshape(-1), rtol=2e-5, atol=1e-9)
+    r = _train_losses(case, levels, W, H)
+    dloc, diou, dbox, dcls = (t.cpu().numpy() for t in ops.train_loss_bwd(r["st"], r["maps"], None))
+    np.testing.assert_allclose(dloc.reshape(-1), gold["dloc"].reshape(-1), rtol=2e-5, atol=1e-9)
     # rel_iou of the CPU-run reference differs by ~1e-7 absolute (atan last bit); 2*(p-rel)/R inherits it
-    np.testing.assert_allclose(diou.cpu().numpy().reshape(-1), gold["diou"].reshape(-1), rtol=2e-5, atol=2e-8)
-    rows = gold["grad_rows"]
-    np.testing.assert_array_equal(pos_index.cpu().numpy(), rows)
-    if dense_rows:
-        dbox, dcls = ops.pos_loss_bwd(pos_index, None, P, A, res["iou"], res["assignment"], off, sc, W, H, r["gt"], box, cls,
-                                      True, r["sums"], None)
-        dbox = dbox.reshape(B * A, 4)[pos_index.long()]
-        dcls = dcls.reshape(B * A, -1)[pos_index.long()]
-    else:
-        box_c = box.reshape(B * A, 4)[pos_index.long()].contiguous()
-        cls_c = cls.reshape(B * A, -1)[pos_index.long()].contiguous()
-        dbox, dcls = ops.pos_loss_bwd(pos_index, None, P, A, res["iou"], res["assignment"], off, sc, W, H, r["gt"], box_c,
-                                      cls_c, False, r["sums"], None)
-    np.testing.assert_allclose(dbox.cpu().numpy(), gold["dbox"], rtol=2e-4, atol=2e-7)
-    np.testing.assert_allclose(dcls.cpu().numpy(), gold["dcls"], rtol=2e-5, atol=1e-9)
-
-
-def test_dense_loss_standalone_matches_fused():
-    case = gc.TRAIN_CASES["train_cfg1"]
-    g, levels, W, H = _geom(case["geom"])
-    r = _train(case, g, levels, W, H, fused=False)
-    off, sc, anchors, loc, iou, box, cls = r["dev"]
-    sums2 = ops.new_sums(DEV)
-    ops.dense_loss(loc, iou, r["res"]["iou"], sums2)
-    a, b = r["sums"].cpu().numpy(), sums2.cpu().numpy()
-    np.testing.assert_allclose(b[[0, 1, 2, 3, 6]], a[[0, 1, 2, 3, 6]], rtol=1e-7)   # fp32 partials grouped differently
+    np.testing.assert_allclose(diou.reshape(-1), gold["diou"].reshape(-1), rtol=2e-5, atol=2e-8)
+    np.testing.assert_array_equal(r["pos_index"], gold["grad_rows"])
+    P = len(r["pos_index"])
+    np.testing.assert_allclose(dbox[:P], gold["dbox"], rtol=2e-4, atol=2e-7)
+    np.testing.assert_allclose(dcls[:P], gold["dcls"], rtol=2e-5, atol=1e-9)
+    np.testing.assert_array_equal(dbox[P:], 0)                       # padding rows: zero gradient (sihl_od.h)
+    np.testing.assert_array_equal(dcls[P:], 0)
 
 
 # --------------------------------------------------------------------------- a11
