@@ -443,6 +443,42 @@ SIHL_OD_API int sihl_od_batched_nms(const float *boxes, const float *scores, con
                         float iou_thr, int64_t *keep, int32_t *keep_count,
                         void *workspace, void *stream);
 
+/* Class-aware Soft-NMS (Bodla et al., ICCV 2017, Algorithm 1; mmcv's soft_nms) per image.  Scores are decayed
+ * instead of dropped: starting from the candidates with score >= score_thr, repeatedly select the alive candidate
+ * with the largest current score (ties: lowest location, or lowest input index for the stand-alone entry), emit it
+ * with its current score, and multiply the score of every alive candidate of the SAME class by w(iou) where
+ * iou = inter / ((area_m + area_j) - inter) in fp32 (the operator order of the hard NMS; NaN -> 0):
+ *   SIHL_OD_SOFT_NMS_LINEAR:   w = iou > iou_thr ? 1 - iou : 1                           (fp32)
+ *   SIHL_OD_SOFT_NMS_GAUSSIAN: w = (float)exp(-(double)iou * (double)iou / (double)sigma) (fp64 exp, one rounding)
+ * A candidate whose decayed score falls below score_thr (or is NaN) is dropped.  Emitted scores never increase
+ * along the output and are never below score_thr.  iou_thr is only read by the linear method, sigma (> 0) only by
+ * the Gaussian one. */
+#define SIHL_OD_SOFT_NMS_LINEAR 1
+#define SIHL_OD_SOFT_NMS_GAUSSIAN 2
+
+/* Soft-NMS over the candidate lists of sihl_od_dense_decode: same preconditions (distinct keys), output layout
+ * (first K detections per image, zero padded past num_instances) and reset_counts meaning as sihl_od_nms_topk.
+ * workspace: sihl_od_soft_nms_workspace_bytes(batch, cand_capacity) bytes (0 up to 32768 candidates per image, which
+ * stay in shared memory; NULL is then accepted). */
+SIHL_OD_API size_t sihl_od_soft_nms_workspace_bytes(int batch, int64_t cand_capacity);
+SIHL_OD_API int sihl_od_soft_nms_topk(const int32_t *cand_count, int64_t cand_capacity,
+                     const uint64_t *cand_key, const float *cand_box, const int32_t *cand_cls,
+                     int batch, int method, float iou_thr, float sigma, float score_thr, int k,
+                     int64_t *num_instances, float *scores, int64_t *classes, float *boxes,
+                     void *workspace, int reset_counts, void *stream);
+
+/* Segment form of the same operation, beside sihl_od_batched_nms: boxes [N,4], scores [N], classes int64 [N] in
+ * [0, 2^32), seg_offsets int32 [n_images+1] (device).  Per segment s, at most max_out kept input indices (global, into
+ * [0,N)) in selection order and their decayed scores are written at keep[seg_offsets[s] ...] and
+ * keep_scores[seg_offsets[s] ...]; keep_count int32 [n_images].  Entries past keep_count are left untouched.
+ * workspace: sihl_od_batched_soft_nms_workspace_bytes(N) bytes (0 up to N = 32768; NULL is then accepted). */
+SIHL_OD_API size_t sihl_od_batched_soft_nms_workspace_bytes(int64_t n);
+SIHL_OD_API int sihl_od_batched_soft_nms(const float *boxes, const float *scores, const int64_t *classes,
+                        const int32_t *seg_offsets, int n_images, int64_t n,
+                        int method, float iou_thr, float sigma, float score_thr, int max_out,
+                        int64_t *keep, float *keep_scores, int32_t *keep_count,
+                        void *workspace, void *stream);
+
 /* ---- N3 (SURVEY.md §8f): detection <-> ground-truth matching for the validation mAP ----------
  * What torchmetrics' MeanAveragePrecision (ref object_detection.py:219-237, :245; COCOeval.evaluateImg of its
  * faster_coco_eval backend) does per image on the CPU at epoch end, done on the GPU right after forward():

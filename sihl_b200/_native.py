@@ -60,6 +60,10 @@ _SIGNATURES = {
     "sihl_od_nms_topk_split": (I, [P, I64, P, P, P, I, F, I, P, P, P, P, P, I, P]),
     "sihl_od_batched_nms_workspace_bytes": (C.c_size_t, [I64]),
     "sihl_od_batched_nms": (I, [P, P, P, P, I, I64, F, P, P, P, P]),
+    "sihl_od_soft_nms_workspace_bytes": (C.c_size_t, [I, I64]),
+    "sihl_od_soft_nms_topk": (I, [P, I64, P, P, P, I, I, F, F, F, I, P, P, P, P, P, I, P]),
+    "sihl_od_batched_soft_nms_workspace_bytes": (C.c_size_t, [I64]),
+    "sihl_od_batched_soft_nms": (I, [P, P, P, P, I, I64, I, F, F, F, I, P, P, P, P, P]),
     "sihl_od_mlp_hidden": (I, [P, I64, I, P, P, P, P, F, P, P]),
     "sihl_od_mlp_out": (I, [P, I64, I, P, P, I, I, P, P]),
     "sihl_od_mlp_hidden_train": (I, [P, I64, I, P, P, P, P, F, P, P, P, P]),

@@ -22,7 +22,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsihl_b200.so")
 STAMP_PATH = os.path.join(LIB_DIR, "libsihl_b200.stamp")
-SOURCES = ["od_api.cu", "od_anchors.cu", "od_assign.cu", "od_quad.cu", "od_loss.cu", "od_train.cu", "od_exchange.cu", "od_infer.cu", "od_nms.cu", "od_nms_wide.cu", "od_map.cu", "od_mlp.cu"]
+SOURCES = ["od_api.cu", "od_anchors.cu", "od_assign.cu", "od_quad.cu", "od_loss.cu", "od_train.cu", "od_exchange.cu", "od_infer.cu", "od_nms.cu", "od_nms_wide.cu", "od_soft_nms.cu", "od_map.cu", "od_mlp.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

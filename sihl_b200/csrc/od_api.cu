@@ -25,6 +25,6 @@ int cuda_status(cudaError_t e, const char *what)
 
 }  // namespace sihl
 
-extern "C" int sihl_od_version(void) { return 101; }   // 0.1.1
+extern "C" int sihl_od_version(void) { return 102; }   // 0.1.2
 
 extern "C" const char *sihl_od_last_error_string(void) { return sihl::g_error; }

@@ -160,6 +160,16 @@ template <> __device__ __forceinline__ void st_vec16<__nv_bfloat16>(__nv_bfloat1
 
 __device__ __forceinline__ Box4 to_box(float4 b) { return Box4{b.x, b.y, b.z, b.w}; }
 
+// IoU of two xyxy boxes with the operator order of od_nms.cu's iou_gt (torchvision's CPU nms kernel):
+// inter / ((area_a + area_b) - inter), areas as (x2 - x1) * (y2 - y1).  NaN when both boxes have zero area.
+__device__ __forceinline__ float box_iou(float4 a, float area_a, float4 b, float area_b)
+{
+    const float w = fmaxf(0.f, fminf(a.z, b.z) - fmaxf(a.x, b.x));
+    const float h = fmaxf(0.f, fminf(a.w, b.w) - fmaxf(a.y, b.y));
+    const float inter = w * h;
+    return inter / ((area_a + area_b) - inter);
+}
+
 template <typename T>
 __device__ __forceinline__ T warp_sum(T v)
 {

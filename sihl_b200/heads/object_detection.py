@@ -324,14 +324,20 @@ class ObjectDetection(nn.Module):
 
     @torch.no_grad()
     def postprocess(self, inputs: List[Tensor], score_threshold: float = 0.05, iou_threshold: float = 0.5,
-                    mode: Optional[str] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                    mode: Optional[str] = None, nms: str = "hard", sigma: float = 0.5) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
         """North-star extension (the reference has no NMS): every location is decoded with the
         score/class semantics of ``forward`` (score = sigmoid(location logit), class = argmax),
         thresholded, and de-duplicated by class-aware NMS; same output format as ``forward``.
 
         ``mode``: ``"dense"`` streams the whole class map (TMA ring), ``"candidate_first"`` reads the class row and raw
         box of the locations that pass the threshold only — identical results; default: ``"dense"`` for fp32 maps,
-        ``"candidate_first"`` for half maps (autocast), which are then read as they are (no fp32 copies)."""
+        ``"candidate_first"`` for half maps (autocast), which are then read as they are (no fp32 copies).
+
+        ``nms``: ``"hard"`` (greedy NMS), ``"soft_linear"`` (Soft-NMS, ``iou_threshold`` is Nt) or ``"soft_gaussian"``
+        (Soft-NMS with ``sigma``): overlapping boxes of a class have their scores decayed instead of being dropped,
+        which keeps real objects in crowds; the returned scores are the decayed ones."""
+        if nms not in ops.NMS_KINDS:
+            raise ValueError(f"nms={nms!r}: expected one of {ops.NMS_KINDS}")
         (_, _, height, width) = inputs[0].shape
         flat_feats = self._tower_feats(inputs)
         loc_logits = self._tower("loc_head", flat_feats).squeeze(2)
@@ -340,7 +346,7 @@ class ObjectDetection(nn.Module):
         if mode is None:
             mode = "dense" if loc_logits.dtype == torch.float32 else "candidate_first"
         return ops.dense_postprocess(loc_logits, cls_logits, box_raw, self._level_sizes(inputs), int(width), int(height),
-                                     score_threshold, iou_threshold, self.max_instances, mode=mode)
+                                     score_threshold, iou_threshold, self.max_instances, mode=mode, nms=nms, sigma=sigma)
 
     # ------------------------------------------------------------------ training
     def _reduce_sums(self) -> Optional[callable]:

@@ -624,18 +624,61 @@ def nms_topk(cand: CandidateBuffers, batch: int, iou_thr: float, k: int, out: Op
     return out
 
 
+SOFT_NMS_METHODS = {"linear": 1, "gaussian": 2}          # SIHL_OD_SOFT_NMS_LINEAR / _GAUSSIAN (sihl_od.h)
+NMS_KINDS = ("hard", "soft_linear", "soft_gaussian")
+
+
+def _soft_method(method) -> int:
+    if isinstance(method, str) and method in SOFT_NMS_METHODS:
+        return SOFT_NMS_METHODS[method]
+    if not isinstance(method, str) and method in SOFT_NMS_METHODS.values():
+        return int(method)
+    raise ValueError(f"method={method!r}: expected one of {tuple(SOFT_NMS_METHODS)}")
+
+
+def soft_nms_topk(cand: CandidateBuffers, batch: int, method, iou_thr: float, sigma: float, score_thr: float, k: int,
+                  out: Optional[tuple] = None, reset_counts: bool = False):
+    """Class-aware Soft-NMS (Bodla et al. 2017) + top-k over the candidate lists, one launch; same outputs as
+    :func:`nms_topk` with the decayed scores.  ``method``: ``"linear"`` (``iou_thr`` is Nt) or ``"gaussian"`` (``sigma``)."""
+    code = _soft_method(method)
+    dev = cand.count.device
+    if out is None:
+        out = (torch.empty((batch,), dtype=torch.int64, device=dev), torch.empty((batch, k), dtype=torch.float32, device=dev),
+               torch.empty((batch, k), dtype=torch.int64, device=dev), torch.empty((batch, k, 4), dtype=torch.float32, device=dev))
+    need = int(_lib().sihl_od_soft_nms_workspace_bytes(int(batch), cand.capacity))
+    ws = None
+    if need:
+        ws = getattr(cand, "_soft_ws", None)
+        if ws is None or ws.numel() < need:
+            ws = torch.empty((need,), dtype=torch.uint8, device=dev)
+            cand._soft_ws = ws
+    with _on(dev):
+        rc = _lib().sihl_od_soft_nms_topk(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
+                                          code, float(iou_thr), float(sigma), float(score_thr), int(k), _p(out[0]), _p(out[1]),
+                                          _p(out[2]), _p(out[3]), _p(ws), int(reset_counts), _stream(dev))
+    _native.check(rc, "sihl_od_soft_nms_topk")
+    return out
+
+
 def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, levels, img_w: int, img_h: int,
                       score_thr: float = 0.05, iou_thr: float = 0.5, max_instances: int = 100,
-                      cand: Optional[CandidateBuffers] = None, mode: str = "dense", split_nms: Optional[bool] = None):
+                      cand: Optional[CandidateBuffers] = None, mode: str = "dense", split_nms: Optional[bool] = None,
+                      nms: str = "hard", sigma: float = 0.5):
     """Extension (no reference counterpart): dense decode of every location + class-aware NMS.
     Output format of ``ObjectDetection.forward`` (ref :122), zero padded past ``num_instances``.
     ``mode``: see :func:`dense_decode` (identical results).  ``split_nms``: class-split NMS (default: whenever the
-    lists can hold more than ``SPLIT_NMS_FROM`` candidates)."""
+    lists can hold more than ``SPLIT_NMS_FROM`` candidates).  ``nms``: ``"hard"`` (greedy, torchvision's semantics),
+    ``"soft_linear"`` (Soft-NMS with ``iou_thr`` as Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``); the soft
+    methods keep decaying scores down to ``score_thr`` and ignore ``split_nms``."""
+    if nms not in NMS_KINDS:
+        raise ValueError(f"nms={nms!r}: expected one of {NMS_KINDS}")
     B, A = loc_logits.shape
     offsets, scales, _ = anchor_tables(levels, img_w, img_h, loc_logits.device)
     if cand is None:
         cand = CandidateBuffers.allocate(B, A, loc_logits.device)
     dense_decode(loc_logits, cls_logits, box_raw, offsets, scales, img_w, img_h, score_thr, cand, mode=mode)
+    if nms != "hard":
+        return soft_nms_topk(cand, B, nms[len("soft_"):], iou_thr, sigma, score_thr, max_instances)
     if split_nms is None:
         # The list lengths are only known on the device, so the choice goes by what can happen: big images (>= 896^2)
         # can yield many thousands of candidates, which one CTA per image would serialise on a few SMs; with many
@@ -673,6 +716,46 @@ def batched_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: floa
     if single:
         return keep[: int(count.item())]
     return keep[:N], count
+
+
+def batched_soft_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, max_output: int, method="gaussian",
+                     iou_threshold: float = 0.3, sigma: float = 0.5, score_threshold: float = 0.001,
+                     seg_offsets: Optional[Tensor] = None):
+    """Class-aware Soft-NMS with :func:`batched_nms`'s inputs: the kept indices in selection order and their decayed
+    scores, at most ``max_output`` per segment.  ``method``: ``"linear"`` (``iou_threshold`` is Nt) or ``"gaussian"``
+    (``sigma``).  Boxes whose score is below ``score_threshold``, or decays below it, are dropped.
+
+    With ``seg_offsets`` (int32 ``[n_images+1]``) returns ``(keep [N] i64, keep_scores [N] f32, keep_count [n_images]
+    i32)``, segment s at ``[seg_offsets[s], seg_offsets[s] + keep_count[s])``; without it, ``(keep, keep_scores)`` of
+    the single segment (one deliberate sync to size the result)."""
+    code = _soft_method(method)
+    if int(max_output) < 1:
+        raise ValueError(f"max_output={max_output}: expected >= 1")
+    boxes = _req(boxes, torch.float32, "boxes", 2)
+    scores = _req(scores, torch.float32, "scores", 1)
+    idxs = _req(idxs, torch.int64, "idxs", 1)
+    dev = boxes.device
+    N = scores.numel()
+    single = seg_offsets is None
+    if single:
+        seg_offsets = torch.tensor([0, N], dtype=torch.int32, device=dev)
+    else:
+        seg_offsets = _req(seg_offsets, torch.int32, "seg_offsets", 1)
+    n_images = seg_offsets.numel() - 1
+    keep = torch.empty((max(N, 1),), dtype=torch.int64, device=dev)
+    keep_scores = torch.empty((max(N, 1),), dtype=torch.float32, device=dev)
+    count = torch.zeros((n_images,), dtype=torch.int32, device=dev)
+    ws_bytes = int(_lib().sihl_od_batched_soft_nms_workspace_bytes(N))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+    with _on(dev):
+        rc = _lib().sihl_od_batched_soft_nms(_p(boxes), _p(scores), _p(idxs), _p(seg_offsets), n_images, N, code,
+                                             float(iou_threshold), float(sigma), float(score_threshold), int(max_output),
+                                             _p(keep), _p(keep_scores), _p(count), _p(ws), _stream(dev))
+    _native.check(rc, "sihl_od_batched_soft_nms")
+    if single:
+        m = int(count.item())
+        return keep[:m], keep_scores[:m]
+    return keep[:N], keep_scores[:N], count
 
 
 # --------------------------------------------------------------------------- N3: matching for the validation mAP
