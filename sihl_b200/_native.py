@@ -99,9 +99,8 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     with _lock:
         if _lib is not None:
             return _lib
-        override = os.environ.get("SIHL_B200_LIB")      # developer builds (e.g. -DSIHL_PHASE_TIMING)
-        path = override or _build.LIB_PATH
-        if build_if_missing and not override:
+        path = _build.LIB_PATH
+        if build_if_missing:
             try:
                 path = _build.build()
             except Exception as exc:                       # nvcc absent or compile error

@@ -31,10 +31,6 @@ NVCC_FLAGS = [
 ]
 
 
-_extra = os.environ.get("SIHL_B200_NVCC_EXTRA", "").split()     # developer experiments (-DSIHL_...); part of the stamp
-NVCC_FLAGS += _extra
-
-
 def _nvcc() -> str:
     exe = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(exe):

@@ -33,9 +33,6 @@ int fill_level_table(const int32_t *level_hw_host, int n_levels, LevelTable *lv)
 // ---------------------------------------------------------------------------
 // Stage 1: select
 // ---------------------------------------------------------------------------
-#ifdef SIHL_PHASE_TIMING
-__device__ unsigned g_sel_dbg[3 * 16384];     // per gt: start (globaltimer ns, low bits), cycles, candidates evaluated
-#endif
 constexpr int kSelWarps = 4;
 constexpr int kSelMinBlocks = 12;     // <= 40 registers: the 1600 CTAs of cfg1 (6400 gts) fit in one wave of 148 x 12
 constexpr int kBufCap = 64;
@@ -120,12 +117,6 @@ k_assign_select(SelectParams p, const float4 *__restrict__ anchors, const float4
     const int g = blockIdx.x * kSelWarps + warp;
     if (g >= total_gt) return;                       // warp-uniform; no block barriers below
 
-#ifdef SIHL_PHASE_TIMING
-    const long long dbg_c0 = clock64();
-    unsigned long long dbg_t0;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(dbg_t0));
-    unsigned dbg_chunks = 0;
-#endif
     unsigned long long *bk = s_key[warp];
     const int topk = p.topk;
     const BoxTerms gt = box_terms(to_box(__ldg(gt_boxes + g)));
@@ -136,9 +127,6 @@ k_assign_select(SelectParams p, const float4 *__restrict__ anchors, const float4
     // The arithmetic is ciou_pair() (od_math.h) cut in three so that a chunk leaves early when no lane
     // can still rank: no overlap => CIoU <= 0; IoU < thr => CIoU < thr (CIoU <= IoU).
     auto consider = [&](bool valid, int a) {
-#ifdef SIHL_PHASE_TIMING
-        ++dbg_chunks;
-#endif
         BoxTerms an;
         an.x1 = an.y1 = an.x2 = an.y2 = an.area = an.cx = an.cy = an.at = 0.f;
         if (valid) {
@@ -264,13 +252,6 @@ k_assign_select(SelectParams p, const float4 *__restrict__ anchors, const float4
         sel_val[(int64_t)g * topk + lane] = lane < cnt ? sel_key_val(mine) : 0.f;
     }
     if (lane == 0) best_iou[g] = cnt ? sel_key_val(mine) : 0.f;      // ref :277 topk_ious[0]
-#ifdef SIHL_PHASE_TIMING
-    if (lane == 0 && g < 16384) {
-        g_sel_dbg[3 * g] = (unsigned)(dbg_t0 & 0xffffffffu);
-        g_sel_dbg[3 * g + 1] = (unsigned)(clock64() - dbg_c0);
-        g_sel_dbg[3 * g + 2] = dbg_chunks;
-    }
-#endif
 }
 
 // Per-anchor terms of the CIoU (box_terms() of od_math.h), cached next to the anchor table.
@@ -285,12 +266,6 @@ __global__ void __launch_bounds__(256) k_anchor_terms(const float4 *__restrict__
 // ---------------------------------------------------------------------------
 // Stage 2: resolve (+ dense losses, + compaction, + fused positive losses)
 // ---------------------------------------------------------------------------
-#ifdef SIHL_PHASE_TIMING
-__device__ long long g_res_phase[8 * 16];
-#define SIHL_RP(i) do { if ((blockIdx.x == 0 || blockIdx.x == 16) && blockIdx.y < 4 && threadIdx.x == 0) g_res_phase[((blockIdx.x ? 4 : 0) + blockIdx.y) * 16 + (i)] = clock64(); } while (0)
-#else
-#define SIHL_RP(i) do { } while (0)
-#endif
 constexpr int kResThreads = 128;
 constexpr int kChunks = kTile / kResThreads;
 constexpr int kResWarps = kResThreads / 32;
@@ -331,7 +306,6 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
     const int b = blockIdx.y, tile = blockIdx.x, n_tiles = gridDim.x;
     const int A = p.num_anchors, a0 = tile * kTile;
     const int na = min(kTile, A - a0);
-    SIHL_RP(0);
     const int g0 = __ldg(p.gt_offsets + b), g1 = __ldg(p.gt_offsets + b + 1);
 
     // issue the streaming loads first: they are independent of the key reduction below
@@ -346,7 +320,6 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
 
     for (int i = tid; i < kTile; i += kResThreads) { s_v[i] = 0u; s_g[i] = 0xffffffffu; }
     __syncthreads();
-    SIHL_RP(1);
     // per anchor: max value over the gts that selected it, ties -> lowest gt (ref :270), as two passes
     // of native 32-bit shared-memory atomics (max of the value bits, then min of the gt among the maxima)
     const int n_entries = (g1 - g0) * p.topk;
@@ -400,7 +373,6 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
         }
     }
     __syncthreads();
-    SIHL_RP(2);
 
     float acc_bce = 0.f, acc_one = 0.f, acc_mse = 0.f, acc_rel = 0.f, acc_pos = 0.f;
     unsigned ballots[kChunks];
@@ -452,7 +424,6 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
         if (want_list && lane == 0) s_seg[c * kResWarps + warp] = __popc(ballots[c]);
     }
 
-    SIHL_RP(3);
     int n_pos = 0;
     if (want_list) {
         // ordered compaction: segment (chunk, warp) order == ascending anchor order (ref :182-184)
@@ -505,13 +476,11 @@ __global__ void __launch_bounds__(kResThreads) k_assign_resolve(ResolveParams p)
         }
     }
 
-    SIHL_RP(4);
     if (p.sums != nullptr && p.loc != nullptr) {
         float v[5] = {acc_bce, acc_one, acc_mse, acc_rel, acc_pos};
         const int slot[5] = {0, 1, 2, 3, 6};
         block_accumulate_f<5>(v, s_red, p.sums, slot);
     }
-    SIHL_RP(5);
 }
 
 // ---------------------------------------------------------------------------
@@ -748,14 +717,3 @@ extern "C" int sihl_od_assign_resolve_t(const int32_t *sel_anchor, const float *
     SIHL_CHECK_LAUNCH("k_assign_resolve");
     return SIHL_OD_OK;
 }
-
-#ifdef SIHL_PHASE_TIMING
-extern "C" __attribute__((visibility("default"))) int sihl_od_debug_resolve(long long *out_host)
-{
-    return cudaMemcpyFromSymbol(out_host, sihl::g_res_phase, sizeof(long long) * 128) == cudaSuccess ? 0 : 2;
-}
-extern "C" __attribute__((visibility("default"))) int sihl_od_debug_select(unsigned *out_host, int n)
-{
-    return cudaMemcpyFromSymbol(out_host, sihl::g_sel_dbg, sizeof(unsigned) * 3 * n) == cudaSuccess ? 0 : 2;
-}
-#endif

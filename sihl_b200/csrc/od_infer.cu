@@ -10,9 +10,7 @@
 //                     _tma  C % 4 == 0, C <= 128: TMA bulk copies into a shared-memory ring
 //                     _v4   C % 4 == 0, larger C: 16-byte loads, 4 or 32 lanes per row
 //                     plain any C: 4-byte loads, 8 lanes per row
-#include <cstdio>
 #include <type_traits>
-#include <cstdlib>
 
 #include "od_common.cuh"
 
@@ -422,7 +420,8 @@ struct StagedCand {
 // Programmatic dependent launch (sm_90+): the scan only READS the maps until its first flush, so a launch made with
 // cudaLaunchAttributeProgrammaticStreamSerialization may start streaming while the previous kernel of the stream (the
 // NMS of the lane's previous step, or the previous scan in a back-to-back loop) is still draining; everything that
-// touches the candidate lists / counters waits for that kernel first.  Both instructions are no-ops in a normal launch.
+// touches the candidate lists / counters waits for that kernel first.  Both instructions are no-ops in a normal launch,
+// which is how the scan is launched: the overlap was measured and does not shorten the pipelined step (DESIGN.md).
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait_prior_grids() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
@@ -862,25 +861,6 @@ extern "C" int sihl_od_decode_rows_t(const float *top_logits, const int64_t *idx
     return SIHL_OD_OK;
 }
 
-// Launch of the TMA scan, optionally (SIHL_DECODE_PDL=1; off by default) as a programmatic dependent launch.  Measured:
-// back-to-back scans then overlap their tails and heads — 400 launches at cfg1 average 24.4 us instead of 30.0 us, i.e.
-// 7.26 TB/s of pure reads, above the 6.47 TB/s copy bandwidth the roofline is quoted against — but that is the
-// throughput of OVERLAPPING launches, not one kernel's duration, and inside the 4-lane pipeline, where other kernels
-// already fill those gaps, the step does not change (41.5 vs 41.6 us).  Kept as an opt-in for single-lane callers.
-template <typename Kern>
-static int launch_scan(Kern kern, int blocks, int threads, size_t smem, cudaStream_t st, const DenseDecodeParams &p, int stages,
-                       int n_chunks)
-{
-    static const bool pdl = []() { const char *e = getenv("SIHL_DECODE_PDL"); return e != nullptr && atoi(e) != 0; }();
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)blocks); cfg.blockDim = dim3((unsigned)threads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    return cuda_status(cudaLaunchKernelEx(&cfg, kern, p, stages, n_chunks), "cudaLaunchKernelEx(k_dense_decode_tma)");
-}
-
 // Argument checks, optional counter zeroing and the parameter block shared by the dense and the
 // candidate-first decode.  Returns 1 when there is nothing to do (batch == 0).
 static int decode_prologue(const float *loc_logits, const float *cls_logits, const float *box_raw, int batch,
@@ -947,8 +927,8 @@ static int launch_decode_tma_half(const DenseDecodeParams &p, int64_t rows, int 
         int rc = cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),  \
                              "cudaFuncSetAttribute(k_dense_decode_tma)");                                         \
         if (rc) return rc;                                                                                        \
-        rc = launch_scan(kern, blocks, THREADS, smem, st, p, stages, n_chunks);                                   \
-        if (rc) return rc;                                                                                        \
+        kern<<<blocks, THREADS, smem, st>>>(p, stages, n_chunks);                                                 \
+        SIHL_CHECK_LAUNCH("k_dense_decode_tma (half maps)");                                                      \
     } while (0)
 #define SIHL_DH(VPL)                                                                                              \
     do {                                                                                                          \
@@ -969,7 +949,6 @@ static int launch_decode_tma_half(const DenseDecodeParams &p, int64_t rows, int 
     }
 #undef SIHL_DH
 #undef SIHL_DH_LAUNCH
-    SIHL_CHECK_LAUNCH("k_dense_decode_tma (half maps)");
     return SIHL_OD_OK;
 }
 
@@ -1013,31 +992,25 @@ extern "C" int sihl_od_dense_decode_t(const void *loc_logits_v, const void *cls_
         // SMALL scans (fewer than ~16 such stages per CTA: the 1024^2 / batch 8 crowd config has 9) are dominated by
         // ring start-up, the last partial round and the end-of-kernel flush: they take 32-row stages on 128-thread
         // CTAs, 3 per SM with 2 stages each — half as long work items (5 % instead of 10 % imbalance in the last round)
-        // and 1.5x the CTAs.  Measured at crowd (tools/decode_sweep.py, profiles/r02_decode_sweep_crowd.json): 18.5 us
-        // with the cfg1 ring, 14.1 us with this one (14.0-14.5 us for every 32-row ring with >= 3 CTAs per SM; this is
-        // the one with the smallest shared-memory footprint, 60 KB per SM).
-        int rows_per_stage = kChunkRows, stages = 2, ctas_per_sm = 2;
-        if ((rows + kChunkRows - 1) / kChunkRows < (int64_t)16 * kNumSMs * 2) { rows_per_stage = 32; stages = 2; ctas_per_sm = 3; }
-        if (const char *e = getenv("SIHL_DECODE_ROWS")) { const int v = atoi(e); if (v == 32 || v == 64) rows_per_stage = v; }
+        // and 1.5x the CTAs.  Measured at crowd (profiles/r02_decode_sweep_crowd.json): 18.5 us with the cfg1 ring,
+        // 14.1 us with this one (14.0-14.5 us for every 32-row ring with >= 3 CTAs per SM; this is the one with the
+        // smallest shared-memory footprint, 60 KB per SM).
+        const int stages = 2;
+        int rows_per_stage = kChunkRows, ctas_per_sm = 2;
+        if ((rows + kChunkRows - 1) / kChunkRows < (int64_t)16 * kNumSMs * 2) { rows_per_stage = 32; ctas_per_sm = 3; }
         const size_t stage_bytes = (size_t)rows_per_stage * num_classes * 4;
-        if (const char *e = getenv("SIHL_DECODE_STAGES")) { const int v = atoi(e); if (v >= 2 && v <= 16 && (size_t)v * stage_bytes < 200 * 1024) stages = v; }
-        if (const char *e = getenv("SIHL_DECODE_CTAS_PER_SM")) { const int v = atoi(e); if (v >= 1 && v <= 8) ctas_per_sm = v; }
-        while ((size_t)stages * stage_bytes * ctas_per_sm > 200 * 1024 && stages > 2) --stages;
         const size_t smem = stages * stage_bytes + stages * sizeof(uint64_t);
         const int n_chunks = (int)((rows + rows_per_stage - 1) / rows_per_stage);
         int blocks = kNumSMs * ctas_per_sm;
         if (blocks > n_chunks) blocks = n_chunks;
-        if (getenv("SIHL_DECODE_DEBUG"))
-            fprintf(stderr, "k_dense_decode_tma: rows/stage %d, stages %d, CTAs/SM %d, grid %d, smem %zu B, chunks %d\n",
-                    rows_per_stage, stages, ctas_per_sm, blocks, smem, n_chunks);
 #define SIHL_DT_LAUNCH(KERN, THREADS)                                                                             \
     do {                                                                                                          \
         auto kern = KERN;                                                                                         \
         int rc = cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),  \
                              "cudaFuncSetAttribute(k_dense_decode_tma)");                                         \
         if (rc) return rc;                                                                                        \
-        rc = launch_scan(kern, blocks, THREADS, smem, st, p, stages, n_chunks);                                   \
-        if (rc) return rc;                                                                                        \
+        kern<<<blocks, THREADS, smem, st>>>(p, stages, n_chunks);                                                 \
+        SIHL_CHECK_LAUNCH("k_dense_decode_tma");                                                                  \
     } while (0)
 #define SIHL_DT(VPL)                                                                                              \
     do {                                                                                                          \
@@ -1149,8 +1122,6 @@ extern "C" int sihl_od_candidate_decode_t(const void *loc_logits_v, const void *
                            "box_raw / cls_logits must be device memory or PINNED host memory (got a pageable host pointer)");
             if (map == cls_logits_v) host = attr.type == cudaMemoryTypeHost;
         }
-        if (const char *e = getenv("SIHL_HOST_ROWS")) host = host && atoi(e) != 0;                            // developer A/B
-        if (const char *e = getenv("SIHL_HOST_CAND")) host = host && atoi(e) != 0;                            // developer A/B (this kernel only)
         // the whole-row reads need 16-byte rows of at most 32 vectors
         const size_t row_bytes = (size_t)num_classes * (map_dtype == SIHL_OD_F32 ? 4 : 2);
         host = host && row_bytes % 16 == 0 && row_bytes <= 32 * 16 && (reinterpret_cast<uintptr_t>(cls_logits_v) & 15u) == 0;

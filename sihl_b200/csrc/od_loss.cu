@@ -8,8 +8,6 @@
 //
 // Sums are accumulated per thread in fp32 over a handful of elements, then in fp64
 // through warp shuffles, one shared-memory hop and one atomicAdd per CTA and term.
-#include <cstdlib>
-
 #include "od_common.cuh"
 #include "od_pos.cuh"
 
@@ -23,13 +21,6 @@ namespace sihl {
 // round trip; the class-logit row was prefetched into L2 by k_assign_resolve.
 // The last CTA to finish may also fold k_loss_finalize in (single-GPU case).
 constexpr int kPosTileThreads = 128;
-#ifdef SIHL_PHASE_TIMING
-__device__ unsigned long long g_pos_blk[4 * 4096];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-#define SIHL_PT(i) do { if (threadIdx.x == 0 && blockIdx.x < 4096) g_pos_blk[4 * blockIdx.x + (i)] = gtimer(); } while (0)
-#else
-#define SIHL_PT(i) do { } while (0)
-#endif
 
 struct PosTileParams {
     const int32_t *pos_chunks; const int32_t *tile_pos_rows; const int2 *tile_pos_aux; int n_tiles; int num_anchors;
@@ -91,9 +82,6 @@ __device__ __noinline__ void exchange_sums(unsigned long long *const *peer, int 
         double *dst = reinterpret_cast<double *>(theirs) + ((size_t)parity * W + rank) * SIHL_OD_NUM_SUMS;
 #pragma unroll
         for (int i = 0; i < SIHL_OD_NUM_SUMS; ++i) dst[i] = s_in[i];
-#ifdef SIHL_EXCHANGE_FENCE
-        __threadfence_system();
-#endif
         // the release store orders THIS thread's eight stores above before the flag at system scope: no separate
         // (and, over NVLink, microsecond-expensive) __threadfence_system() is needed
         st_release_sys(theirs + 16 * W + parity * W + rank, step);
@@ -206,7 +194,6 @@ __global__ void __launch_bounds__(kPosTileThreads, 8) k_pos_loss_tiles(PosTilePa
     __shared__ double s_red[2 * 32];
     __shared__ bool s_last;
     const int tid = threadIdx.x;
-    SIHL_PT(0);
     // the first descriptor is fetched together with the list length (stale entries are harmless: they are
     // only used when blockIdx.x < n_chunks)
     // pos_chunks == NULL: a shard without a single image still takes part in the exchange (it pushes its zero sums)
@@ -379,11 +366,9 @@ __global__ void __launch_bounds__(kPosTileThreads, 8) k_pos_loss_tiles(PosTilePa
         }
     }
     }
-    SIHL_PT(1);
     double v[2] = {acc_box, acc_cls};
     const int slot_idx[2] = {4, 5};
     block_accumulate<2>(v, s_red, p.sums, slot_idx);
-    SIHL_PT(2);
     if (p.losses != nullptr) {                                    // last CTA out computes the five losses
         if (tid == 0) {
             __threadfence();
@@ -402,7 +387,6 @@ __global__ void __launch_bounds__(kPosTileThreads, 8) k_pos_loss_tiles(PosTilePa
             *p.done_counter = 0u;
         }
     }
-    SIHL_PT(3);
 }
 
 __global__ void k_loss_finalize(const double *__restrict__ sums, float *__restrict__ losses)
@@ -493,11 +477,9 @@ extern "C" int sihl_od_pos_loss_tiles_exchange_t(const int32_t *pos_chunks, cons
         if (map == cls_logits) p.host_rows = attr.type == cudaMemoryTypeHost;
     }
     if (!p.cls_vec4) p.host_rows = 0;
-    if (p.host_rows) {                                            // pinned host maps (zero-copy): wider row reads
-        // 2 = whole row per warp instruction (rows of at most 32 vectors), 1 = 8 lanes x 16 B
-        if (p.host_rows && (size_t)num_classes * esz <= 32 * 16) p.host_rows = 2;
-        if (const char *e = getenv("SIHL_HOST_ROWS")) { const int v = atoi(e); if (v >= 0 && v < p.host_rows) p.host_rows = v; }             // developer A/B: 0, 1
-    }
+    // pinned host maps (zero-copy) take wider row reads: 2 = whole row per warp instruction (rows of at most 32
+    // vectors), 1 = 8 lanes x 16 B
+    if (p.host_rows && (size_t)num_classes * esz <= 32 * 16) p.host_rows = 2;
     ExchangeParams x;
     x.world = world; x.rank = rank;
     x.peer = reinterpret_cast<unsigned long long *const *>(peer_regions);
@@ -507,9 +489,7 @@ extern "C" int sihl_od_pos_loss_tiles_exchange_t(const int32_t *pos_chunks, cons
     // fp64 atomics on one 64-byte line + the completion ticket, and ~1800 of those serialise in one L2 slice.  Measured
     // in the cfg1 pipeline (same box A/B): 12 -> 41.6 / 28.2 us per step (dense / candidate-first), 6 -> 40.8 / 25.6,
     // 4 -> 40.6 / 26.0.
-    int per_sm = 6;
-    if (const char *e = getenv("SIHL_POS_TILE_CTAS_PER_SM")) { const int v = atoi(e); if (v >= 1 && v <= 12) per_sm = v; }   // developer A/B
-    const int64_t cap = (int64_t)kNumSMs * per_sm;
+    const int64_t cap = (int64_t)kNumSMs * 6;
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     if (p.host_rows) {
@@ -520,10 +500,3 @@ extern "C" int sihl_od_pos_loss_tiles_exchange_t(const int32_t *pos_chunks, cons
     SIHL_CHECK_LAUNCH("k_pos_loss_tiles");
     return SIHL_OD_OK;
 }
-
-#ifdef SIHL_PHASE_TIMING
-extern "C" __attribute__((visibility("default"))) int sihl_od_debug_pos_blocks(unsigned long long *out_host, int n)
-{
-    return cudaMemcpyFromSymbol(out_host, sihl::g_pos_blk, sizeof(unsigned long long) * 4 * n) == cudaSuccess ? 0 : 2;
-}
-#endif

@@ -33,7 +33,6 @@
 
 #include <cstdint>
 #include <cstdio>
-#include <cstdlib>
 
 #include "../../include/sihl_od.h"
 
@@ -190,19 +189,6 @@ __device__ __forceinline__ void epi_sync() { asm volatile("bar.sync 1, 512;" :::
 
 __host__ __device__ constexpr int tmem_stage_cols(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 128 ? 128 : 256; }
 
-#ifdef SIHL_MLP_TRACE
-// Developer build only (SIHL_B200_NVCC_EXTRA=-DSIHL_MLP_TRACE, tools/mlp_trace.py): CTA 0 records clock64() at the
-// pipeline's hand-over points, 16 slots per tile.
-constexpr int kTraceTiles = 64;
-__device__ long long g_mlp_trace[kTraceTiles * 16];
-#define MLP_TRACE(tile_no, ev)                                                                   \
-    do {                                                                                         \
-        if (blockIdx.x == 0 && (tile_no) < kTraceTiles) g_mlp_trace[(tile_no) * 16 + (ev)] = clock64(); \
-    } while (0)
-#else
-#define MLP_TRACE(tile_no, ev) do { } while (0)
-#endif
-
 template <int N>
 struct MlpSmem {
     static constexpr int kStages = (N == 256) ? 5 : 8;      // N == 256: W takes 128 KB of the 227
@@ -293,7 +279,6 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
                 for (int c = 0; c < kChunks; ++c, ++it) {
                     const uint32_t s = it % S, ph = (it / S) & 1;
                     mbar_wait(&empty[s], ph ^ 1, 0);
-                    MLP_TRACE(it / kChunks, c);                       // 0..3: slot free, chunk c requested
                     mbar_expect_tx(&full[s], kXStageBytes);
                     tma_load_2d(&map_x, &full[s], sX + s * kXStageBytes, c * kChunkK, tile * kBlockM);
                 }
@@ -308,13 +293,11 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
             for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++t) {
                 const uint32_t as = t & 1, aph = (t >> 1) & 1;
                 mbar_wait(&t_empty[as], aph ^ 1, 2);
-                MLP_TRACE(t, 4);                                      // 4: accumulator stage free
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + as * kStageCols;
                 for (int c = 0; c < kChunks; ++c, ++it) {
                     const uint32_t s = it % S, ph = (it / S) & 1;
                     mbar_wait(&full[s], ph, 3);
-                    MLP_TRACE(t, 5 + c);                              // 5..8: chunk c landed, MMAs issued
                     tc_fence_after();
                     const uint32_t a_base = smem_u32(sX + s * kXStageBytes);
                     const uint32_t b_base = smem_u32(sW + c * (N * 128));
@@ -340,7 +323,6 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
         for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++t) {
             const uint32_t as = t & 1, aph = (t >> 1) & 1;
             mbar_wait(&t_full[as], aph, 4);
-            if (warp == 2 && lane == 0) MLP_TRACE(t, 9);              // 9: accumulator complete
             tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + as * kStageCols;
             const long long grow = static_cast<long long>(tile) * kBlockM + row;
@@ -403,7 +385,6 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&t_empty[as]);              // the accumulator stage is free for tile t + 2
-                if (warp == 2 && lane == 0) MLP_TRACE(t, 10);          // 10: accumulator in registers
                 uint64_t x[kPartCols / 2];
                 // statistics of the thread's own 64 columns: x = acc + bias, sum, then the sum of squares about the
                 // LOCAL mean (two passes over registers, no synchronisation in between)
@@ -434,7 +415,6 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
                 stat[(0 * kParts + part) * kBlockM + row] = sum_p;
                 stat[(1 * kParts + part) * kBlockM + row] = (lo_of(q2a) + hi_of(q2a)) + (lo_of(q2b) + hi_of(q2b));
                 epi_sync();
-                if (warp == 2 && lane == 0) MLP_TRACE(t, 11);          // 11: row statistics exchanged
                 float sums[kParts], mean = 0.f, m2 = 0.f;
 #pragma unroll
                 for (int q = 0; q < kParts; ++q) {
@@ -470,9 +450,7 @@ k_mlp_layer(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ C
 #pragma unroll
                     for (int j = 0; j < kPartCols / 2; ++j) packed[j] = bf16x2_of(x[j]);       // kLinear: bias only
                 }
-                if (warp == 2 && lane == 0) MLP_TRACE(t, 13);          // 13: row computed
                 store_rows(packed, reinterpret_cast<__nv_bfloat16*>(p.out), MODE == kLinear);
-                if (warp == 2 && lane == 0) MLP_TRACE(t, 14);          // 14: stores issued
                 continue;                                              // t_empty was signalled right after the load
             } else {
                 uint32_t v[16];
@@ -543,7 +521,7 @@ __global__ void __launch_bounds__(256) k_nchw_to_rows_bf16(const float* __restri
     }
 }
 
-// Backward of LayerNorm + SiLU for the towers' training path: one warp per row, lane = 8 columns.
+// Backward of LayerNorm + SiLU for the towers' training path, lane = 8 columns.
 //   n = (v - mean) rstd, z = n gamma + beta, dz = dy * SiLU'(z), dn = dz gamma,
 //   dv = rstd (dn - mean_j(dn) - n mean_j(dn n));  column sums of dz n, dz, dv = d gamma, d beta, d bias
 // v is the layer's pre-activation (x W^T + b in bf16: kept by the forward, MODE kHiddenPre, or recomputed by the linear mode
@@ -554,100 +532,13 @@ __global__ void __launch_bounds__(256) k_nchw_to_rows_bf16(const float* __restri
 // tower, ref :56, :60), so the upstream gradient is the outer product dy[m,:] = bf16(dout[m]) * w_out[:] (rounded to bf16
 // like the library GEMM it replaces would): read as 4 B per row + one weight row instead of a materialised [M,256] matrix.
 constexpr int kBwdWarps = 8;
-constexpr int kBwdRows = 2;                   // rows per warp and iteration: both rows' loads are in flight before the arithmetic
 __device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
-template <bool RANK1>
-__global__ void __launch_bounds__(kBwdWarps * 32) k_mlp_hidden_bwd_rows(const __nv_bfloat16* __restrict__ v, const __nv_bfloat16* __restrict__ dy,
-                                                                         const float* __restrict__ dout, const __nv_bfloat16* __restrict__ w_out,
-                                                                         const float* __restrict__ row_stats, const float* __restrict__ gamma,
-                                                                         const float* __restrict__ beta, long long M, __nv_bfloat16* __restrict__ dv,
-                                                                         float* __restrict__ partials) {
-    __shared__ float red[kBwdWarps][3][kK];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int c0 = lane * 8;
-    float g[8], be[8], acc_g[8], acc_b[8], acc_v[8], wo[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-        g[j] = gamma[c0 + j]; be[j] = beta[c0 + j]; acc_g[j] = acc_b[j] = acc_v[j] = 0.f;
-        wo[j] = RANK1 ? __bfloat162float(w_out[c0 + j]) : 0.f;
-    }
-    const long long stride = static_cast<long long>(gridDim.x) * kBwdWarps * kBwdRows;
-    for (long long row0 = (static_cast<long long>(blockIdx.x) * kBwdWarps + warp) * kBwdRows; row0 < M; row0 += stride) {
-        uint4 v4[kBwdRows], d4[kBwdRows];
-        float2 st[kBwdRows];
-        float dcol[kBwdRows];
-#pragma unroll
-        for (int r = 0; r < kBwdRows; ++r) {
-            const long long row = row0 + r < M ? row0 + r : M - 1;          // the tail repeats the last row (not stored, not summed)
-            v4[r] = *reinterpret_cast<const uint4*>(v + row * kK + c0);
-            if constexpr (RANK1) { dcol[r] = bf16_round(dout[row]); d4[r] = make_uint4(0, 0, 0, 0); }
-            else { d4[r] = *reinterpret_cast<const uint4*>(dy + row * kK + c0); dcol[r] = 0.f; }
-            st[r] = *reinterpret_cast<const float2*>(row_stats + 2 * row);
-        }
-#pragma unroll
-        for (int r = 0; r < kBwdRows; ++r) {
-            const bool live = row0 + r < M;
-            const uint32_t vw[4] = {v4[r].x, v4[r].y, v4[r].z, v4[r].w}, dw[4] = {d4[r].x, d4[r].y, d4[r].z, d4[r].w};
-            float n[8], dn[8], s1 = 0.f, s2 = 0.f;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float2 vf = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&vw[q]));
-                const float2 df = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&dw[q]));
-                const float up[2] = {RANK1 ? bf16_round(dcol[r] * wo[2 * q]) : df.x, RANK1 ? bf16_round(dcol[r] * wo[2 * q + 1]) : df.y};
-                const float vv[2] = {vf.x, vf.y}, dd[2] = {live ? up[0] : 0.f, live ? up[1] : 0.f};
-#pragma unroll
-                for (int u = 0; u < 2; ++u) {
-                    const int j = 2 * q + u;
-                    n[j] = (vv[u] - st[r].x) * st[r].y;
-                    const float z = __fmaf_rn(n[j], g[j], be[j]);
-                    const float sg = __fmaf_rn(0.5f, tanh_fast(0.5f * z), 0.5f);          // sigmoid(z), one MUFU op
-                    const float dz = dd[u] * (sg * __fmaf_rn(z, 1.f - sg, 1.f));           // dy * SiLU'(z)
-                    acc_g[j] = __fmaf_rn(dz, n[j], acc_g[j]);
-                    acc_b[j] += dz;
-                    dn[j] = dz * g[j];
-                    s1 += dn[j];
-                    s2 = __fmaf_rn(dn[j], n[j], s2);
-                }
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-                s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-            }
-            const float a = s1 * (1.f / kK), b = s2 * (1.f / kK);
-            uint32_t ow[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                float o2[2];
-#pragma unroll
-                for (int u = 0; u < 2; ++u) {
-                    const int j = 2 * q + u;
-                    o2[u] = st[r].y * (dn[j] - a - n[j] * b);
-                    acc_v[j] += o2[u];
-                }
-                const __nv_bfloat162 p2 = __floats2bfloat162_rn(o2[0], o2[1]);
-                ow[q] = *reinterpret_cast<const uint32_t*>(&p2);
-            }
-            if (live) *reinterpret_cast<uint4*>(dv + (row0 + r) * kK + c0) = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-        }
-    }
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { red[warp][0][c0 + j] = acc_g[j]; red[warp][1][c0 + j] = acc_b[j]; red[warp][2][c0 + j] = acc_v[j]; }
-    __syncthreads();
-    for (int i = threadIdx.x; i < 3 * kK; i += kBwdWarps * 32) {
-        float t = 0.f;
-#pragma unroll
-        for (int w = 0; w < kBwdWarps; ++w) t += red[w][i / kK][i % kK];
-        partials[static_cast<long long>(blockIdx.x) * 3 * kK + i] = t;
-    }
-}
 
-// The same backward with the rows streamed through a shared-memory ring by the TMA unit (the default; the register-staged
-// kernel above is kept as the A/B, SIHL_MLP_BWD_RING=0).  k_mlp_hidden_bwd_rows holds ~106 registers per thread, so two
-// CTAs = 16 warps fit on an SM and every warp's loads are exposed once per iteration: measured 200 us per [537 600, 256]
-// layer = 4.1 TB/s for 825 MB.  Here the TMA unit keeps kRingStages x 32 rows of v and dy (one contiguous
-// cp.async.bulk each, completion on an mbarrier) in flight per CTA regardless of what the warps hold in registers;
-// the eight warps take 4 rows each per stage (lane = 8 columns, conflict-free LDS.128) and hand the stage back through an
+// The rows are streamed through a shared-memory ring by the TMA unit.  The register-staged design this replaced (one warp
+// per row, two rows' loads in flight per warp) held ~106 registers per thread, so two CTAs = 16 warps fit on an SM and every
+// warp's loads were exposed once per iteration: measured 200 us per [537 600, 256] layer = 4.1 TB/s for 825 MB.  Here the
+// TMA unit keeps kRingStages x 32 rows of v and dy (one contiguous cp.async.bulk each, completion on an mbarrier) in
+// flight per CTA regardless of what the warps hold in registers; the eight warps take 4 rows each per stage (lane = 8 columns, conflict-free LDS.128) and hand the stage back through an
 // `empty` mbarrier; thread 0 refills a stage at the top of the next iteration (a ninth, dedicated producer warp would cap
 // the kernel at 96 registers per thread and spill).  Row statistics (8 B per row) and, RANK1, dout (4 B per row) are plain broadcast loads one
 // stage ahead.  Same arithmetic, and the same row -> (CTA, warp) order for both variants of RANK1, so they stay bit-equal.
@@ -849,8 +740,8 @@ __global__ void __launch_bounds__(256) k_bf16_to_f32(const uint4* __restrict__ s
 }
 
 // ---- training path of the laterals (1x1 conv + batch-statistics BatchNorm over rows [M,256]) ---------------------------------
-// Backward of the BatchNorm, reductions over ROWS (per channel): same skeleton as k_mlp_hidden_bwd_rows (warp per row,
-// lane = 8 channels, register accumulators, per-CTA partials).
+// Backward of the BatchNorm, reductions over ROWS (per channel): one warp per row, lane = 8 channels, register
+// accumulators, per-CTA partials.
 //   pass 1 (k_bn_bwd_colsums): partials[cta][0][c] = sum_m dz[m,c], partials[cta][1][c] = sum_m dz[m,c] n[m,c]
 //   pass 2 (k_bn_bwd_apply):   dy[m,c] = scale[c] (dz[m,c] - mean_dz[c] - n[m,c] mean_dzn[c])
 // n = (y - mean) invstd is the normalised conv output (recomputed by the caller with the linear mode of the layer kernel).
@@ -1040,22 +931,15 @@ int launch_layer(const void* x, long long M, const void* w, const MlpParams& p_i
     return cudaGetLastError() == cudaSuccess ? SIHL_OD_OK : SIHL_OD_ECUDA;
 }
 
-// Either kernel writes partials[gridDim.x][3][256]; any partial_rows in [1, 8 x SMs] is a valid grid.
+// The kernel writes partials[gridDim.x][3][256]; any partial_rows in [1, 8 x SMs] is a valid grid.
 template <bool RANK1>
 int launch_hidden_bwd(const void* v, const void* dy, const float* dout, const void* w_out, const float* row_stats, const float* gamma,
                              const float* beta, int64_t M, void* dv, float* partials, int partial_rows, cudaStream_t st) {
-    static const bool use_ring = [] { const char* e = getenv("SIHL_MLP_BWD_RING"); return e == nullptr || atoi(e) != 0; }();
-    if (use_ring) {
-        if (cudaFuncSetAttribute(k_mlp_hidden_bwd_ring<RANK1>, cudaFuncAttributeMaxDynamicSharedMemorySize, ring_smem_bytes<RANK1>()) != cudaSuccess)
-            return SIHL_OD_ECUDA;
-        k_mlp_hidden_bwd_ring<RANK1><<<partial_rows, kRingThreads, ring_smem_bytes<RANK1>(), st>>>(
-            static_cast<const __nv_bfloat16*>(v), static_cast<const __nv_bfloat16*>(dy), dout, static_cast<const __nv_bfloat16*>(w_out), row_stats, gamma,
-            beta, M, static_cast<__nv_bfloat16*>(dv), partials);
-    } else {
-        k_mlp_hidden_bwd_rows<RANK1><<<partial_rows, kBwdWarps * 32, 0, st>>>(
-            static_cast<const __nv_bfloat16*>(v), static_cast<const __nv_bfloat16*>(dy), dout, static_cast<const __nv_bfloat16*>(w_out), row_stats, gamma,
-            beta, M, static_cast<__nv_bfloat16*>(dv), partials);
-    }
+    if (cudaFuncSetAttribute(k_mlp_hidden_bwd_ring<RANK1>, cudaFuncAttributeMaxDynamicSharedMemorySize, ring_smem_bytes<RANK1>()) != cudaSuccess)
+        return SIHL_OD_ECUDA;
+    k_mlp_hidden_bwd_ring<RANK1><<<partial_rows, kRingThreads, ring_smem_bytes<RANK1>(), st>>>(
+        static_cast<const __nv_bfloat16*>(v), static_cast<const __nv_bfloat16*>(dy), dout, static_cast<const __nv_bfloat16*>(w_out), row_stats, gamma,
+        beta, M, static_cast<__nv_bfloat16*>(dv), partials);
     return cudaGetLastError() == cudaSuccess ? SIHL_OD_OK : SIHL_OD_ECUDA;
 }
 
@@ -1144,13 +1028,6 @@ SIHL_OD_API int sihl_od_mlp_out(const void* x_bf16, int64_t M, int channels, con
         default: return launch_layer<256, kOutF32>(x_bf16, M, w_bf16, p, st);
     }
 }
-
-#ifdef SIHL_MLP_TRACE
-__attribute__((visibility("default"))) int sihl_od_mlp_debug_trace(long long* host_out, int n) {
-    if (n > kTraceTiles * 16) n = kTraceTiles * 16;
-    return cudaMemcpyFromSymbol(host_out, g_mlp_trace, sizeof(long long) * n) == cudaSuccess ? n : -1;
-}
-#endif
 
 SIHL_OD_API int sihl_od_lateral_rows(const float* x_nchw, int batch, int channels, int64_t hw, void* rows_bf16, void* stream) {
     if (batch < 0 || channels <= 0 || (channels & 63) != 0 || hw < 0 || batch > 65535) return SIHL_OD_EINVAL;

@@ -25,15 +25,6 @@
 
 namespace sihl {
 
-// Developer instrumentation (compiled out unless -DSIHL_PHASE_TIMING): SM clock of block 0 /
-// thread 0 at phase boundaries, read back with sihl_od_debug_phases().
-#ifdef SIHL_PHASE_TIMING
-__device__ long long g_phase_clock[16];
-#define SIHL_PHASE(i) do { if (blockIdx.x == 0 && threadIdx.x == 0) g_phase_clock[i] = clock64(); } while (0)
-#else
-#define SIHL_PHASE(i) do { } while (0)
-#endif
-
 constexpr int kNmsThreads = 1024;
 constexpr int kSmemItems = 4096;          // per-image candidates held on chip
 constexpr int kBigSegment = 512;
@@ -432,7 +423,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
     const int img = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
     const int64_t lb = p.mode == 0 ? list_base(p, img) : 0;
     const int item = tid >> 2, sub = tid & 3;
-    SIHL_PHASE(0);
     int n, src0;
     if (p.mode == 0) {
         const int c = __ldg(p.cand_count + img);
@@ -443,7 +433,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
         n = __ldg(p.seg_offsets + img + 1) - src0;
     }
     if (sel != nullptr) n = n_sel;
-    SIHL_PHASE(1);
     int n_kept = 0;
     if (n > 0) {
         const bool have = item < n;
@@ -475,7 +464,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
             s_keep[item] = 0u; s_dead[item] = 0; s_box[item] = make_float4(0.f, 0.f, 0.f, 0.f); s_area[item] = 0.f;
         }
         __syncthreads();
-        SIHL_PHASE(2);
         // one pass: r = #better keys; seg0 = #smaller classes; k = #better keys of the same class; len = #same class
         int r = 0, seg0 = 0, k = 0, len = 0;
         if (have) {
@@ -509,7 +497,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
             if (len > 32) s_big = 1;
         }
         __syncthreads();
-        SIHL_PHASE(3);
         // suppressor masks: the 4 lanes of a candidate split its earlier same-class boxes
         unsigned mask = 0;
         if (have && len <= 32) {
@@ -521,7 +508,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
         mask |= __shfl_xor_sync(kFullMask, mask, 2);
         if (have && sub == 0) s_mask[q] = mask;
         __syncthreads();
-        SIHL_PHASE(4);
         if (have && sub == 0 && k == 0 && len <= 32) {          // segment leader: greedy pass on bits only
             unsigned kept = 1u;
             for (int i = 1; i < len; ++i)
@@ -545,7 +531,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
             }
             __syncthreads();
         }
-        SIHL_PHASE(5);
         // survivors in rank order
         n_kept = block_ordered_compact(
             n, s_warp,
@@ -568,7 +553,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
                 }
             });
     }
-    SIHL_PHASE(6);
     if (!finalize) return n_kept;
     if (p.mode == 0) {
         const int m = n_kept < p.K ? n_kept : p.K;
@@ -585,7 +569,6 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
     } else if (tid == 0) {
         p.keep_count[img] = n_kept;
     }
-    SIHL_PHASE(7);
     return n_kept;
 }
 
@@ -722,7 +705,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
         return p.mode == 0 ? (unsigned)__ldg(p.cand_cls + lb + i) : (unsigned)__ldg(p.classes + src0 + i);
     };
 
-    SIHL_PHASE(0);
     for (int h = tid; h < kHashSlots; h += blockDim.x) { h_cls[h] = kHashEmpty; h_cnt[h] = 0; }
     if (tid == 0) s_distinct = 0;
     __syncthreads();
@@ -741,7 +723,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
     }
     __syncthreads();
     if (s_distinct > kHashSlots / 2) return false;                // block-uniform
-    SIHL_PHASE(1);
     // 2. exclusive scan of the slot counts (one slot per thread)
     {
         const int c = tid < kHashSlots ? h_cnt[tid] : 0;
@@ -767,7 +748,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
         if (tid < kHashSlots) { h_start[tid] = s_warp[warp] + incl - c; h_cnt[tid] = 0; }     // h_cnt becomes the fill cursor
     }
     __syncthreads();
-    SIHL_PHASE(2);
     // 3. scatter (key, slot) into the class buckets
     for (int i = tid; i < n; i += blockDim.x) {
         const int h = ar.b_id[i];
@@ -776,7 +756,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
         ar.u_slot[pos] = (unsigned)i;
     }
     __syncthreads();
-    SIHL_PHASE(3);
     // 4. rank inside the bucket by counting -> class-major position q; gather the box
     for (int pp = tid; pp < n; pp += blockDim.x) {
         const unsigned long long key = ar.u_key[pp];
@@ -801,7 +780,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
         ar.f_dead[q] = 0;
     }
     __syncthreads();
-    SIHL_PHASE(4);
     // 5. suppression inside each class.  Segments of up to 64 boxes: every box gets the bitmask of the earlier
     //    boxes of its class that overlap it (all pairs in parallel, u_key is free to hold the masks), then one
     //    lane per class runs the greedy chain on bits.  Longer segments: one warp per class, the kept box is
@@ -858,12 +836,10 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
     //    mode 0 needs the K best only -> radix select of the K-th score + rank-by-counting of the few above it;
     //    mode 1 needs all of them     -> rank-by-counting over the survivors (bitonic only beyond 4096 of them).
     //    (Barrier-heavy sorts are slow here: every __syncthreads drains the shared-memory stores of 32 warps.)
-    SIHL_PHASE(5);
     const int n_kept = block_ordered_compact(
         n, s_warp, [&](int q) { return ar.f_dead[q] == 0; },
         [&](int q, int k) { ar.u_key[k] = ar.f_key[q]; ar.u_slot[k] = (unsigned)q; });
     __syncthreads();
-    SIHL_PHASE(6);
     auto emit = [&](int k_src, int rank) {                       // survivor k_src goes to output position rank
         const unsigned q = ar.u_slot[k_src], slot = ar.f_slot[q];
         if (p.mode == 0) {
@@ -958,8 +934,6 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
             if (rank < want) emit((int)pass_src[r], rank);
         }
     }
-    SIHL_PHASE(7);
-    SIHL_PHASE(8);
     *n_kept_out = n_kept;
     return true;
 }
@@ -1240,13 +1214,6 @@ extern "C" int sihl_od_batched_nms(const float *boxes, const float *scores, cons
     p.workspace = static_cast<unsigned char *>(workspace); p.ws_stride = 0;
     return launch_nms(p, n_images, n, (cudaStream_t)stream);
 }
-
-#ifdef SIHL_PHASE_TIMING
-extern "C" __attribute__((visibility("default"))) int sihl_od_debug_phases(long long *out_host)
-{
-    return cudaMemcpyFromSymbol(out_host, sihl::g_phase_clock, sizeof(long long) * 16) == cudaSuccess ? 0 : 2;
-}
-#endif
 
 // ---- class-split variant (long lists) ------------------------------------------------------------------
 static int split_factor(int64_t cand_capacity)

@@ -81,10 +81,7 @@ class DetectionHeadPipeline:
         self.tile_pos_aux = torch.zeros((B * n_tiles * tile, 2), dtype=torch.int32, device=dev)
         self.done_counter = torch.zeros((1,), dtype=torch.int32, device=dev)
         self.cand = ops.CandidateBuffers.allocate(B, int(cand_capacity or A), dev)
-        # the inference chain's stream; SIHL_SIDE_PRIORITY (developer A/B): CUDA stream priority of that chain
-        import os
-        prio = os.environ.get("SIHL_SIDE_PRIORITY")
-        self.side = torch.cuda.Stream(device=dev) if prio is None else torch.cuda.Stream(device=dev, priority=int(prio))
+        self.side = torch.cuda.Stream(device=dev)                 # the inference chain's stream
         self.lib = _native.load()
         self._exchange = None
 

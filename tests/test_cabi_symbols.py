@@ -30,6 +30,21 @@ def test_every_declared_symbol_is_exported_and_bound():
     assert sorted(_native.EXPORTED_SYMBOLS) == declared, "ctypes signatures and header disagree"
 
 
+def test_library_reads_no_environment_variables():
+    """Which kernel and grid an entry launches depends on its arguments alone, never on the process environment."""
+    import shutil
+    import subprocess
+
+    import pytest
+    nm = shutil.which("nm")
+    if nm is None:
+        pytest.skip("nm not found")
+    path = build.build()
+    out = subprocess.run([nm, "-D", "--undefined-only", path], capture_output=True, text=True, check=True).stdout
+    imported = {line.split()[-1].split("@")[0] for line in out.splitlines() if line.strip()}
+    assert not {name for name in imported if "getenv" in name}
+
+
 def test_argument_errors_do_not_need_a_gpu():
     lib = _native.load()
     # n_levels out of range is rejected on the host, before any CUDA call
