@@ -401,7 +401,9 @@ SIHL_OD_API int sihl_od_candidate_decode_t(const void *loc_logits, const void *c
  * (ops/boxes.py:102-120): visit by (score desc, location asc); a kept box
  * suppresses later boxes of the same class with IoU > iou_thr.  Emits the first
  * K kept detections per image, zero padded, in the reference forward()'s output
- * format.  workspace: sihl_od_nms_workspace_bytes(batch, cand_capacity).
+ * format.  workspace: sihl_od_nms_workspace_bytes(batch, cand_capacity) bytes (0 up to 256
+ * candidates per image; NULL is then accepted): lists longer than 256 keep their working
+ * arrays there, not in shared memory, so that the kernel fits on an SM beside the dense scan.
  * reset_counts != 0: cand_count[b] is zeroed once consumed, so the next
  * sihl_od_dense_decode needs no zeroing launch.
  * Precondition: the sort keys of a list are DISTINCT (every location listed at most once per image — what the decode

@@ -5,7 +5,7 @@
 // inter / (area_i + area_j - inter) > thr.
 //
 // k_nms: one CTA per image (segment), sort-free, the list length (known only on the device) picks the body:
-//   * n <= 256 (nms_small_body): 4 lanes per candidate; ONE counting pass over the list gives every candidate its
+//   * n <= 256 (nms_small_body): 2 (top-K entry) or 4 lanes per candidate; ONE counting pass over the list gives every candidate its
 //     rank (score desc, index asc), its class-major position and its class segment; suppression bitmasks per
 //     candidate against the earlier boxes of its class (all pairs in parallel), greedy chain on bits.
 //   * top-K entry with n > 256 and K <= 128 (lazy prefix): greedy NMS is prefix-closed — whether a box is kept
@@ -16,20 +16,27 @@
 //     rank by counting inside the class, 64-bit suppression masks for classes <= 64 boxes, 32-box chunks (all
 //     pairs of a chunk in parallel by shuffles, then the chunk's kept boxes against the rest) by one warp per
 //     class up to 2048 boxes and by the whole CTA beyond, top-K by radix select of the K-th score; arrays in
-//     shared memory up to 4096 candidates, in the global workspace beyond.
+//     shared memory up to 4096 candidates, in the global workspace beyond (the top-K entry: always the workspace).
 //   * more than 512 distinct classes (nms_big_body): the two-bitonic-sort fallback — sort by rank, sort by
 //     (class, rank), per-segment suppression, ordered compaction.
+// Footprint: the top-K entry runs next to the dense scan of the other steps in flight (two 256-thread scan CTAs per SM,
+// 16 384 registers and ~46 KB of shared memory each).  Its CTA (k_nms<kNmsThreadsTopk>) therefore stays within half the
+// register file (512 threads x <= 64 registers) and reserves no dynamic shared memory: its long-list arrays live in the
+// per-image workspace (small and L2-resident), and the short-list body needs only the ~27 KB of static shared memory.
+// The stand-alone entries (segment-mode batched NMS, the class-split sub-lists) run with 1024 threads and keep their
+// long-list arrays on chip: with 512 threads and the workspace, batched NMS of 1 000-5 000 boxes took 8-63 % longer.
+// tests/test_kernel_footprint.py checks the top-K budget on the built library.
 // sihl_od_nms_topk_split deals an image's candidates to several CTAs by class; stand-alone batched NMS of
 // 8192..90000 boxes takes the multi-CTA bitmask path of od_nms_wide.cu (whole GPU) instead of one CTA.
 #include "od_common.cuh"
 
 namespace sihl {
 
-constexpr int kNmsThreads = 1024;
+constexpr int kNmsThreadsTopk = 512;     // the top-K entry (beside the dense scan)
+constexpr int kNmsThreadsAlone = 1024;   // the stand-alone entries
 constexpr int kSmemItems = 4096;          // per-image candidates held on chip
 constexpr int kBigSegment = 512;
 constexpr int kSmallItems = 256;          // lists up to this size take the single-pass rank-sort kernel
-static_assert(4 * kSmallItems == kNmsThreads, "short-list path: four lanes per candidate");
 constexpr size_t kSmemItemBytes = 47;     // dynamic shared memory per on-chip candidate: max over the two long-list layouts (41, 47)
 constexpr size_t kWsItemBytes = 48;       // workspace stride per item (keeps every image 16-B aligned)
 
@@ -397,7 +404,7 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
     }
 }
 
-// Short lists (n <= kSmallItems, the common case after a 0.05 score threshold).  Four lanes per
+// Short lists (n <= kSmallItems, the common case after a 0.05 score threshold).  THREADS / 256 lanes per
 // candidate; ONE counting pass over shared memory yields, per candidate, its rank r in
 // (score desc, index asc) order, its class-major position q, and the start / length of its
 // class segment.  Suppression is then a per-candidate bitmask of earlier same-class boxes with
@@ -407,8 +414,11 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
 // `sel` (optional, shared memory): the body runs on the n_sel candidates lb + sel[0..n_sel) instead of the whole list
 // (lazy top-K prefix).  Returns the number of survivors; with finalize == false the per-image epilogue
 // (num_instances, zero padding, counter reset) is left to the caller.
+template <int THREADS>
 __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel = nullptr, int n_sel = 0, bool finalize = true)
 {
+    constexpr int kLanes = THREADS / kSmallItems;
+    static_assert(kLanes * kSmallItems == THREADS && (kLanes == 2 || kLanes == 4), "short-list path: 2 or 4 lanes per candidate");
     __shared__ unsigned long long s_key[kSmallItems];
     __shared__ unsigned s_cls[kSmallItems];        // by slot
     __shared__ float4 s_box[kSmallItems];          // by q
@@ -422,7 +432,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
 
     const int img = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
     const int64_t lb = p.mode == 0 ? list_base(p, img) : 0;
-    const int item = tid >> 2, sub = tid & 3;
+    const int item = tid / kLanes, sub = tid % kLanes;
     int n, src0;
     if (p.mode == 0) {
         const int c = __ldg(p.cand_count + img);
@@ -468,7 +478,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
         int r = 0, seg0 = 0, k = 0, len = 0;
         if (have) {
 #pragma unroll 4
-            for (int j = sub; j < n; j += 4) {
+            for (int j = sub; j < n; j += kLanes) {
                 const unsigned long long kj = s_key[j];
                 const unsigned cj = s_cls[j];
                 const bool better = kj > key, same = cj == cls;
@@ -479,7 +489,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
             }
         }
 #pragma unroll
-        for (int o = 2; o > 0; o >>= 1) {
+        for (int o = kLanes / 2; o > 0; o >>= 1) {
             r += __shfl_xor_sync(kFullMask, r, o);
             seg0 += __shfl_xor_sync(kFullMask, seg0, o);
             k += __shfl_xor_sync(kFullMask, k, o);
@@ -497,15 +507,15 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
             if (len > 32) s_big = 1;
         }
         __syncthreads();
-        // suppressor masks: the 4 lanes of a candidate split its earlier same-class boxes
+        // suppressor masks: the lanes of a candidate split its earlier same-class boxes
         unsigned mask = 0;
         if (have && len <= 32) {
             const float area = (bx.z - bx.x) * (bx.w - bx.y);
-            for (int j = sub; j < k; j += 4)
+            for (int j = sub; j < k; j += kLanes)
                 if (iou_gt(s_box[seg0 + j], s_area[seg0 + j], bx, area, p.iou_thr)) mask |= 1u << j;
         }
-        mask |= __shfl_xor_sync(kFullMask, mask, 1);
-        mask |= __shfl_xor_sync(kFullMask, mask, 2);
+#pragma unroll
+        for (int o = kLanes / 2; o > 0; o >>= 1) mask |= __shfl_xor_sync(kFullMask, mask, o);
         if (have && sub == 0) s_mask[q] = mask;
         __syncthreads();
         if (have && sub == 0 && k == 0 && len <= 32) {          // segment leader: greedy pass on bits only
@@ -682,7 +692,7 @@ __device__ __forceinline__ MedArrays carve_med(unsigned char *base, int n_al)
 
 // SMEM: the arrays are in shared memory (tells the compiler the address space: generic loads from shared are
 // several times slower than LDS and do not pipeline in the counting loops).
-template <bool SMEM>
+template <bool SMEM, int THREADS>
 __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int src0, unsigned char *base, int n_al,
                                                 int *s_warp, unsigned *h_cls, int *h_cnt, int *h_start, ChunkScratch *chunk_scratch,
                                                 int *n_kept_out)
@@ -723,9 +733,13 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
     }
     __syncthreads();
     if (s_distinct > kHashSlots / 2) return false;                // block-uniform
-    // 2. exclusive scan of the slot counts (one slot per thread)
+    // 2. exclusive scan of the slot counts (kSlotsPerThread consecutive slots per thread)
     {
-        const int c = tid < kHashSlots ? h_cnt[tid] : 0;
+        constexpr int kSlotsPerThread = kHashSlots / THREADS;
+        static_assert(kSlotsPerThread * THREADS == kHashSlots, "hash slots split evenly over the threads");
+        int cs[kSlotsPerThread], c = 0;
+#pragma unroll
+        for (int j = 0; j < kSlotsPerThread; ++j) { cs[j] = h_cnt[kSlotsPerThread * tid + j]; c += cs[j]; }
         int incl = c;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
@@ -745,7 +759,13 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
             s_warp[lane] = wi - x;
         }
         __syncthreads();
-        if (tid < kHashSlots) { h_start[tid] = s_warp[warp] + incl - c; h_cnt[tid] = 0; }     // h_cnt becomes the fill cursor
+        int run = s_warp[warp] + incl - c;
+#pragma unroll
+        for (int j = 0; j < kSlotsPerThread; ++j) {                 // h_cnt becomes the fill cursor
+            h_start[kSlotsPerThread * tid + j] = run;
+            h_cnt[kSlotsPerThread * tid + j] = 0;
+            run += cs[j];
+        }
     }
     __syncthreads();
     // 3. scatter (key, slot) into the class buckets
@@ -939,7 +959,8 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
 }
 
 // One launch for every path: the list length (known only on the device) picks the body.
-__global__ void __launch_bounds__(kNmsThreads) k_nms(NmsParams p)
+template <int THREADS>   // <= 64 registers per thread either way: 512 threads take half the register file
+__global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
 {
     extern __shared__ __align__(16) unsigned char s_dyn_top[];
     __shared__ int s_warp_top[33];
@@ -955,7 +976,7 @@ __global__ void __launch_bounds__(kNmsThreads) k_nms(NmsParams p)
         src0 = __ldg(p.seg_offsets + blockIdx.x);
         n = __ldg(p.seg_offsets + blockIdx.x + 1) - src0;
     }
-    if (n <= kSmallItems) { nms_small_body(p); return; }
+    if (n <= kSmallItems) { nms_small_body<THREADS>(p); return; }
     if (p.mode == 0 && p.K <= kLazyMaxK) {
         // top-K of a long list: try the highest-ranked ~200 candidates first (exact: see the file header)
         __shared__ int s_sel[kSmallItems];
@@ -964,7 +985,7 @@ __global__ void __launch_bounds__(kNmsThreads) k_nms(NmsParams p)
         const int64_t lb = list_base(p, (int)blockIdx.x);
         const int m = lazy_prefix_select(p, lb, n, s_sel, reinterpret_cast<unsigned *>(s_hcnt), s_pick, &s_count);
         if (m > 0) {
-            const int kept = nms_small_body(p, s_sel, m, false);
+            const int kept = nms_small_body<THREADS>(p, s_sel, m, false);
             if (kept >= p.K) {                             // the K best survivors are all inside the prefix: done
                 if (threadIdx.x == 0) {
                     p.num_instances[blockIdx.x] = p.K;
@@ -980,10 +1001,10 @@ __global__ void __launch_bounds__(kNmsThreads) k_nms(NmsParams p)
     int n_kept = 0;
     bool done;
     if (n_al <= p.smem_items) {
-        done = nms_medium_body<true>(p, n, src0, s_dyn_top, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
+        done = nms_medium_body<true, THREADS>(p, n, src0, s_dyn_top, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
     } else {
         unsigned char *ws = list_workspace(p, (int)blockIdx.x, src0);
-        done = nms_medium_body<false>(p, n, src0, ws, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
+        done = nms_medium_body<false, THREADS>(p, n, src0, ws, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
     }
     if (done) {
         const int img = blockIdx.x, tid = threadIdx.x;
@@ -1127,20 +1148,22 @@ static int pow2ceil(int64_t n)
     return p;
 }
 
-static int launch_nms(NmsParams p, int n_images, int64_t max_items, cudaStream_t st, int smem_items = kSmemItems)
+// smem_items: candidates per list whose long-list arrays the launch keeps in dynamic shared memory (0: none, every long
+// list uses the workspace).  Dynamic shared memory is reserved only when a list can exceed the short-list path.
+template <int THREADS>
+static int launch_nms(NmsParams p, int n_images, int64_t max_items, cudaStream_t st, int smem_items)
 {
-    // dynamic shared memory only when a list can exceed the short-list path
     p.smem_items = smem_items;
     const size_t smem = max_items > kSmallItems ? (size_t)smem_items * kSmemItemBytes : 0;
     static thread_local bool attr_set = false;
     if (smem && !attr_set) {
-        int rc = cuda_status(cudaFuncSetAttribute(k_nms, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        int rc = cuda_status(cudaFuncSetAttribute(k_nms<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                   (int)((size_t)kSmemItems * kSmemItemBytes)),
                              "cudaFuncSetAttribute(k_nms)");
         if (rc) return rc;
         attr_set = true;
     }
-    k_nms<<<n_images, kNmsThreads, smem, st>>>(p);
+    k_nms<THREADS><<<n_images, THREADS, smem, st>>>(p);
     SIHL_CHECK_LAUNCH("k_nms");
     return SIHL_OD_OK;
 }
@@ -1153,7 +1176,7 @@ extern "C" size_t sihl_od_nms_workspace_bytes(int batch, int64_t cand_capacity)
 {
     if (batch <= 0 || cand_capacity <= 0) return 0;
     const int np = pow2ceil(cand_capacity);
-    if (np <= kSmemItems) return 0;
+    if (np <= kSmallItems) return 0;                           // every list fits the short-list body
     return (size_t)batch * (size_t)np * kWsItemBytes;
 }
 
@@ -1177,7 +1200,8 @@ extern "C" int sihl_od_nms_topk(const int32_t *cand_count, int64_t cand_capacity
     p.out_boxes = reinterpret_cast<float4 *>(boxes);
     p.workspace = static_cast<unsigned char *>(workspace);
     p.ws_stride = (size_t)pow2ceil(cand_capacity) * kWsItemBytes;
-    return launch_nms(p, batch, cand_capacity, (cudaStream_t)stream);
+    // runs next to the dense scan of the neighbouring steps: no dynamic shared memory (see the file header)
+    return launch_nms<kNmsThreadsTopk>(p, batch, cand_capacity, (cudaStream_t)stream, 0);
 }
 
 namespace sihl {                 // od_nms_wide.cu: the multi-CTA bitmask path for one long list
@@ -1212,7 +1236,7 @@ extern "C" int sihl_od_batched_nms(const float *boxes, const float *scores, cons
     p.boxes = reinterpret_cast<const float4 *>(boxes); p.scores = scores; p.classes = classes; p.seg_offsets = seg_offsets;
     p.mode = 1; p.iou_thr = iou_thr; p.keep = keep; p.keep_count = keep_count;
     p.workspace = static_cast<unsigned char *>(workspace); p.ws_stride = 0;
-    return launch_nms(p, n_images, n, (cudaStream_t)stream);
+    return launch_nms<kNmsThreadsAlone>(p, n_images, n, (cudaStream_t)stream, kSmemItems);
 }
 
 // ---- class-split variant (long lists) ------------------------------------------------------------------
@@ -1277,7 +1301,7 @@ extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity
     p.num_instances = sub_num; p.out_scores = sub_scores; p.out_classes = sub_classes; p.out_boxes = sub_boxes;
     p.out_keys = sub_keys; p.workspace = nms_ws; p.ws_stride = 0;
     // sub-lists rarely exceed 2048 candidates: half the shared memory per CTA lets two of them share an SM
-    int rc = launch_nms(p, batch * S, cand_capacity, st, kSmemItems / 2);
+    int rc = launch_nms<kNmsThreadsAlone>(p, batch * S, cand_capacity, st, kSmemItems / 2);
     if (rc) return rc;
     MergeParams mp;
     mp.S = S; mp.K = k; mp.sub_num = sub_num; mp.sub_keys = sub_keys; mp.sub_scores = sub_scores; mp.sub_classes = sub_classes;
