@@ -586,7 +586,6 @@ struct TrainWorkspace {
     int32_t *sel_anchor; float *sel_val; float *best_iou; int32_t *tile_pos_count; int32_t *tile_pos_rows;
     size_t bytes;
 };
-inline size_t align_up(size_t v) { return (v + 255) & ~(size_t)255; }
 TrainWorkspace carve_train_workspace(void *base, int batch, int64_t num_anchors, int gt_capacity, int topk)
 {
     const size_t n_tiles = (size_t)((num_anchors + kTile - 1) / kTile);
@@ -594,11 +593,11 @@ TrainWorkspace carve_train_workspace(void *base, int batch, int64_t num_anchors,
     unsigned char *b = reinterpret_cast<unsigned char *>(base);
     size_t o = 0;
     TrainWorkspace w;
-    w.sel_anchor = reinterpret_cast<int32_t *>(b + o); o += align_up(gk * 4);
-    w.sel_val = reinterpret_cast<float *>(b + o); o += align_up(gk * 4);
-    w.best_iou = reinterpret_cast<float *>(b + o); o += align_up((size_t)(gt_capacity > 0 ? gt_capacity : 0) * 4);
-    w.tile_pos_count = reinterpret_cast<int32_t *>(b + o); o += align_up((size_t)batch * n_tiles * 4);
-    w.tile_pos_rows = reinterpret_cast<int32_t *>(b + o); o += align_up((size_t)batch * n_tiles * kTile * 4);
+    w.sel_anchor = reinterpret_cast<int32_t *>(b + o); o += round_up_256(gk * 4);
+    w.sel_val = reinterpret_cast<float *>(b + o); o += round_up_256(gk * 4);
+    w.best_iou = reinterpret_cast<float *>(b + o); o += round_up_256((size_t)(gt_capacity > 0 ? gt_capacity : 0) * 4);
+    w.tile_pos_count = reinterpret_cast<int32_t *>(b + o); o += round_up_256((size_t)batch * n_tiles * 4);
+    w.tile_pos_rows = reinterpret_cast<int32_t *>(b + o); o += round_up_256((size_t)batch * n_tiles * kTile * 4);
     w.bytes = o;
     return w;
 }

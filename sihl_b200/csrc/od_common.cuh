@@ -40,6 +40,14 @@ constexpr int kNumSMs = 148;          // B200
 constexpr unsigned kFullMask = 0xffffffffu;
 constexpr int kTile = 512;            // anchors per CTA of k_assign_resolve == capacity of one tile's positive list
 
+// v rounded up to a multiple of 256 bytes: the alignment of every array carved out of a workspace.
+size_t round_up_256(size_t v);
+
+// The class / box maps may be device memory or pinned host memory read in place over PCIe; pageable host memory would
+// fault in the kernel.  Returns SIHL_OD_EINVAL (error text set) when a map is pageable host memory, SIHL_OD_OK
+// otherwise, and sets *cls_host to whether cls_logits is pinned host memory.  A NULL map is skipped.
+int classify_maps(const void *cls_logits, const void *box_raw, bool *cls_host);
+
 struct LevelTable {                   // passed by value as a kernel parameter
     int n;
     int h[SIHL_OD_MAX_LEVELS];
@@ -160,14 +168,43 @@ template <> __device__ __forceinline__ void st_vec16<__nv_bfloat16>(__nv_bfloat1
 
 __device__ __forceinline__ Box4 to_box(float4 b) { return Box4{b.x, b.y, b.z, b.w}; }
 
-// IoU of two xyxy boxes with the operator order of od_nms.cu's iou_gt (torchvision's CPU nms kernel):
-// inter / ((area_a + area_b) - inter), areas as (x2 - x1) * (y2 - y1).  NaN when both boxes have zero area.
+// Order-preserving map fp32 -> uint32 (ascending) and its inverse.
+__device__ __forceinline__ unsigned f2ord(float f)
+{
+    const unsigned u = __float_as_uint(f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float ord2f(unsigned k)
+{
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// IoU of two xyxy boxes with the operator order of torchvision's CPU nms kernel
+// (torchvision/csrc/ops/cpu/nms_kernel.cpp: ovr = inter / (iarea + areas[j] - inter)),
+// areas as (x2 - x1) * (y2 - y1).  NaN when both boxes have zero area.
 __device__ __forceinline__ float box_iou(float4 a, float area_a, float4 b, float area_b)
 {
     const float w = fmaxf(0.f, fminf(a.z, b.z) - fmaxf(a.x, b.x));
     const float h = fmaxf(0.f, fminf(a.w, b.w) - fmaxf(a.y, b.y));
     const float inter = w * h;
     return inter / ((area_a + area_b) - inter);
+}
+
+// torchvision's NMS suppression test: ovr > thr (false for a NaN overlap)
+__device__ __forceinline__ bool iou_gt(float4 a, float area_a, float4 b, float area_b, float thr)
+{
+    return box_iou(a, area_a, b, area_b) > thr;
+}
+
+// Shared-memory address and mbarrier set-up of the TMA rings (od_infer.cu, od_mlp.cu).
+__device__ __forceinline__ uint32_t smem_u32(const void *ptr) { return (uint32_t)__cvta_generic_to_shared(ptr); }
+__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
+{
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 
 template <typename T>

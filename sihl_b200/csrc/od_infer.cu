@@ -6,7 +6,7 @@
 //   k_dense_decode* extension: the same per-location decode over ALL locations of the
 //                   dense maps + score threshold, feeding class-aware NMS (od_nms.cu).
 //                   This is the HBM-bound kernel of the path: 4*A*(C+5) B per image are read
-//                   exactly once.  Three variants, picked by sihl_od_dense_decode():
+//                   exactly once.  Three variants, picked by sihl_od_dense_decode_t():
 //                     _tma  C % 4 == 0, C <= 128: TMA bulk copies into a shared-memory ring
 //                     _v4   C % 4 == 0, larger C: 16-byte loads, 4 or 32 lanes per row
 //                     plain any C: 4-byte loads, 8 lanes per row
@@ -15,17 +15,6 @@
 #include "od_common.cuh"
 
 namespace sihl {
-
-// Order-preserving map fp32 -> uint32 (ascending).
-__device__ __forceinline__ unsigned f2ord(float f)
-{
-    const unsigned u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(unsigned k)
-{
-    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
 
 // ---------------------------------------------------------------------------
 // top-K of one row per CTA: 4-pass MSB radix select for the K-th largest value, one
@@ -159,23 +148,13 @@ k_topk(const T *__restrict__ loc, int A, int K, int KP /* pow2 >= K */, int64_t 
 // Lane gl visits c = gl, gl+8, ...; strict '>' keeps the lowest index inside a lane and
 // the cross-lane reduction prefers the lower index on equal values (torch.max, ref :117).
 // ---------------------------------------------------------------------------
-template <int CPL>   // logits per lane when C == 8*CPL (fully unrolled, all loads in flight); 0 = runtime C
 __device__ __forceinline__ int row_argmax8(const float *__restrict__ z, int C, int gl)
 {
-    float best = -CUDART_INF_F;
     int arg = 0x7fffffff;
-    if (CPL > 0) {
-        float v[CPL > 0 ? CPL : 1];
-#pragma unroll
-        for (int i = 0; i < CPL; ++i) v[i] = __ldcs(z + gl + 8 * i);      // streamed once: evict-first
-#pragma unroll
-        for (int i = 0; i < CPL; ++i)
-            if (v[i] > best || arg == 0x7fffffff) { best = v[i]; arg = gl + 8 * i; }
-    } else {
-        for (int c = gl; c < C; c += 8) {
-            const float x = __ldcs(z + c);
-            if (x > best || arg == 0x7fffffff) { best = x; arg = c; }
-        }
+    float best = -CUDART_INF_F;
+    for (int c = gl; c < C; c += 8) {
+        const float x = __ldcs(z + c);                                      // streamed once: evict-first
+        if (x > best || arg == 0x7fffffff) { best = x; arg = c; }
     }
 #pragma unroll
     for (int o = 4; o > 0; o >>= 1) {
@@ -276,7 +255,6 @@ __device__ __forceinline__ void emit_candidate(const DenseDecodeParams &p, int64
 }
 
 // Scalar variant (any C): 8 lanes per row, 4-byte loads.
-template <int CPL>
 __global__ void __launch_bounds__(256) k_dense_decode(DenseDecodeParams p)
 {
     const int gl = threadIdx.x & 7;
@@ -289,7 +267,7 @@ __global__ void __launch_bounds__(256) k_dense_decode(DenseDecodeParams p)
         const bool ok = row < rows;
         const int64_t rr = ok ? row : rows - 1;
         const float x = __ldcs(p.loc + rr);
-        const int arg = row_argmax8<CPL>(p.cls + rr * p.C, p.C, gl);
+        const int arg = row_argmax8(p.cls + rr * p.C, p.C, gl);
         if (ok && gl == 0) emit_candidate(p, row, x, arg);
     }
 }
@@ -353,24 +331,14 @@ __global__ void __launch_bounds__(256) k_dense_decode_v4(DenseDecodeParams p)
 // Bulk-async variant (C % 4 == 0, C <= 128): the class-logit map is streamed through shared
 // memory by the TMA unit — cp.async.bulk of 64 consecutive rows (64*C*4 B, contiguous in
 // HBM) + their 64 location logits per stage, completion signalled on an mbarrier — in a
-// ring of kStages stages per CTA, persistent CTAs striding over the chunks.  Bytes in flight
-// are set by the ring (2 CTAs x 4 stages x 20 KB per SM at C = 80), not by what the compiler
-// keeps in registers, and every byte is read from HBM exactly once.  Consumers: 4 lanes per
-// row, conflict-free LDS.128, first-argmax as above.
+// ring of stages per CTA, persistent CTAs striding over the chunks.  Bytes in flight are set
+// by the ring (its shape: launch_decode_tma), not by what the compiler keeps in registers,
+// and every byte is read from HBM exactly once.  Consumers: 4 lanes per row, conflict-free
+// LDS.128, first-argmax as above.
 // ---------------------------------------------------------------------------
 constexpr int kChunkRows = 64;             // rows per ring stage of the default variant == rows one pass of a 256-thread CTA covers
-                                           // (4 lanes per row); small scans use 32-row stages on 128-thread CTAs (see the entry point)
+                                           // (4 lanes per row); small scans use 32-row stages on 128-thread CTAs (launch_decode_tma)
 
-__device__ __forceinline__ uint32_t smem_u32(const void *ptr) { return (uint32_t)__cvta_generic_to_shared(ptr); }
-
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
 // Streamed exactly once: tag the lines evict-first so the scan does not push the L2-resident working set of the
 // concurrently running kernels (anchor tables, selections, candidate and positive lists) out of the 126 MB L2.
 __device__ __forceinline__ uint64_t l2_evict_first_policy()
@@ -477,7 +445,7 @@ __device__ __forceinline__ void flush_staged(const DenseDecodeParams &p, const S
 
 // T: element type of the three maps.  Half maps put ROWS x C x 2 bytes into a stage (half the HBM traffic); a lane then
 // owns 16-byte vectors of EIGHT logits (VPL counts those).
-template <int VPL, bool EXACT, int ROWS = kChunkRows, typename T = float>     // ROWS per stage; the CTA has 4 * ROWS threads
+template <int VPL, bool EXACT, int ROWS, typename T>     // ROWS per stage; the CTA has 4 * ROWS threads
 __global__ void __launch_bounds__(4 * ROWS) k_dense_decode_tma(DenseDecodeParams p, int stages, int n_chunks)
 {
     constexpr int kPerVec = 16 / (int)sizeof(T);
@@ -863,7 +831,7 @@ extern "C" int sihl_od_decode_rows_t(const float *top_logits, const int64_t *idx
 
 // Argument checks, optional counter zeroing and the parameter block shared by the dense and the
 // candidate-first decode.  Returns 1 when there is nothing to do (batch == 0).
-static int decode_prologue(const float *loc_logits, const float *cls_logits, const float *box_raw, int batch,
+static int decode_prologue(const void *loc_logits, const void *cls_logits, const void *box_raw, int batch,
                            int64_t num_anchors, int num_classes, const float *offsets, const float *scales,
                            int img_w, int img_h, float score_thr, int32_t *cand_count, int64_t cand_capacity,
                            uint64_t *cand_key, float *cand_box, int32_t *cand_cls, int zero_counts, cudaStream_t st,
@@ -882,7 +850,8 @@ static int decode_prologue(const float *loc_logits, const float *cls_logits, con
         SIHL_CHECK_LAUNCH("k_zero_i32");
     }
     DenseDecodeParams &p = *out;
-    p.loc = loc_logits; p.cls = cls_logits; p.box_raw = box_raw; p.batch = batch; p.A = (int)num_anchors; p.C = num_classes;
+    p.loc = static_cast<const float *>(loc_logits); p.cls = static_cast<const float *>(cls_logits);
+    p.box_raw = static_cast<const float *>(box_raw); p.batch = batch; p.A = (int)num_anchors; p.C = num_classes;
     p.offsets = reinterpret_cast<const float4 *>(offsets); p.scales = reinterpret_cast<const float4 *>(scales);
     p.img_w = (float)img_w; p.img_h = (float)img_h; p.score_thr = score_thr;
     {   // logit(thr) minus a safety margin: only saves the exp for the bulk of the rows
@@ -906,135 +875,92 @@ extern "C" int sihl_od_dense_decode(const float *loc_logits, const float *cls_lo
                                   stream);
 }
 
-// Half maps: the TMA ring with 2-byte elements (C % 8 == 0, C <= 256, 16-byte aligned maps).
+// The TMA ring over `rows` rows of T maps (fp32: C % 4 == 0, C <= 128; half: C % 8 == 0, C <= 256).  Its shape, measured
+// on B200:
+//   * 2 stages x 2 CTAs per SM of 64-row stages: the fp32 kernel is already at the HBM roof with ~87 KB in flight per SM
+//     (3 and 4 stages give the same 32 us), and the smaller ring leaves ~120 KB of shared memory per SM to the kernels
+//     of the other chain / the neighbouring step running concurrently.  Half maps have half-size stages: twice as many
+//     (4) keep the same bytes in flight.
+//   * SMALL scans (fewer than ~16 such stages per CTA: the 1024^2 / batch 8 crowd config has 9) are dominated by ring
+//     start-up, the last partial round and the end-of-kernel flush: they take 32-row stages on 128-thread CTAs, 3 per
+//     SM with 2 stages each — half as long work items (5 % instead of 10 % imbalance in the last round) and 1.5x the
+//     CTAs.  Measured at crowd (profiles/r02_decode_sweep_crowd.json): 18.5 us with the cfg1 ring, 14.1 us with this
+//     one (14.0-14.5 us for every 32-row ring with >= 3 CTAs per SM; this is the one with the smallest shared-memory
+//     footprint, 60 KB per SM).
 template <typename T>
-static int launch_decode_tma_half(const DenseDecodeParams &p, int64_t rows, int num_classes, cudaStream_t st)
+static int launch_decode_tma(const DenseDecodeParams &p, int64_t rows, cudaStream_t st)
 {
-    const int cv = num_classes / 8;
-    const int vpl = (cv + 3) / 4;
+    const int cv = p.C / (16 / (int)sizeof(T));                    // 16-byte vectors per row
+    int vpl = (cv + 3) / 4;                                        // per lane, 4 lanes per row
+    if (sizeof(T) == 2 && vpl > 4) vpl = 8;                        // half maps: kernels for 1-4 and 8 vectors per lane
     const bool exact = vpl * 4 == cv;
-    int rows_per_stage = kChunkRows, stages = 2, ctas_per_sm = 2;
-    if ((rows + kChunkRows - 1) / kChunkRows < (int64_t)16 * kNumSMs * 2) { rows_per_stage = 32; stages = 2; ctas_per_sm = 3; }
-    else { stages = 4; }                                   // half-size stages: twice as many keep the same bytes in flight
-    const size_t stage_bytes = (size_t)rows_per_stage * num_classes * sizeof(T);
-    const size_t smem = stages * stage_bytes + stages * sizeof(uint64_t);
+    const bool small = (rows + kChunkRows - 1) / kChunkRows < (int64_t)16 * kNumSMs * 2;
+    const int rows_per_stage = small ? 32 : kChunkRows;
+    const int stages = small || sizeof(T) == 4 ? 2 : 4;
+    const int ctas_per_sm = small ? 3 : 2;
+    const size_t smem = stages * ((size_t)rows_per_stage * p.C * sizeof(T) + sizeof(uint64_t));
     const int n_chunks = (int)((rows + rows_per_stage - 1) / rows_per_stage);
     int blocks = kNumSMs * ctas_per_sm;
     if (blocks > n_chunks) blocks = n_chunks;
-#define SIHL_DH_LAUNCH(KERN, THREADS)                                                                             \
-    do {                                                                                                          \
-        auto kern = KERN;                                                                                         \
-        int rc = cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),  \
-                             "cudaFuncSetAttribute(k_dense_decode_tma)");                                         \
-        if (rc) return rc;                                                                                        \
-        kern<<<blocks, THREADS, smem, st>>>(p, stages, n_chunks);                                                 \
-        SIHL_CHECK_LAUNCH("k_dense_decode_tma (half maps)");                                                      \
-    } while (0)
-#define SIHL_DH(VPL)                                                                                              \
-    do {                                                                                                          \
-        if (rows_per_stage == 64) {                                                                               \
-            if (exact) SIHL_DH_LAUNCH((k_dense_decode_tma<VPL, true, 64, T>), 256);                               \
-            else SIHL_DH_LAUNCH((k_dense_decode_tma<VPL, false, 64, T>), 256);                                    \
-        } else {                                                                                                  \
-            if (exact) SIHL_DH_LAUNCH((k_dense_decode_tma<VPL, true, 32, T>), 128);                               \
-            else SIHL_DH_LAUNCH((k_dense_decode_tma<VPL, false, 32, T>), 128);                                    \
-        }                                                                                                         \
-    } while (0)
+    auto launch = [&](auto kern) -> int {
+        int rc = cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
+                             "cudaFuncSetAttribute(k_dense_decode_tma)");
+        if (rc) return rc;
+        kern<<<blocks, 4 * rows_per_stage, smem, st>>>(p, stages, n_chunks);
+        SIHL_CHECK_LAUNCH("k_dense_decode_tma");
+        return SIHL_OD_OK;
+    };
+    auto launch_vpl = [&](auto vpl_c) -> int {
+        constexpr int V = decltype(vpl_c)::value;
+        if (small) return exact ? launch(k_dense_decode_tma<V, true, 32, T>) : launch(k_dense_decode_tma<V, false, 32, T>);
+        return exact ? launch(k_dense_decode_tma<V, true, 64, T>) : launch(k_dense_decode_tma<V, false, 64, T>);
+    };
     switch (vpl) {
-        case 1: SIHL_DH(1); break;
-        case 2: SIHL_DH(2); break;
-        case 3: SIHL_DH(3); break;
-        case 4: SIHL_DH(4); break;
-        default: SIHL_DH(8); break;
+        case 1: return launch_vpl(std::integral_constant<int, 1>());
+        case 2: return launch_vpl(std::integral_constant<int, 2>());
+        case 3: return launch_vpl(std::integral_constant<int, 3>());
+        case 4: return launch_vpl(std::integral_constant<int, 4>());
     }
-#undef SIHL_DH
-#undef SIHL_DH_LAUNCH
-    return SIHL_OD_OK;
+    if constexpr (sizeof(T) == 4) {
+        switch (vpl) {
+            case 5: return launch_vpl(std::integral_constant<int, 5>());
+            case 6: return launch_vpl(std::integral_constant<int, 6>());
+            case 7: return launch_vpl(std::integral_constant<int, 7>());
+        }
+    }
+    return launch_vpl(std::integral_constant<int, 8>());
 }
 
-extern "C" int sihl_od_dense_decode_t(const void *loc_logits_v, const void *cls_logits_v, const void *box_raw_v, int map_dtype,
+extern "C" int sihl_od_dense_decode_t(const void *loc_logits, const void *cls_logits, const void *box_raw, int map_dtype,
                                       int batch, int64_t num_anchors, int num_classes, const float *offsets,
                                       const float *scales, int img_w, int img_h, float score_thr, int32_t *cand_count,
                                       int64_t cand_capacity, uint64_t *cand_key, float *cand_box, int32_t *cand_cls,
                                       int zero_counts, void *stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
-    const float *loc_logits = reinterpret_cast<const float *>(loc_logits_v), *cls_logits = reinterpret_cast<const float *>(cls_logits_v);
-    const float *box_raw = reinterpret_cast<const float *>(box_raw_v);
     DenseDecodeParams p;
     int nothing = 0;
     int rc0 = decode_prologue(loc_logits, cls_logits, box_raw, batch, num_anchors, num_classes, offsets, scales, img_w, img_h,
                               score_thr, cand_count, cand_capacity, cand_key, cand_box, cand_cls, zero_counts, st, &p, &nothing);
     if (rc0 || nothing) return rc0;
+    const int64_t rows = (int64_t)batch * num_anchors;
     if (map_dtype != SIHL_OD_F32) {
         SIHL_CHECK_ARG(map_dtype == SIHL_OD_F16 || map_dtype == SIHL_OD_BF16, "map dtype code %d", map_dtype);
-        const bool ok = num_classes % 8 == 0 && num_classes <= 256 && (int64_t)batch * num_anchors >= 4 * kChunkRows &&
-                        ((reinterpret_cast<uintptr_t>(cls_logits_v) | reinterpret_cast<uintptr_t>(box_raw_v)) & 15u) == 0;
+        const bool ok = num_classes % 8 == 0 && num_classes <= 256 && rows >= 4 * kChunkRows &&
+                        ((reinterpret_cast<uintptr_t>(cls_logits) | reinterpret_cast<uintptr_t>(box_raw)) & 15u) == 0;
         SIHL_CHECK_ARG(ok, "the dense scan of half maps needs C %% 8 == 0, C <= 256, >= 256 rows and 16-byte aligned maps "
                            "(C=%d): use sihl_od_candidate_decode_t", num_classes);
         // scores are sigmoid() rounded to the map type and may cross the threshold from below: widen the pre-filter
         if (p.logit_thr > -HUGE_VALF && p.logit_thr < HUGE_VALF) p.logit_thr -= 0.05f * (1.f + fabsf(p.logit_thr));
-        const int64_t rows_h = (int64_t)batch * num_anchors;
-        if (map_dtype == SIHL_OD_F16) return launch_decode_tma_half<__half>(p, rows_h, num_classes, st);
-        return launch_decode_tma_half<__nv_bfloat16>(p, rows_h, num_classes, st);
+        if (map_dtype == SIHL_OD_F16) return launch_decode_tma<__half>(p, rows, st);
+        return launch_decode_tma<__nv_bfloat16>(p, rows, st);
     }
-    const int64_t rows = (int64_t)batch * num_anchors;
     const bool aligned = (num_classes % 4 == 0) && ((reinterpret_cast<uintptr_t>(cls_logits) & 15u) == 0) &&
                          ((reinterpret_cast<uintptr_t>(box_raw) & 15u) == 0);
     const int c4 = num_classes / 4;
     const bool loc_aligned = (reinterpret_cast<uintptr_t>(loc_logits) & 15u) == 0;
-    if (aligned && loc_aligned && c4 <= 32 && rows >= 4 * kChunkRows) {
-        const int vpl = (c4 + 3) / 4;
-        const bool exact = vpl * 4 == c4;
-        // 2 stages x 2 CTAs per SM of 64-row stages: measured on B200 the kernel is already at the HBM roof with ~87 KB
-        // in flight per SM (3 and 4 stages give the same 32 us), and the smaller ring leaves ~120 KB of shared
-        // memory per SM to the kernels of the other chain / the neighbouring step running concurrently.
-        // SMALL scans (fewer than ~16 such stages per CTA: the 1024^2 / batch 8 crowd config has 9) are dominated by
-        // ring start-up, the last partial round and the end-of-kernel flush: they take 32-row stages on 128-thread
-        // CTAs, 3 per SM with 2 stages each — half as long work items (5 % instead of 10 % imbalance in the last round)
-        // and 1.5x the CTAs.  Measured at crowd (profiles/r02_decode_sweep_crowd.json): 18.5 us with the cfg1 ring,
-        // 14.1 us with this one (14.0-14.5 us for every 32-row ring with >= 3 CTAs per SM; this is the one with the
-        // smallest shared-memory footprint, 60 KB per SM).
-        const int stages = 2;
-        int rows_per_stage = kChunkRows, ctas_per_sm = 2;
-        if ((rows + kChunkRows - 1) / kChunkRows < (int64_t)16 * kNumSMs * 2) { rows_per_stage = 32; ctas_per_sm = 3; }
-        const size_t stage_bytes = (size_t)rows_per_stage * num_classes * 4;
-        const size_t smem = stages * stage_bytes + stages * sizeof(uint64_t);
-        const int n_chunks = (int)((rows + rows_per_stage - 1) / rows_per_stage);
-        int blocks = kNumSMs * ctas_per_sm;
-        if (blocks > n_chunks) blocks = n_chunks;
-#define SIHL_DT_LAUNCH(KERN, THREADS)                                                                             \
-    do {                                                                                                          \
-        auto kern = KERN;                                                                                         \
-        int rc = cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),  \
-                             "cudaFuncSetAttribute(k_dense_decode_tma)");                                         \
-        if (rc) return rc;                                                                                        \
-        kern<<<blocks, THREADS, smem, st>>>(p, stages, n_chunks);                                                 \
-        SIHL_CHECK_LAUNCH("k_dense_decode_tma");                                                                  \
-    } while (0)
-#define SIHL_DT(VPL)                                                                                              \
-    do {                                                                                                          \
-        if (rows_per_stage == 64) {                                                                               \
-            if (exact) SIHL_DT_LAUNCH((k_dense_decode_tma<VPL, true, 64>), 256);                                  \
-            else SIHL_DT_LAUNCH((k_dense_decode_tma<VPL, false, 64>), 256);                                       \
-        } else {                                                                                                  \
-            if (exact) SIHL_DT_LAUNCH((k_dense_decode_tma<VPL, true, 32>), 128);                                  \
-            else SIHL_DT_LAUNCH((k_dense_decode_tma<VPL, false, 32>), 128);                                       \
-        }                                                                                                         \
-    } while (0)
-        switch (vpl) {
-            case 1: SIHL_DT(1); break;
-            case 2: SIHL_DT(2); break;
-            case 3: SIHL_DT(3); break;
-            case 4: SIHL_DT(4); break;
-            case 5: SIHL_DT(5); break;
-            case 6: SIHL_DT(6); break;
-            case 7: SIHL_DT(7); break;
-            default: SIHL_DT(8); break;
-        }
-#undef SIHL_DT
-#undef SIHL_DT_LAUNCH
-    } else if (aligned && c4 <= 32 * 8) {
+    if (aligned && loc_aligned && c4 <= 32 && rows >= 4 * kChunkRows) return launch_decode_tma<float>(p, rows, st);
+    if (aligned && c4 <= 32 * 8) {
         // 4 lanes per row up to C = 128, a full warp per row beyond; grid = 4 resident CTAs per SM
         const int lpr = c4 <= 32 ? 4 : 32;
         int64_t blocks = (rows * lpr / 2 + 255) / 256;
@@ -1074,7 +1000,7 @@ extern "C" int sihl_od_dense_decode_t(const void *loc_logits_v, const void *cls_
         const int64_t cap = (int64_t)kNumSMs * 8;          // 8 resident CTAs of 256 threads per SM
         if (blocks > cap) blocks = cap;
         const dim3 grid((unsigned)(blocks < 1 ? 1 : blocks));
-        k_dense_decode<0><<<grid, 256, 0, st>>>(p);
+        k_dense_decode<<<grid, 256, 0, st>>>(p);
     }
     SIHL_CHECK_LAUNCH("k_dense_decode");
     return SIHL_OD_OK;
@@ -1091,15 +1017,13 @@ extern "C" int sihl_od_candidate_decode(const float *loc_logits, const float *cl
                                       zero_counts, stream);
 }
 
-extern "C" int sihl_od_candidate_decode_t(const void *loc_logits_v, const void *cls_logits_v, const void *box_raw_v, int map_dtype,
+extern "C" int sihl_od_candidate_decode_t(const void *loc_logits, const void *cls_logits, const void *box_raw, int map_dtype,
                                           int batch, int64_t num_anchors, int num_classes, const float *offsets,
                                           const float *scales, int img_w, int img_h, float score_thr, int32_t *cand_count,
                                           int64_t cand_capacity, uint64_t *cand_key, float *cand_box, int32_t *cand_cls,
                                           int zero_counts, void *stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
-    const float *loc_logits = reinterpret_cast<const float *>(loc_logits_v), *cls_logits = reinterpret_cast<const float *>(cls_logits_v);
-    const float *box_raw = reinterpret_cast<const float *>(box_raw_v);
     DenseDecodeParams p;
     int nothing = 0;
     int rc0 = decode_prologue(loc_logits, cls_logits, box_raw, batch, num_anchors, num_classes, offsets, scales, img_w, img_h,
@@ -1113,19 +1037,11 @@ extern "C" int sihl_od_candidate_decode_t(const void *loc_logits_v, const void *
     const bool vec = (num_classes % 4 == 0) && ((reinterpret_cast<uintptr_t>(cls_logits) & 15u) == 0);
     SIHL_CHECK_ARG((reinterpret_cast<uintptr_t>(box_raw) & 15u) == 0, "box_raw must be 16-byte aligned");
     bool host = false;                                             // pinned host maps (zero-copy)
-    {
-        const void *host_ok_maps[2] = {cls_logits_v, box_raw_v};
-        for (const void *map : host_ok_maps) {       // pageable host memory would fault in the kernel: refuse it here
-            cudaPointerAttributes attr;
-            if (cudaPointerGetAttributes(&attr, map) != cudaSuccess) { (void)cudaGetLastError(); continue; }
-            SIHL_CHECK_ARG(attr.type != cudaMemoryTypeUnregistered,
-                           "box_raw / cls_logits must be device memory or PINNED host memory (got a pageable host pointer)");
-            if (map == cls_logits_v) host = attr.type == cudaMemoryTypeHost;
-        }
-        // the whole-row reads need 16-byte rows of at most 32 vectors
-        const size_t row_bytes = (size_t)num_classes * (map_dtype == SIHL_OD_F32 ? 4 : 2);
-        host = host && row_bytes % 16 == 0 && row_bytes <= 32 * 16 && (reinterpret_cast<uintptr_t>(cls_logits_v) & 15u) == 0;
-    }
+    const int rc = classify_maps(cls_logits, box_raw, &host);
+    if (rc) return rc;
+    // the whole-row reads need 16-byte rows of at most 32 vectors
+    const size_t row_bytes = (size_t)num_classes * (map_dtype == SIHL_OD_F32 ? 4 : 2);
+    host = host && row_bytes % 16 == 0 && row_bytes <= 32 * 16 && (reinterpret_cast<uintptr_t>(cls_logits) & 15u) == 0;
     if (map_dtype == SIHL_OD_F32) {
         if (host) k_candidate_decode<4, float, true><<<(unsigned)blocks, 256, 0, st>>>(p);
         else if (vec) k_candidate_decode<4><<<(unsigned)blocks, 256, 0, st>>>(p);

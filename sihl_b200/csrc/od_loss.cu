@@ -466,17 +466,10 @@ extern "C" int sihl_od_pos_loss_tiles_exchange_t(const int32_t *pos_chunks, cons
     p.cls_vec4 = (((size_t)num_classes * esz) % 16 == 0) && ((reinterpret_cast<uintptr_t>(cls_logits) & 15u) == 0);
     SIHL_CHECK_ARG(box_raw == nullptr || (reinterpret_cast<uintptr_t>(box_raw) & (4 * esz - 1)) == 0, "box_raw rows must be aligned");
     p.sums = sums; p.losses = losses; p.done_counter = done_counter;
-    p.host_rows = 0;
-    const void *host_ok_maps[2] = {cls_logits, box_raw};
-    for (const void *map : host_ok_maps) {               // pageable host memory would fault in the kernel: refuse it here
-        cudaPointerAttributes attr;
-        if (map == nullptr) continue;
-        if (cudaPointerGetAttributes(&attr, map) != cudaSuccess) { (void)cudaGetLastError(); continue; }
-        SIHL_CHECK_ARG(attr.type != cudaMemoryTypeUnregistered,
-                       "box_raw / cls_logits must be device memory or PINNED host memory (got a pageable host pointer)");
-        if (map == cls_logits) p.host_rows = attr.type == cudaMemoryTypeHost;
-    }
-    if (!p.cls_vec4) p.host_rows = 0;
+    bool cls_host = false;
+    const int rc = classify_maps(cls_logits, box_raw, &cls_host);
+    if (rc) return rc;
+    p.host_rows = cls_host && p.cls_vec4;
     // pinned host maps (zero-copy) take wider row reads: 2 = whole row per warp instruction (rows of at most 32
     // vectors), 1 = 8 lanes x 16 B
     if (p.host_rows && (size_t)num_classes * esz <= 32 * 16) p.host_rows = 2;

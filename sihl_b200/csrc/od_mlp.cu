@@ -34,9 +34,13 @@
 #include <cstdint>
 #include <cstdio>
 
-#include "../../include/sihl_od.h"
+#include "od_common.cuh"
 
 namespace {
+
+using sihl::mbar_expect_tx;
+using sihl::mbar_init;
+using sihl::smem_u32;
 
 constexpr int kK = 256;                       // in_features of every tower layer (the reference's num_channels default)
 constexpr int kBlockM = 128;                  // rows per tile = TMEM lanes
@@ -48,14 +52,6 @@ constexpr int kThreads = 576;                 // warp 0: TMA producer, warp 1: M
 constexpr int kParts = 4;                     // epilogue warps per TMEM lane quarter of a hidden layer
 constexpr int kPartCols = 64;                 // columns each of them owns (held in registers for the whole epilogue)
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }

@@ -40,12 +40,6 @@ constexpr int kSmallItems = 256;          // lists up to this size take the sing
 constexpr size_t kSmemItemBytes = 47;     // dynamic shared memory per on-chip candidate: max over the two long-list layouts (41, 47)
 constexpr size_t kWsItemBytes = 48;       // workspace stride per item (keeps every image 16-B aligned)
 
-__device__ __forceinline__ unsigned f2ord_nms(float f)
-{
-    const unsigned u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 struct NmsArrays {
     unsigned long long *key;   // [np] sort keys; after step 2: (class << 32 | r) by q
     float4 *box;               // [np] by q
@@ -119,15 +113,6 @@ __device__ __forceinline__ int block_ordered_compact(int n, int *s_warp /* [33] 
         __syncthreads();
     }
     return running;
-}
-
-// torchvision/csrc/ops/cpu/nms_kernel.cpp: ovr = inter / (iarea + areas[j] - inter); ovr > thr
-__device__ __forceinline__ bool iou_gt(float4 a, float area_a, float4 b, float area_b, float thr)
-{
-    const float w = fmaxf(0.f, fminf(a.z, b.z) - fmaxf(a.x, b.x));
-    const float h = fmaxf(0.f, fminf(a.w, b.w) - fmaxf(a.y, b.y));
-    const float inter = w * h;
-    return inter / ((area_a + area_b) - inter) > thr;
 }
 
 __device__ __forceinline__ float4 shfl4(float4 v, int src)
@@ -296,7 +281,7 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
             unsigned long long key = 0ull;
             if (i < n) {
                 if (p.mode == 0) key = __ldg(p.cand_key + lb + i);
-                else key = ((unsigned long long)f2ord_nms(__ldg(p.scores + src0 + i)) << 32) |
+                else key = ((unsigned long long)f2ord(__ldg(p.scores + src0 + i)) << 32) |
                            (unsigned long long)(0xffffffffu - (unsigned)i);
             }
             ar.key[i] = key;
@@ -456,7 +441,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
                 cls = (unsigned)__ldg(p.cand_cls + lb + src);
                 bx = __ldg(p.cand_box + lb + src);
             } else {
-                key = ((unsigned long long)f2ord_nms(__ldg(p.scores + src0 + item)) << 32) |
+                key = ((unsigned long long)f2ord(__ldg(p.scores + src0 + item)) << 32) |
                       (unsigned long long)(0xffffffffu - (unsigned)item);
                 cls = (unsigned)__ldg(p.classes + src0 + item);
                 bx = __ldg(p.boxes + src0 + item);
@@ -709,7 +694,7 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
 
     auto key_of = [&](int i) -> unsigned long long {
         if (p.mode == 0) return __ldg(p.cand_key + lb + i);
-        return ((unsigned long long)f2ord_nms(__ldg(p.scores + src0 + i)) << 32) | (unsigned long long)(0xffffffffu - (unsigned)i);
+        return ((unsigned long long)f2ord(__ldg(p.scores + src0 + i)) << 32) | (unsigned long long)(0xffffffffu - (unsigned)i);
     };
     auto cls_of = [&](int i) -> unsigned {
         return p.mode == 0 ? (unsigned)__ldg(p.cand_cls + lb + i) : (unsigned)__ldg(p.classes + src0 + i);
@@ -1248,18 +1233,16 @@ static int split_factor(int64_t cand_capacity)
     return (int)s;
 }
 
-static size_t align256(size_t x) { return (x + 255) / 256 * 256; }
-
 extern "C" size_t sihl_od_nms_split_workspace_bytes(int batch, int64_t cand_capacity, int k)
 {
     if (batch <= 0 || cand_capacity <= 0 || k <= 0) return 0;
     const size_t S = (size_t)split_factor(cand_capacity), B = (size_t)batch, cap = (size_t)cand_capacity, K = (size_t)k;
     size_t bytes = 0;
-    bytes += align256(B * cap * 8) + align256(B * cap * 16) + align256(B * cap * 4);          // key2, box2, cls2
-    bytes += 2 * align256(B * S * 4);                                                         // sub_count, sub_offset
-    bytes += align256(B * S * 8) + align256(B * S * K * 8) + align256(B * S * K * 4) + align256(B * S * K * 8) +
-             align256(B * S * K * 16);                                                        // per-sub-list outputs
-    bytes += align256((size_t)(2 * B * cap + 2) * kWsItemBytes);                              // k_nms workspace for long sub-lists
+    bytes += round_up_256(B * cap * 8) + round_up_256(B * cap * 16) + round_up_256(B * cap * 4);      // key2, box2, cls2
+    bytes += 2 * round_up_256(B * S * 4);                                                             // sub_count, sub_offset
+    bytes += round_up_256(B * S * 8) + round_up_256(B * S * K * 8) + round_up_256(B * S * K * 4) + round_up_256(B * S * K * 8) +
+             round_up_256(B * S * K * 16);                                                            // per-sub-list outputs
+    bytes += round_up_256((size_t)(2 * B * cap + 2) * kWsItemBytes);                                  // k_nms workspace for long sub-lists
     return bytes;
 }
 
@@ -1276,7 +1259,7 @@ extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity
     const int S = split_factor(cand_capacity);
     const size_t B = (size_t)batch, cap = (size_t)cand_capacity, K = (size_t)k;
     unsigned char *w = static_cast<unsigned char *>(workspace);
-    auto take = [&](size_t bytes) { unsigned char *ptr = w; w += align256(bytes); return ptr; };
+    auto take = [&](size_t bytes) { unsigned char *ptr = w; w += round_up_256(bytes); return ptr; };
     SplitParams sp;
     sp.cand_count = cand_count; sp.cap = cand_capacity;
     sp.key = reinterpret_cast<const unsigned long long *>(cand_key); sp.box = reinterpret_cast<const float4 *>(cand_box);

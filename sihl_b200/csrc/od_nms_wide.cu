@@ -41,15 +41,13 @@ struct WideBuffers {
     size_t bytes;
 };
 
-static size_t wide_align(size_t v) { return (v + 255) & ~(size_t)255; }
-
 static WideBuffers carve_wide(void *base, int64_t n)
 {
     WideBuffers w;
     unsigned char *b = reinterpret_cast<unsigned char *>(base);
     size_t o = 0;
     const size_t N = (size_t)n;
-    auto take = [&](size_t bytes) { unsigned char *ptr = b + o; o += wide_align(bytes); return ptr; };
+    auto take = [&](size_t bytes) { unsigned char *ptr = b + o; o += round_up_256(bytes); return ptr; };
     w.cnt_q = reinterpret_cast<int *>(take(4 * N * 4));   // the four counter arrays are contiguous: one memset
     w.cnt_r = w.cnt_q + N; w.cnt_cs = w.cnt_r + N; w.cnt_len = w.cnt_cs + N;
     w.akey = reinterpret_cast<unsigned long long *>(take(N * 8));
@@ -74,12 +72,6 @@ size_t wide_nms_workspace_bytes(int64_t n) { return carve_wide(nullptr, n).bytes
 
 bool wide_nms_applies(int64_t n) { return n >= 8192 && n <= 90000; }
 
-__device__ __forceinline__ unsigned f2ord_w(float f)
-{
-    const unsigned u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 // per item: sort key and segment
 __global__ void __launch_bounds__(256)
 k_wide_keys(const float *__restrict__ scores, const int64_t *__restrict__ classes, const int32_t *__restrict__ seg_offsets,
@@ -93,7 +85,7 @@ k_wide_keys(const float *__restrict__ scores, const int64_t *__restrict__ classe
         if (__ldg(seg_offsets + mid) <= i) lo = mid; else hi = mid;
     }
     seg_of[i] = lo;
-    akey[i] = ((unsigned long long)(unsigned)__ldg(classes + i) << 32) | (unsigned long long)(~f2ord_w(__ldg(scores + i)));
+    akey[i] = ((unsigned long long)(unsigned)__ldg(classes + i) << 32) | (unsigned long long)(~f2ord(__ldg(scores + i)));
 }
 
 // Rank by counting over all pairs of a segment.  CTA (x, y): items [256x, 256x+256) against the y-th slab of 4096
@@ -217,14 +209,6 @@ __global__ void __launch_bounds__(1024) k_wide_rowoff(const int *__restrict__ sc
     if (tid == 0) rowoff[n] = s_carry;
 }
 
-__device__ __forceinline__ bool iou_gt_w(float4 a, float area_a, float4 b, float area_b, float thr)
-{
-    const float w = fmaxf(0.f, fminf(a.z, b.z) - fmaxf(a.x, b.x));
-    const float h = fmaxf(0.f, fminf(a.w, b.w) - fmaxf(a.y, b.y));
-    const float inter = w * h;
-    return inter / ((area_a + area_b) - inter) > thr;
-}
-
 // CTA (R, y): row tile R (rows q = 64R + t, one per thread) against the column tiles Cg = R + 8y .. R + 8y + 7.
 // Row q writes word (Cg - cs(q)/64) for every Cg from its own tile to the last tile of its class segment — every
 // word of the mask is written exactly once (zero where nothing overlaps), so the mask needs no memset.
@@ -258,7 +242,7 @@ __global__ void __launch_bounds__(64) k_wide_mask(WideBuffers w, int n, float th
         unsigned long long word = 0ull;
         const int b0 = Cg == R ? t + 1 : 0;                // only later boxes (q' > q)
         for (int b = b0; b < 64; ++b)
-            if (s_cs[b] == cs && iou_gt_w(bq, aq, s_box[b], s_area[b], thr)) word |= 1ull << b;
+            if (s_cs[b] == cs && iou_gt(bq, aq, s_box[b], s_area[b], thr)) word |= 1ull << b;
         w.mask[off + (Cg - (cs >> 6))] = word;
     }
 }

@@ -27,15 +27,7 @@ constexpr int kQuadBuf = 64;
 constexpr int kQuadResThreads = 128;
 
 // float -> uint32 whose unsigned order is the float order (-0 folded into +0 first: torch.topk / max compare them equal)
-__device__ __forceinline__ unsigned ord_bits(float v)
-{
-    const unsigned u = __float_as_uint(v + 0.f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float ord_value(unsigned o)
-{
-    return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
-}
+__device__ __forceinline__ unsigned ord_bits(float v) { return f2ord(v + 0.f); }
 
 __device__ __forceinline__ int quad_compress(unsigned long long *bk, int cnt, int topk, int lane)
 {
@@ -98,7 +90,7 @@ k_quad_select(const float4 *__restrict__ anchors, const float4 *__restrict__ anc
     if (lane < topk) {
         const unsigned long long k = lane < cnt ? bk[lane] : 0ull;
         sel_anchor[(int64_t)g * topk + lane] = lane < cnt ? (int)(0xffffffffu - (unsigned)k) : -1;
-        sel_val[(int64_t)g * topk + lane] = lane < cnt ? ord_value((unsigned)(k >> 32)) : 0.f;
+        sel_val[(int64_t)g * topk + lane] = lane < cnt ? ord2f((unsigned)(k >> 32)) : 0.f;
     }
 }
 
@@ -157,7 +149,7 @@ __global__ void __launch_bounds__(kQuadResThreads) k_quad_resolve(QuadResolvePar
         int64_t asg = -1;
         float iou = 0.f, rel = 0.f;
         if (cnt > 0) {
-            const float v = ord_value(s_v[la]);
+            const float v = ord2f(s_v[la]);
             const int g = (int)s_g[la];
             // the max of ref :283 runs over the selected values and one zero per gt that did not select this anchor
             if (v > 0.f || cnt == n_gt) {

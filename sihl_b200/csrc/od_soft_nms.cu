@@ -83,12 +83,6 @@ struct SoftParams {
     int smem_items;                               // candidates one CTA holds in its dynamic shared memory
 };
 
-__device__ __forceinline__ unsigned f2ord_soft(float f)
-{
-    const unsigned u = __float_as_uint(f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __device__ __forceinline__ void warp_argmax(unsigned long long &key, int &idx)
 {
 #pragma unroll
@@ -159,7 +153,7 @@ __device__ __forceinline__ void soft_body(const SoftParams &p, SoftArrays a, int
                 if (!(s >= p.score_thr)) { a.score[l] = nan; continue; }
                 a.score[l] = s;
             }
-            const unsigned long long key = ((unsigned long long)f2ord_soft(s) << 32) | a.lo[l];
+            const unsigned long long key = ((unsigned long long)f2ord(s) << 32) | a.lo[l];
             if (key > best) { best = key; bidx = l; }
         }
         // 2. the CTA's best -> its slot

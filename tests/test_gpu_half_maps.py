@@ -72,9 +72,8 @@ def test_pipeline_on_half_maps(dtype, mode, size, B, C):
         torch.testing.assert_close(out.boxes[b, :n], wb, rtol=1e-6, atol=1e-4)
 
 
-@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16])
-def test_dense_and_candidate_first_lists_agree_on_half_maps(dtype):
-    size, B, C = 320, 4, 80
+def _dense_and_candidate_first_lists_agree(dtype, C):
+    size, B = 320, 4
     levels = synth.level_sizes(size, size)
     A = synth.num_anchors(levels)
     maps = synth.dense_maps_np(5, B, A, C, loc_mean=-3.0, loc_std=2.0)
@@ -83,3 +82,14 @@ def test_dense_and_candidate_first_lists_agree_on_half_maps(dtype):
     for a, b in zip(*res):
         assert torch.equal(a, b)
     assert int(res[0][0].sum()) > 0
+
+
+@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16])
+def test_dense_and_candidate_first_lists_agree_on_half_maps(dtype):
+    _dense_and_candidate_first_lists_agree(dtype, 80)
+
+
+@pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16])
+def test_dense_scan_of_half_rows_not_a_multiple_of_its_vectors_per_lane(dtype):
+    """C = 160: rows of 20 16-byte vectors, 5 per lane; the scan takes its 8-vector kernel, which must stop at the row end."""
+    _dense_and_candidate_first_lists_agree(dtype, 160)
