@@ -445,6 +445,32 @@ SIHL_OD_API int sihl_od_batched_nms(const float *boxes, const float *scores, con
                         float iou_thr, int64_t *keep, int32_t *keep_count,
                         void *workspace, void *stream);
 
+/* Class-aware DIoU-NMS (Zheng et al., "Distance-IoU Loss", AAAI 2020): the greedy NMS above with another suppression
+ * test.  Visit by (score desc, location / index asc); a kept box i suppresses every later box j of the same class with
+ *   diou(i, j) > diou_thr,  diou = iou - cd / diag  (torchvision's _box_diou_iou, eps = 1e-7), in fp32, in this order:
+ *     w = max(0, min(x2_i, x2_j) - max(x1_i, x1_j)), h likewise;  inter = w * h
+ *     iou = inter / ((area_i + area_j) - inter),  area = (x2 - x1) * (y2 - y1)
+ *     wi = max(0, max(x2_i, x2_j) - min(x1_i, x1_j)), hi likewise;  diag = (wi * wi + hi * hi) + 1e-7
+ *     dx = (x1_i + x2_i) / 2 - (x1_j + x2_j) / 2, dy likewise;  cd = dx * dx + dy * dy
+ * so two strongly overlapping boxes with distinct centres (neighbouring objects in a crowd) can both survive.  diou lies
+ * in (-1, 1]; any threshold is accepted, and a negative one also suppresses same-class boxes that do not overlap.  A NaN
+ * diou (two zero-area boxes) never suppresses.  Each entry takes exactly the arguments of its greedy-NMS counterpart,
+ * with the same preconditions, workspace query (sihl_od_nms_workspace_bytes, sihl_od_nms_split_workspace_bytes,
+ * sihl_od_batched_nms_workspace_bytes), output layout and choice of kernels. */
+SIHL_OD_API int sihl_od_diou_nms_topk(const int32_t *cand_count, int64_t cand_capacity,
+                     const uint64_t *cand_key, const float *cand_box, const int32_t *cand_cls,
+                     int batch, float diou_thr, int k,
+                     int64_t *num_instances, float *scores, int64_t *classes, float *boxes,
+                     void *workspace, int reset_counts, void *stream);
+SIHL_OD_API int sihl_od_diou_nms_topk_split(int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                     const float *cand_box, const int32_t *cand_cls, int batch, float diou_thr, int k,
+                     int64_t *num_instances, float *scores, int64_t *classes, float *boxes,
+                     void *workspace, int reset_counts, void *stream);
+SIHL_OD_API int sihl_od_batched_diou_nms(const float *boxes, const float *scores, const int64_t *classes,
+                        const int32_t *seg_offsets, int n_images, int64_t n,
+                        float diou_thr, int64_t *keep, int32_t *keep_count,
+                        void *workspace, void *stream);
+
 /* Class-aware Soft-NMS (Bodla et al., ICCV 2017, Algorithm 1; mmcv's soft_nms) per image.  Scores are decayed
  * instead of dropped: starting from the candidates with score >= score_thr, repeatedly select the alive candidate
  * with the largest current score (ties: lowest location, or lowest input index for the stand-alone entry), emit it

@@ -190,9 +190,17 @@ __device__ __forceinline__ float box_iou(float4 a, float area_a, float4 b, float
     return inter / ((area_a + area_b) - inter);
 }
 
-// torchvision's NMS suppression test: ovr > thr (false for a NaN overlap)
-__device__ __forceinline__ bool iou_gt(float4 a, float area_a, float4 b, float area_b, float thr)
+// The overlap a greedy NMS compares with its threshold: kIoU is torchvision's nms (box_iou), kDIoU is DIoU-NMS
+// (od_math.h diou_pair).  A compile-time kind: the kernels of each kind are separate instantiations.
+constexpr int kIoU = 0;
+constexpr int kDIoU = 1;
+
+// The suppression test of a kept box a against a later box b: overlap > thr (false for a NaN overlap).
+template <int KIND>
+__device__ __forceinline__ bool overlap_gt(float4 a, float area_a, float4 b, float area_b, float thr)
 {
+    static_assert(KIND == kIoU || KIND == kDIoU, "overlap kind");
+    if (KIND == kDIoU) return diou_pair(to_box(a), area_a, to_box(b), area_b) > thr;
     return box_iou(a, area_a, b, area_b) > thr;
 }
 

@@ -69,6 +69,26 @@ SIHL_HD float ciou_pair(const BoxTerms &a, const BoxTerms &g)
     return diou - (alpha * v);
 }
 
+// torchvision.ops.distance_box_iou for one pair (tv:ops/boxes.py _box_diou_iou, eps = 1e-7): the IoU in the operator
+// order of the hard NMS, minus the squared distance of the centres over the squared diagonal of the enclosing box.
+// area_a / area_b are (x2 - x1) * (y2 - y1).  Bitwise symmetric in (a, b); NaN only when both boxes have zero area.
+// The DIoU-NMS suppression test (Zheng et al., AAAI 2020) is diou_pair(kept, later) > thr.
+SIHL_HD float diou_pair(Box4 a, float area_a, Box4 b, float area_b)
+{
+    const float eps = 1e-7f;
+    const float w = fmaxf(0.f, fminf(a.x2, b.x2) - fmaxf(a.x1, b.x1));
+    const float h = fmaxf(0.f, fminf(a.y2, b.y2) - fmaxf(a.y1, b.y1));
+    const float inter = w * h;
+    const float iou = inter / ((area_a + area_b) - inter);
+    const float wi = fmaxf(0.f, fmaxf(a.x2, b.x2) - fminf(a.x1, b.x1));
+    const float hi = fmaxf(0.f, fmaxf(a.y2, b.y2) - fminf(a.y1, b.y1));
+    const float diag = ((wi * wi) + (hi * hi)) + eps;
+    const float dx = (a.x1 + a.x2) / 2.f - (b.x1 + b.x2) / 2.f;
+    const float dy = (a.y1 + a.y2) / 2.f - (b.y1 + b.y2) / 2.f;
+    const float cd = (dx * dx) + (dy * dy);
+    return iou - (cd / diag);
+}
+
 // torchvision.ops.complete_box_iou_loss for one row — tv:ops/ciou_loss.py:47-64,
 // tv:ops/diou_loss.py:64-91, tv:ops/_utils.py:87-106.  If grad != nullptr it receives
 // dLoss/d(pred x1,y1,x2,y2) with alpha held constant (ciou_loss.py:61-62) and the

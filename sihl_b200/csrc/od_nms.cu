@@ -3,6 +3,9 @@
 // (_batched_nms_vanilla, tv:ops/boxes.py:102-120, over the CPU nms kernel): visit boxes by
 // (score desc, index asc); a kept box suppresses every later box of the same class with
 // inter / (area_i + area_j - inter) > thr.
+// DIoU-NMS (sihl_od_diou_nms_*, Zheng et al. AAAI 2020) is the same greedy rule with the test diou_pair(i, j) > thr
+// (od_math.h): every body below is templated on the overlap kind (od_common.cuh overlap_gt), and k_nms_diou<THREADS>
+// instantiates them next to k_nms<THREADS>.  The rule stays prefix-closed, so every path below serves both.
 //
 // k_nms: one CTA per image (segment), sort-free, the list length (known only on the device) picks the body:
 //   * n <= 256 (nms_small_body): 2 (top-K entry) or 4 lanes per candidate; ONE counting pass over the list gives every candidate its
@@ -124,6 +127,7 @@ __device__ __forceinline__ float4 shfl4(float4 v, int src)
 // Greedy suppression inside one 32-box chunk of a score-ordered class segment, by one warp (lane = box).
 // `dead` = already suppressed by an earlier chunk.  Returns the kept bits of the chunk (same value in every lane):
 // all 32 x 31 / 2 pairs are tested in parallel (boxes broadcast by shuffles), then the greedy chain runs on bits.
+template <int KIND>
 __device__ __forceinline__ unsigned chunk_greedy(float4 bi, float ai, bool dead, float thr, int lane)
 {
     unsigned over = 0u;                                   // earlier boxes of the chunk that overlap this one
@@ -131,7 +135,7 @@ __device__ __forceinline__ unsigned chunk_greedy(float4 bi, float ai, bool dead,
     for (int l = 0; l < 31; ++l) {
         const float4 bl = shfl4(bi, l);
         const float al = __shfl_sync(kFullMask, ai, l);
-        if (l < lane && iou_gt(bl, al, bi, ai, thr)) over |= 1u << l;
+        if (l < lane && overlap_gt<KIND>(bl, al, bi, ai, thr)) over |= 1u << l;
     }
     const unsigned alive = __ballot_sync(kFullMask, !dead);
     unsigned kept = 0u;
@@ -146,7 +150,7 @@ __device__ __forceinline__ unsigned chunk_greedy(float4 bi, float ai, bool dead,
 // One warp, one class segment [q0, q0 + m) in score order: chunks of 32 boxes; the kept boxes of a chunk then
 // suppress the later boxes of the segment (32 at a time).  m^2/2 pair tests like the serial formulation, but
 // m/32 dependent steps instead of m.
-template <bool SMEM>   // SMEM: the arrays live in shared memory (lets the compiler emit LDS/STS instead of generic accesses)
+template <int KIND, bool SMEM>   // SMEM: the arrays live in shared memory (lets the compiler emit LDS/STS instead of generic accesses)
 __device__ __forceinline__ void warp_segment_nms(const float4 *box, const float *area, unsigned char *dead_flag, int q0, int m,
                                                  float thr, int lane)
 {
@@ -159,7 +163,7 @@ __device__ __forceinline__ void warp_segment_nms(const float4 *box, const float 
         const float4 bi = valid ? box[q0 + i] : make_float4(0.f, 0.f, 0.f, 0.f);
         const float ai = valid ? area[q0 + i] : 0.f;
         const bool dead = valid ? dead_flag[q0 + i] != 0 : true;
-        const unsigned kept = chunk_greedy(bi, ai, dead, thr, lane);
+        const unsigned kept = chunk_greedy<KIND>(bi, ai, dead, thr, lane);
         if (valid && !dead && !((kept >> lane) & 1u)) dead_flag[q0 + i] = 1;
         for (int j0 = c0 + 32; j0 < m; j0 += 32) {
             const int j = j0 + lane;
@@ -171,7 +175,7 @@ __device__ __forceinline__ void warp_segment_nms(const float4 *box, const float 
                 const int l = __ffs(k) - 1;
                 const float4 bl = shfl4(bi, l);
                 const float al = __shfl_sync(kFullMask, ai, l);
-                if (live && !kill && iou_gt(bl, al, bj, aj, thr)) kill = true;
+                if (live && !kill && overlap_gt<KIND>(bl, al, bj, aj, thr)) kill = true;
             }
             if (kill) dead_flag[q0 + j] = 1;
         }
@@ -182,7 +186,7 @@ __device__ __forceinline__ void warp_segment_nms(const float4 *box, const float 
 // shared memory; every thread then tests its share of the later boxes against them.  2 barriers per 32 boxes.
 struct ChunkScratch { float4 box[32]; float area[32]; unsigned kept; int n_big; int big[32]; };
 
-template <bool SMEM>
+template <int KIND, bool SMEM>
 __device__ __forceinline__ void cta_segment_nms(const float4 *box, const float *area, unsigned char *dead_flag, int q0, int m,
                                                 float thr, ChunkScratch *sc)
 {
@@ -198,7 +202,7 @@ __device__ __forceinline__ void cta_segment_nms(const float4 *box, const float *
             const float4 bi = valid ? box[q0 + i] : make_float4(0.f, 0.f, 0.f, 0.f);
             const float ai = valid ? area[q0 + i] : 0.f;
             const bool dead = valid ? dead_flag[q0 + i] != 0 : true;
-            const unsigned kept = chunk_greedy(bi, ai, dead, thr, lane);
+            const unsigned kept = chunk_greedy<KIND>(bi, ai, dead, thr, lane);
             if (valid && !dead && !((kept >> lane) & 1u)) dead_flag[q0 + i] = 1;
             sc->box[lane] = bi;
             sc->area[lane] = ai;
@@ -213,7 +217,7 @@ __device__ __forceinline__ void cta_segment_nms(const float4 *box, const float *
             const float aj = area[q0 + j];
             for (unsigned k = kept; k != 0u; k &= k - 1u) {
                 const int l = __ffs(k) - 1;
-                if (iou_gt(sc->box[l], sc->area[l], bj, aj, thr)) { dead_flag[q0 + j] = 1; break; }
+                if (overlap_gt<KIND>(sc->box[l], sc->area[l], bj, aj, thr)) { dead_flag[q0 + j] = 1; break; }
             }
         }
     }
@@ -250,6 +254,7 @@ __device__ __forceinline__ unsigned char *list_workspace(const NmsParams &p, int
     return p.workspace + (size_t)img * p.ws_stride;
 }
 
+template <int KIND>
 __device__ __forceinline__ void nms_big_body(const NmsParams &p)
 {
     extern __shared__ __align__(16) unsigned char s_dyn[];
@@ -330,7 +335,7 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
                 const float4 bi = ar.box[q0 + i];
                 const float ai = ar.area[q0 + i];
                 for (int j = i + 1 + lane; j < m; j += 32)
-                    if (!ar.dead[q0 + j] && iou_gt(bi, ai, ar.box[q0 + j], ar.area[q0 + j], p.iou_thr)) ar.dead[q0 + j] = 1;
+                    if (!ar.dead[q0 + j] && overlap_gt<KIND>(bi, ai, ar.box[q0 + j], ar.area[q0 + j], p.iou_thr)) ar.dead[q0 + j] = 1;
             }
         }
         for (int s = 0; s < n_seg; ++s) any_big |= (ar.seg[s + 1] - ar.seg[s]) > kBigSegment;
@@ -345,7 +350,7 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
                     const float4 bi = ar.box[q0 + i];
                     const float ai = ar.area[q0 + i];
                     for (int j = i + 1 + tid; j < m; j += blockDim.x)
-                        if (!ar.dead[q0 + j] && iou_gt(bi, ai, ar.box[q0 + j], ar.area[q0 + j], p.iou_thr))
+                        if (!ar.dead[q0 + j] && overlap_gt<KIND>(bi, ai, ar.box[q0 + j], ar.area[q0 + j], p.iou_thr))
                             ar.dead[q0 + j] = 1;
                 }
                 __syncthreads();
@@ -399,7 +404,7 @@ __device__ __forceinline__ void nms_big_body(const NmsParams &p)
 // `sel` (optional, shared memory): the body runs on the n_sel candidates lb + sel[0..n_sel) instead of the whole list
 // (lazy top-K prefix).  Returns the number of survivors; with finalize == false the per-image epilogue
 // (num_instances, zero padding, counter reset) is left to the caller.
-template <int THREADS>
+template <int KIND, int THREADS>
 __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel = nullptr, int n_sel = 0, bool finalize = true)
 {
     constexpr int kLanes = THREADS / kSmallItems;
@@ -497,7 +502,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
         if (have && len <= 32) {
             const float area = (bx.z - bx.x) * (bx.w - bx.y);
             for (int j = sub; j < k; j += kLanes)
-                if (iou_gt(s_box[seg0 + j], s_area[seg0 + j], bx, area, p.iou_thr)) mask |= 1u << j;
+                if (overlap_gt<KIND>(s_box[seg0 + j], s_area[seg0 + j], bx, area, p.iou_thr)) mask |= 1u << j;
         }
 #pragma unroll
         for (int o = kLanes / 2; o > 0; o >>= 1) mask |= __shfl_xor_sync(kFullMask, mask, o);
@@ -521,7 +526,7 @@ __device__ __forceinline__ int nms_small_body(const NmsParams &p, const int *sel
                     const float4 bi = s_box[q0 + i];
                     const float ai = s_area[q0 + i];
                     for (int j = i + 1 + lane; j < m; j += 32)
-                        if (!s_dead[q0 + j] && iou_gt(bi, ai, s_box[q0 + j], s_area[q0 + j], p.iou_thr)) s_dead[q0 + j] = 1;
+                        if (!s_dead[q0 + j] && overlap_gt<KIND>(bi, ai, s_box[q0 + j], s_area[q0 + j], p.iou_thr)) s_dead[q0 + j] = 1;
                 }
             }
             __syncthreads();
@@ -677,7 +682,7 @@ __device__ __forceinline__ MedArrays carve_med(unsigned char *base, int n_al)
 
 // SMEM: the arrays are in shared memory (tells the compiler the address space: generic loads from shared are
 // several times slower than LDS and do not pipeline in the counting loops).
-template <bool SMEM, int THREADS>
+template <int KIND, bool SMEM, int THREADS>
 __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int src0, unsigned char *base, int n_al,
                                                 int *s_warp, unsigned *h_cls, int *h_cnt, int *h_start, ChunkScratch *chunk_scratch,
                                                 int *n_kept_out)
@@ -799,7 +804,7 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
             const float4 bq = ar.f_box[q];
             const float aq = ar.f_area[q];
             for (int j = s0; j < q; ++j)
-                if (iou_gt(ar.f_box[j], ar.f_area[j], bq, aq, p.iou_thr)) bits |= 1ull << (j - s0);
+                if (overlap_gt<KIND>(ar.f_box[j], ar.f_area[j], bq, aq, p.iou_thr)) bits |= 1ull << (j - s0);
         }
         mask[q] = bits;
     }
@@ -821,7 +826,7 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
     for (int h = warp; h < kHashSlots; h += nwarps) {             // long segments: one warp each, 32-box chunks
         const int m = h_cnt[h];
         if (m <= 64 || m > kWarpSegment) continue;
-        warp_segment_nms<SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], m, p.iou_thr, lane);
+        warp_segment_nms<KIND, SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], m, p.iou_thr, lane);
     }
     __syncthreads();
     const int n_big = chunk_scratch->n_big;                       // very long segments: the whole CTA, one after another
@@ -829,12 +834,12 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
         if (n_big <= 32) {
             for (int k = 0; k < n_big; ++k) {
                 const int h = chunk_scratch->big[k];               // (cta_segment_nms only touches box / area / kept)
-                cta_segment_nms<SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], h_cnt[h], p.iou_thr, chunk_scratch);
+                cta_segment_nms<KIND, SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], h_cnt[h], p.iou_thr, chunk_scratch);
             }
         } else {
             for (int h = 0; h < kHashSlots; ++h)
                 if (h_cnt[h] > kWarpSegment)
-                    cta_segment_nms<SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], h_cnt[h], p.iou_thr, chunk_scratch);
+                    cta_segment_nms<KIND, SMEM>(ar.f_box, ar.f_area, ar.f_dead, h_start[h], h_cnt[h], p.iou_thr, chunk_scratch);
         }
     }
     // 6. survivors -> u_key/u_slot (ballot compaction), then ordered by (score desc, index asc) WITHOUT a sort:
@@ -944,8 +949,8 @@ __device__ __forceinline__ bool nms_medium_body(const NmsParams &p, int n, int s
 }
 
 // One launch for every path: the list length (known only on the device) picks the body.
-template <int THREADS>   // <= 64 registers per thread either way: 512 threads take half the register file
-__global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
+template <int KIND, int THREADS>
+__device__ __forceinline__ void nms_entry(const NmsParams &p)
 {
     extern __shared__ __align__(16) unsigned char s_dyn_top[];
     __shared__ int s_warp_top[33];
@@ -961,7 +966,7 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
         src0 = __ldg(p.seg_offsets + blockIdx.x);
         n = __ldg(p.seg_offsets + blockIdx.x + 1) - src0;
     }
-    if (n <= kSmallItems) { nms_small_body<THREADS>(p); return; }
+    if (n <= kSmallItems) { nms_small_body<KIND, THREADS>(p); return; }
     if (p.mode == 0 && p.K <= kLazyMaxK) {
         // top-K of a long list: try the highest-ranked ~200 candidates first (exact: see the file header)
         __shared__ int s_sel[kSmallItems];
@@ -970,7 +975,7 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
         const int64_t lb = list_base(p, (int)blockIdx.x);
         const int m = lazy_prefix_select(p, lb, n, s_sel, reinterpret_cast<unsigned *>(s_hcnt), s_pick, &s_count);
         if (m > 0) {
-            const int kept = nms_small_body<THREADS>(p, s_sel, m, false);
+            const int kept = nms_small_body<KIND, THREADS>(p, s_sel, m, false);
             if (kept >= p.K) {                             // the K best survivors are all inside the prefix: done
                 if (threadIdx.x == 0) {
                     p.num_instances[blockIdx.x] = p.K;
@@ -986,10 +991,10 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
     int n_kept = 0;
     bool done;
     if (n_al <= p.smem_items) {
-        done = nms_medium_body<true, THREADS>(p, n, src0, s_dyn_top, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
+        done = nms_medium_body<KIND, true, THREADS>(p, n, src0, s_dyn_top, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
     } else {
         unsigned char *ws = list_workspace(p, (int)blockIdx.x, src0);
-        done = nms_medium_body<false, THREADS>(p, n, src0, ws, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
+        done = nms_medium_body<KIND, false, THREADS>(p, n, src0, ws, n_al, s_warp_top, s_hcls, s_hcnt, s_hstart, &s_chunk, &n_kept);
     }
     if (done) {
         const int img = blockIdx.x, tid = threadIdx.x;
@@ -1011,8 +1016,14 @@ __global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p)
         return;
     }
     __syncthreads();
-    nms_big_body(p);
+    nms_big_body<KIND>(p);
 }
+
+// Greedy NMS (torchvision's IoU test) and DIoU-NMS: separate kernels over the same bodies.
+template <int THREADS>   // <= 64 registers per thread either way: 512 threads take half the register file
+__global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms(NmsParams p) { nms_entry<kIoU, THREADS>(p); }
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS, 1024 / THREADS) k_nms_diou(NmsParams p) { nms_entry<kDIoU, THREADS>(p); }
 
 // ---------------------------------------------------------------------------
 // Class-split NMS for long lists (mode 0).  Suppression never crosses classes, so an image's candidates can be
@@ -1135,20 +1146,21 @@ static int pow2ceil(int64_t n)
 
 // smem_items: candidates per list whose long-list arrays the launch keeps in dynamic shared memory (0: none, every long
 // list uses the workspace).  Dynamic shared memory is reserved only when a list can exceed the short-list path.
-template <int THREADS>
+template <int KIND, int THREADS>
 static int launch_nms(NmsParams p, int n_images, int64_t max_items, cudaStream_t st, int smem_items)
 {
+    void (*kernel)(NmsParams) = KIND == kDIoU ? k_nms_diou<THREADS> : k_nms<THREADS>;
     p.smem_items = smem_items;
     const size_t smem = max_items > kSmallItems ? (size_t)smem_items * kSmemItemBytes : 0;
     static thread_local bool attr_set = false;
     if (smem && !attr_set) {
-        int rc = cuda_status(cudaFuncSetAttribute(k_nms<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        int rc = cuda_status(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                   (int)((size_t)kSmemItems * kSmemItemBytes)),
                              "cudaFuncSetAttribute(k_nms)");
         if (rc) return rc;
         attr_set = true;
     }
-    k_nms<THREADS><<<n_images, THREADS, smem, st>>>(p);
+    kernel<<<n_images, THREADS, smem, st>>>(p);
     SIHL_CHECK_LAUNCH("k_nms");
     return SIHL_OD_OK;
 }
@@ -1165,10 +1177,12 @@ extern "C" size_t sihl_od_nms_workspace_bytes(int batch, int64_t cand_capacity)
     return (size_t)batch * (size_t)np * kWsItemBytes;
 }
 
-extern "C" int sihl_od_nms_topk(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
-                                const float *cand_box, const int32_t *cand_cls, int batch, float iou_thr, int k,
-                                int64_t *num_instances, float *scores, int64_t *classes, float *boxes, void *workspace,
-                                int reset_counts, void *stream)
+// The entries of greedy NMS and DIoU-NMS share their argument checks, workspaces and launch choices: only the kernels'
+// overlap kind differs.
+template <int KIND>
+static int nms_topk_entry(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key, const float *cand_box,
+                          const int32_t *cand_cls, int batch, float iou_thr, int k, int64_t *num_instances, float *scores,
+                          int64_t *classes, float *boxes, void *workspace, int reset_counts, void *stream)
 {
     SIHL_CHECK_ARG(cand_count && cand_key && cand_box && cand_cls, "NULL input");
     SIHL_CHECK_ARG(num_instances && scores && classes && boxes, "NULL output");
@@ -1186,15 +1200,33 @@ extern "C" int sihl_od_nms_topk(const int32_t *cand_count, int64_t cand_capacity
     p.workspace = static_cast<unsigned char *>(workspace);
     p.ws_stride = (size_t)pow2ceil(cand_capacity) * kWsItemBytes;
     // runs next to the dense scan of the neighbouring steps: no dynamic shared memory (see the file header)
-    return launch_nms<kNmsThreadsTopk>(p, batch, cand_capacity, (cudaStream_t)stream, 0);
+    return launch_nms<KIND, kNmsThreadsTopk>(p, batch, cand_capacity, (cudaStream_t)stream, 0);
+}
+
+extern "C" int sihl_od_nms_topk(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                                const float *cand_box, const int32_t *cand_cls, int batch, float iou_thr, int k,
+                                int64_t *num_instances, float *scores, int64_t *classes, float *boxes, void *workspace,
+                                int reset_counts, void *stream)
+{
+    return nms_topk_entry<kIoU>(cand_count, cand_capacity, cand_key, cand_box, cand_cls, batch, iou_thr, k, num_instances,
+                                scores, classes, boxes, workspace, reset_counts, stream);
+}
+
+extern "C" int sihl_od_diou_nms_topk(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                                     const float *cand_box, const int32_t *cand_cls, int batch, float diou_thr, int k,
+                                     int64_t *num_instances, float *scores, int64_t *classes, float *boxes, void *workspace,
+                                     int reset_counts, void *stream)
+{
+    return nms_topk_entry<kDIoU>(cand_count, cand_capacity, cand_key, cand_box, cand_cls, batch, diou_thr, k, num_instances,
+                                 scores, classes, boxes, workspace, reset_counts, stream);
 }
 
 namespace sihl {                 // od_nms_wide.cu: the multi-CTA bitmask path for one long list
 size_t wide_nms_workspace_bytes(int64_t n);
 bool wide_nms_applies(int64_t n);
 int launch_wide_batched_nms(const float *boxes, const float *scores, const int64_t *classes, const int32_t *seg_offsets,
-                            int n_images, int64_t n, float iou_thr, int64_t *keep, int32_t *keep_count, void *workspace,
-                            cudaStream_t st);
+                            int n_images, int64_t n, int kind, float iou_thr, int64_t *keep, int32_t *keep_count,
+                            void *workspace, cudaStream_t st);
 }
 
 extern "C" size_t sihl_od_batched_nms_workspace_bytes(int64_t n)
@@ -1204,9 +1236,10 @@ extern "C" size_t sihl_od_batched_nms_workspace_bytes(int64_t n)
     return (size_t)(2 * n + 2) * kWsItemBytes;
 }
 
-extern "C" int sihl_od_batched_nms(const float *boxes, const float *scores, const int64_t *classes,
-                                   const int32_t *seg_offsets, int n_images, int64_t n, float iou_thr, int64_t *keep,
-                                   int32_t *keep_count, void *workspace, void *stream)
+template <int KIND>
+static int batched_nms_entry(const float *boxes, const float *scores, const int64_t *classes, const int32_t *seg_offsets,
+                             int n_images, int64_t n, float iou_thr, int64_t *keep, int32_t *keep_count, void *workspace,
+                             void *stream)
 {
     SIHL_CHECK_ARG(seg_offsets && keep_count, "NULL argument");
     SIHL_CHECK_ARG(n >= 0 && n < (1ll << 30) && n_images >= 0, "bad sizes");
@@ -1215,13 +1248,29 @@ extern "C" int sihl_od_batched_nms(const float *boxes, const float *scores, cons
                    (long long)n);
     if (n_images == 0) return SIHL_OD_OK;
     if (wide_nms_applies(n))        // 8192..90000 boxes: bitmask-parallel suppression over all SMs (od_nms_wide.cu)
-        return launch_wide_batched_nms(boxes, scores, classes, seg_offsets, n_images, n, iou_thr, keep, keep_count, workspace,
-                                       (cudaStream_t)stream);
+        return launch_wide_batched_nms(boxes, scores, classes, seg_offsets, n_images, n, KIND, iou_thr, keep, keep_count,
+                                       workspace, (cudaStream_t)stream);
     NmsParams p = {};
     p.boxes = reinterpret_cast<const float4 *>(boxes); p.scores = scores; p.classes = classes; p.seg_offsets = seg_offsets;
     p.mode = 1; p.iou_thr = iou_thr; p.keep = keep; p.keep_count = keep_count;
     p.workspace = static_cast<unsigned char *>(workspace); p.ws_stride = 0;
-    return launch_nms<kNmsThreadsAlone>(p, n_images, n, (cudaStream_t)stream, kSmemItems);
+    return launch_nms<KIND, kNmsThreadsAlone>(p, n_images, n, (cudaStream_t)stream, kSmemItems);
+}
+
+extern "C" int sihl_od_batched_nms(const float *boxes, const float *scores, const int64_t *classes,
+                                   const int32_t *seg_offsets, int n_images, int64_t n, float iou_thr, int64_t *keep,
+                                   int32_t *keep_count, void *workspace, void *stream)
+{
+    return batched_nms_entry<kIoU>(boxes, scores, classes, seg_offsets, n_images, n, iou_thr, keep, keep_count, workspace,
+                                   stream);
+}
+
+extern "C" int sihl_od_batched_diou_nms(const float *boxes, const float *scores, const int64_t *classes,
+                                        const int32_t *seg_offsets, int n_images, int64_t n, float diou_thr, int64_t *keep,
+                                        int32_t *keep_count, void *workspace, void *stream)
+{
+    return batched_nms_entry<kDIoU>(boxes, scores, classes, seg_offsets, n_images, n, diou_thr, keep, keep_count, workspace,
+                                    stream);
 }
 
 // ---- class-split variant (long lists) ------------------------------------------------------------------
@@ -1246,10 +1295,11 @@ extern "C" size_t sihl_od_nms_split_workspace_bytes(int batch, int64_t cand_capa
     return bytes;
 }
 
-extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
-                                      const float *cand_box, const int32_t *cand_cls, int batch, float iou_thr, int k,
-                                      int64_t *num_instances, float *scores, int64_t *classes, float *boxes, void *workspace,
-                                      int reset_counts, void *stream)
+template <int KIND>
+static int nms_topk_split_entry(int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key, const float *cand_box,
+                                const int32_t *cand_cls, int batch, float iou_thr, int k, int64_t *num_instances,
+                                float *scores, int64_t *classes, float *boxes, void *workspace, int reset_counts,
+                                void *stream)
 {
     SIHL_CHECK_ARG(cand_count && cand_key && cand_box && cand_cls, "NULL input");
     SIHL_CHECK_ARG(num_instances && scores && classes && boxes && workspace, "NULL output / workspace");
@@ -1284,7 +1334,7 @@ extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity
     p.num_instances = sub_num; p.out_scores = sub_scores; p.out_classes = sub_classes; p.out_boxes = sub_boxes;
     p.out_keys = sub_keys; p.workspace = nms_ws; p.ws_stride = 0;
     // sub-lists rarely exceed 2048 candidates: half the shared memory per CTA lets two of them share an SM
-    int rc = launch_nms<kNmsThreadsAlone>(p, batch * S, cand_capacity, st, kSmemItems / 2);
+    int rc = launch_nms<KIND, kNmsThreadsAlone>(p, batch * S, cand_capacity, st, kSmemItems / 2);
     if (rc) return rc;
     MergeParams mp;
     mp.S = S; mp.K = k; mp.sub_num = sub_num; mp.sub_keys = sub_keys; mp.sub_scores = sub_scores; mp.sub_classes = sub_classes;
@@ -1305,4 +1355,22 @@ extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity
     }
     SIHL_CHECK_LAUNCH("k_nms_merge");
     return SIHL_OD_OK;
+}
+
+extern "C" int sihl_od_nms_topk_split(int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                                      const float *cand_box, const int32_t *cand_cls, int batch, float iou_thr, int k,
+                                      int64_t *num_instances, float *scores, int64_t *classes, float *boxes, void *workspace,
+                                      int reset_counts, void *stream)
+{
+    return nms_topk_split_entry<kIoU>(cand_count, cand_capacity, cand_key, cand_box, cand_cls, batch, iou_thr, k,
+                                      num_instances, scores, classes, boxes, workspace, reset_counts, stream);
+}
+
+extern "C" int sihl_od_diou_nms_topk_split(int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                                           const float *cand_box, const int32_t *cand_cls, int batch, float diou_thr, int k,
+                                           int64_t *num_instances, float *scores, int64_t *classes, float *boxes,
+                                           void *workspace, int reset_counts, void *stream)
+{
+    return nms_topk_split_entry<kDIoU>(cand_count, cand_capacity, cand_key, cand_box, cand_cls, batch, diou_thr, k,
+                                       num_instances, scores, classes, boxes, workspace, reset_counts, stream);
 }

@@ -10,7 +10,7 @@
 //                   (class asc, score desc, index asc), its score rank r, the start / length of its class segment
 //                   (rank by counting: no sort, no barrier chain; 4 integer comparisons per pair)
 //   k_wide_scatter  items -> class-major order; k_wide_rowoff: exclusive scan of the mask-row lengths
-//   k_wide_mask     bitmask-parallel IoU: 64 x 64 tiles (row tile, column tile >= row tile) WITHIN class segments
+//   k_wide_mask     bitmask-parallel IoU (k_wide_mask_diou: the DIoU test of DIoU-NMS): 64 x 64 tiles (row tile, column tile >= row tile) WITHIN class segments
 //                   only; word w of row q holds the later same-class boxes of tile (first tile of the class + w)
 //                   that q would suppress
 //   k_wide_reduce   the serial greedy pass on mask words: one CTA per class segment, 64 rows per step — the
@@ -212,13 +212,15 @@ __global__ void __launch_bounds__(1024) k_wide_rowoff(const int *__restrict__ sc
 // CTA (R, y): row tile R (rows q = 64R + t, one per thread) against the column tiles Cg = R + 8y .. R + 8y + 7.
 // Row q writes word (Cg - cs(q)/64) for every Cg from its own tile to the last tile of its class segment — every
 // word of the mask is written exactly once (zero where nothing overlaps), so the mask needs no memset.
-__global__ void __launch_bounds__(64) k_wide_mask(WideBuffers w, int n, float thr)
+// t = threadIdx.x, read by the kernel, where the launch bound tells the compiler that t < 64.
+template <int KIND>
+__device__ __forceinline__ void wide_mask(WideBuffers w, int n, float thr, int t)
 {
     __shared__ float4 s_box[64];
     __shared__ float s_area[64];
     __shared__ int s_cs[64];
     __shared__ int s_last;
-    const int t = threadIdx.x, R = blockIdx.x;
+    const int R = blockIdx.x;
     const int q = R * 64 + t;
     const bool have = q < n;
     int cs = 0, ce = 0;
@@ -242,10 +244,14 @@ __global__ void __launch_bounds__(64) k_wide_mask(WideBuffers w, int n, float th
         unsigned long long word = 0ull;
         const int b0 = Cg == R ? t + 1 : 0;                // only later boxes (q' > q)
         for (int b = b0; b < 64; ++b)
-            if (s_cs[b] == cs && iou_gt(bq, aq, s_box[b], s_area[b], thr)) word |= 1ull << b;
+            if (s_cs[b] == cs && overlap_gt<KIND>(bq, aq, s_box[b], s_area[b], thr)) word |= 1ull << b;
         w.mask[off + (Cg - (cs >> 6))] = word;
     }
 }
+
+// the mask of greedy NMS (torchvision's IoU test) and of DIoU-NMS; every other step serves both
+__global__ void __launch_bounds__(64) k_wide_mask(WideBuffers w, int n, float thr) { wide_mask<kIoU>(w, n, thr, threadIdx.x); }
+__global__ void __launch_bounds__(64) k_wide_mask_diou(WideBuffers w, int n, float thr) { wide_mask<kDIoU>(w, n, thr, threadIdx.x); }
 
 // One CTA per 64-tile of the class-major order; it serves every class segment that STARTS in its tile.
 constexpr int kReduceThreads = 512;
@@ -352,8 +358,8 @@ k_wide_emit(WideBuffers w, const int32_t *__restrict__ seg_offsets, int64_t *__r
 }
 
 int launch_wide_batched_nms(const float *boxes, const float *scores, const int64_t *classes, const int32_t *seg_offsets,
-                            int n_images, int64_t n64, float iou_thr, int64_t *keep, int32_t *keep_count, void *workspace,
-                            cudaStream_t st)
+                            int n_images, int64_t n64, int kind, float iou_thr, int64_t *keep, int32_t *keep_count,
+                            void *workspace, cudaStream_t st)
 {
     const int n = (int)n64;
     WideBuffers w = carve_wide(workspace, n64);
@@ -371,7 +377,8 @@ int launch_wide_batched_nms(const float *boxes, const float *scores, const int64
     SIHL_CHECK_LAUNCH("k_wide_rowoff");
     const int tiles = (n + 63) / 64;
     const dim3 mgrid((unsigned)tiles, (unsigned)((tiles + kWideColsPerCta - 1) / kWideColsPerCta));
-    k_wide_mask<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
+    if (kind == kDIoU) k_wide_mask_diou<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
+    else k_wide_mask<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
     SIHL_CHECK_LAUNCH("k_wide_mask");
     k_wide_reduce<<<tiles, kReduceThreads, 0, st>>>(w, n);
     SIHL_CHECK_LAUNCH("k_wide_reduce");

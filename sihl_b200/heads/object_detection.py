@@ -333,9 +333,11 @@ class ObjectDetection(nn.Module):
         box of the locations that pass the threshold only — identical results; default: ``"dense"`` for fp32 maps,
         ``"candidate_first"`` for half maps (autocast), which are then read as they are (no fp32 copies).
 
-        ``nms``: ``"hard"`` (greedy NMS), ``"soft_linear"`` (Soft-NMS, ``iou_threshold`` is Nt) or ``"soft_gaussian"``
-        (Soft-NMS with ``sigma``): overlapping boxes of a class have their scores decayed instead of being dropped,
-        which keeps real objects in crowds; the returned scores are the decayed ones."""
+        ``nms``: ``"hard"`` (greedy NMS), ``"diou"`` (greedy DIoU-NMS, ``iou_threshold`` is the DIoU threshold: a box
+        survives an overlapping box of its class when their centres lie far enough apart), ``"soft_linear"`` (Soft-NMS,
+        ``iou_threshold`` is Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``): overlapping boxes of a class have
+        their scores decayed instead of being dropped, which keeps real objects in crowds; the returned scores are the
+        decayed ones."""
         if nms not in ops.NMS_KINDS:
             raise ValueError(f"nms={nms!r}: expected one of {ops.NMS_KINDS}")
         (_, _, height, width) = inputs[0].shape

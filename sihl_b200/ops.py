@@ -595,11 +595,23 @@ def half_dense_scan_ok(cls_logits: Tensor) -> bool:
 
 SPLIT_NMS_FROM = 16384     # list capacity (locations per image) from which the one-shot postprocess uses the class-split NMS
 
+# The suppression test of the greedy NMS entries -> the infix of their C names: "iou" is torchvision's nms (IoU > thr),
+# "diou" is DIoU-NMS (Zheng et al., AAAI 2020: IoU minus the normalised squared distance of the centres > thr).
+NMS_OVERLAPS = {"iou": "", "diou": "diou_"}
+
+
+def _overlap_infix(overlap: str) -> str:
+    if overlap not in NMS_OVERLAPS:
+        raise ValueError(f"overlap={overlap!r}: expected one of {tuple(NMS_OVERLAPS)}")
+    return NMS_OVERLAPS[overlap]
+
 
 def nms_topk(cand: CandidateBuffers, batch: int, iou_thr: float, k: int, out: Optional[tuple] = None,
-             reset_counts: bool = False, split: bool = False):
+             reset_counts: bool = False, split: bool = False, overlap: str = "iou"):
     """Class-aware NMS + top-k over the candidate lists.  ``split``: the class-split multi-CTA variant for long lists
-    (same results; thousands of candidates per image)."""
+    (same results; thousands of candidates per image).  ``overlap``: ``"iou"`` (greedy NMS) or ``"diou"`` (DIoU-NMS,
+    ``iou_thr`` is the DIoU threshold; same order, outputs and workspace)."""
+    infix = _overlap_infix(overlap)
     dev = cand.count.device
     if out is None:
         out = (torch.empty((batch,), dtype=torch.int64, device=dev), torch.empty((batch, k), dtype=torch.float32, device=dev),
@@ -610,22 +622,24 @@ def nms_topk(cand: CandidateBuffers, batch: int, iou_thr: float, k: int, out: Op
         if ws is None or ws.numel() < need:
             ws = torch.empty((need,), dtype=torch.uint8, device=dev)
             cand._split_ws = ws
+        name = f"sihl_od_{infix}nms_topk_split"
         with _on(dev):
-            rc = _lib().sihl_od_nms_topk_split(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
-                                               float(iou_thr), int(k), _p(out[0]), _p(out[1]), _p(out[2]), _p(out[3]), _p(ws),
-                                               int(reset_counts), _stream(dev))
-        _native.check(rc, "sihl_od_nms_topk_split")
+            rc = getattr(_lib(), name)(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
+                                       float(iou_thr), int(k), _p(out[0]), _p(out[1]), _p(out[2]), _p(out[3]), _p(ws),
+                                       int(reset_counts), _stream(dev))
+        _native.check(rc, name)
         return out
+    name = f"sihl_od_{infix}nms_topk"
     with _on(dev):
-        rc = _lib().sihl_od_nms_topk(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
-                                     float(iou_thr), int(k), _p(out[0]), _p(out[1]), _p(out[2]), _p(out[3]),
-                                     _p(cand.workspace), int(reset_counts), _stream(dev))
-    _native.check(rc, "sihl_od_nms_topk")
+        rc = getattr(_lib(), name)(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
+                                   float(iou_thr), int(k), _p(out[0]), _p(out[1]), _p(out[2]), _p(out[3]),
+                                   _p(cand.workspace), int(reset_counts), _stream(dev))
+    _native.check(rc, name)
     return out
 
 
 SOFT_NMS_METHODS = {"linear": 1, "gaussian": 2}          # SIHL_OD_SOFT_NMS_LINEAR / _GAUSSIAN (sihl_od.h)
-NMS_KINDS = ("hard", "soft_linear", "soft_gaussian")
+NMS_KINDS = ("hard", "diou", "soft_linear", "soft_gaussian")
 
 
 def _soft_method(method) -> int:
@@ -668,8 +682,9 @@ def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, l
     Output format of ``ObjectDetection.forward`` (ref :122), zero padded past ``num_instances``.
     ``mode``: see :func:`dense_decode` (identical results).  ``split_nms``: class-split NMS (default: whenever the
     lists can hold more than ``SPLIT_NMS_FROM`` candidates).  ``nms``: ``"hard"`` (greedy, torchvision's semantics),
-    ``"soft_linear"`` (Soft-NMS with ``iou_thr`` as Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``); the soft
-    methods keep decaying scores down to ``score_thr`` and ignore ``split_nms``."""
+    ``"diou"`` (greedy DIoU-NMS with ``iou_thr`` as the DIoU threshold), ``"soft_linear"`` (Soft-NMS with ``iou_thr`` as
+    Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``); the soft methods keep decaying scores down to ``score_thr``
+    and ignore ``split_nms``."""
     if nms not in NMS_KINDS:
         raise ValueError(f"nms={nms!r}: expected one of {NMS_KINDS}")
     B, A = loc_logits.shape
@@ -677,7 +692,7 @@ def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, l
     if cand is None:
         cand = CandidateBuffers.allocate(B, A, loc_logits.device)
     dense_decode(loc_logits, cls_logits, box_raw, offsets, scales, img_w, img_h, score_thr, cand, mode=mode)
-    if nms != "hard":
+    if nms.startswith("soft_"):
         return soft_nms_topk(cand, B, nms[len("soft_"):], iou_thr, sigma, score_thr, max_instances)
     if split_nms is None:
         # The list lengths are only known on the device, so the choice goes by what can happen: big images (>= 896^2)
@@ -686,16 +701,18 @@ def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, l
         # 3x cheaper than three launches (measured: profiles/r01_postprocess_sweep.json)
         n_sub = min(32, max(2, -(-cand.capacity // 2048)))
         split_nms = cand.capacity >= SPLIT_NMS_FROM and B * n_sub <= 296
-    return nms_topk(cand, B, iou_thr, max_instances, split=split_nms)
+    return nms_topk(cand, B, iou_thr, max_instances, split=split_nms, overlap="diou" if nms == "diou" else "iou")
 
 
 def batched_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: float,
-                seg_offsets: Optional[Tensor] = None):
+                seg_offsets: Optional[Tensor] = None, overlap: str = "iou"):
     """``torchvision.ops.batched_nms`` signature (exact per-class semantics, stable order).
 
     With ``seg_offsets`` (int32 ``[n_images+1]``) the call handles several images at once and
     returns ``(keep [N] i64, keep_count [n_images] i32)``; without it, the kept indices of the
-    single segment (one deliberate sync to size the result, like torchvision)."""
+    single segment (one deliberate sync to size the result, like torchvision).  ``overlap="diou"``: DIoU-NMS,
+    ``iou_threshold`` is the DIoU threshold (same order and outputs)."""
+    infix = _overlap_infix(overlap)
     boxes = _req(boxes, torch.float32, "boxes", 2)
     scores = _req(scores, torch.float32, "scores", 1)
     idxs = _req(idxs, torch.int64, "idxs", 1)
@@ -709,10 +726,11 @@ def batched_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: floa
     count = torch.zeros((n_images,), dtype=torch.int32, device=dev)
     ws_bytes = int(_lib().sihl_od_batched_nms_workspace_bytes(N))
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+    name = f"sihl_od_batched_{infix}nms"
     with _on(dev):
-        rc = _lib().sihl_od_batched_nms(_p(boxes), _p(scores), _p(idxs), _p(seg_offsets), n_images, N,
-                                        float(iou_threshold), _p(keep), _p(count), _p(ws), _stream(dev))
-    _native.check(rc, "sihl_od_batched_nms")
+        rc = getattr(_lib(), name)(_p(boxes), _p(scores), _p(idxs), _p(seg_offsets), n_images, N,
+                                   float(iou_threshold), _p(keep), _p(count), _p(ws), _stream(dev))
+    _native.check(rc, name)
     if single:
         return keep[: int(count.item())]
     return keep[:N], count
