@@ -471,6 +471,37 @@ SIHL_OD_API int sihl_od_batched_diou_nms(const float *boxes, const float *scores
                         float diou_thr, int64_t *keep, int32_t *keep_count,
                         void *workspace, void *stream);
 
+/* Class-aware box voting (merge-NMS; Gidaris & Komodakis, ICCV 2015; YOLOv5's non_max_suppression(merge=True)), one
+ * pass after a greedy NMS (IoU or DIoU) that moves the coordinates of the kept boxes only.  For every emitted
+ * detection k of class c, with the overlap and the threshold of the selection it follows (iou_thr / diou_thr):
+ *   V_k  = { j in the same list : cls_j == c  and  overlap(b_k, b_j) > thr }   any rank, kept or suppressed, k included
+ *   b'_k = sum_{j in V_k} s_j * b_j / sum_{j in V_k} s_j                       per coordinate
+ * overlap is the IoU of sihl_od_nms_topk (the *_box_vote_* entries) or the diou of sihl_od_diou_nms_topk (the
+ * *_diou_box_vote_* entries), in the same fp32 operator order; a NaN overlap never joins a cluster, and a negative
+ * DIoU threshold admits same-class boxes that do not overlap.  s_j is the candidate's score (the high word of cand_key,
+ * or scores[j]).  Every product s_j * x_j is exact in fp64; the sums are fp64 (their order is unspecified) and the
+ * quotient is rounded once to fp32.  When V_k is empty or its score sum is 0 (thr >= 1, a zero-area kept box, scores
+ * that underflow), b_k is left as it is.  Counts, scores, classes, keep indices and their order are not touched.
+ * No workspace, no host synchronisation: the pass can be captured in a CUDA graph.
+ *
+ * Top-K entries: the candidate lists and the outputs of sihl_od_nms_topk / _split (or the DIoU entries) called with
+ * reset_counts = 0, which leaves the lists and cand_count as they were; boxes [batch, k, 4] is rewritten in place,
+ * rows past num_instances[b] (the zero padding) are not touched.  Batched entries: the inputs of sihl_od_batched_nms
+ * (or sihl_od_batched_diou_nms) and its keep / keep_count; voted_boxes [N, 4] receives the voted box of keep[i] at row
+ * i for the first keep_count[s] positions of every segment and nothing elsewhere. */
+SIHL_OD_API int sihl_od_box_vote_topk(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                     const float *cand_box, const int32_t *cand_cls, int batch, float iou_thr, int k,
+                     const int64_t *num_instances, const int64_t *classes, float *boxes, void *stream);
+SIHL_OD_API int sihl_od_diou_box_vote_topk(const int32_t *cand_count, int64_t cand_capacity, const uint64_t *cand_key,
+                     const float *cand_box, const int32_t *cand_cls, int batch, float diou_thr, int k,
+                     const int64_t *num_instances, const int64_t *classes, float *boxes, void *stream);
+SIHL_OD_API int sihl_od_batched_box_vote(const float *boxes, const float *scores, const int64_t *classes,
+                        const int32_t *seg_offsets, int n_images, int64_t n, float iou_thr,
+                        const int64_t *keep, const int32_t *keep_count, float *voted_boxes, void *stream);
+SIHL_OD_API int sihl_od_batched_diou_box_vote(const float *boxes, const float *scores, const int64_t *classes,
+                        const int32_t *seg_offsets, int n_images, int64_t n, float diou_thr,
+                        const int64_t *keep, const int32_t *keep_count, float *voted_boxes, void *stream);
+
 /* Class-aware Soft-NMS (Bodla et al., ICCV 2017, Algorithm 1; mmcv's soft_nms) per image.  Scores are decayed
  * instead of dropped: starting from the candidates with score >= score_thr, repeatedly select the alive candidate
  * with the largest current score (ties: lowest location, or lowest input index for the stand-alone entry), emit it

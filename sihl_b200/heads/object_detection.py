@@ -324,7 +324,8 @@ class ObjectDetection(nn.Module):
 
     @torch.no_grad()
     def postprocess(self, inputs: List[Tensor], score_threshold: float = 0.05, iou_threshold: float = 0.5,
-                    mode: Optional[str] = None, nms: str = "hard", sigma: float = 0.5) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                    mode: Optional[str] = None, nms: str = "hard", sigma: float = 0.5,
+                    box_voting: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
         """North-star extension (the reference has no NMS): every location is decoded with the
         score/class semantics of ``forward`` (score = sigmoid(location logit), class = argmax),
         thresholded, and de-duplicated by class-aware NMS; same output format as ``forward``.
@@ -337,9 +338,15 @@ class ObjectDetection(nn.Module):
         survives an overlapping box of its class when their centres lie far enough apart), ``"soft_linear"`` (Soft-NMS,
         ``iou_threshold`` is Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``): overlapping boxes of a class have
         their scores decayed instead of being dropped, which keeps real objects in crowds; the returned scores are the
-        decayed ones."""
+        decayed ones.
+
+        ``box_voting`` (with ``"hard"`` or ``"diou"``): box voting / merge-NMS (YOLOv5's ``merge=True``): every kept box
+        becomes the score-weighted mean of the boxes of its class that its suppression test claims; the detections,
+        scores and classes are those of the call without it."""
         if nms not in ops.NMS_KINDS:
             raise ValueError(f"nms={nms!r}: expected one of {ops.NMS_KINDS}")
+        if box_voting and nms.startswith("soft_"):
+            raise ValueError(f"box_voting=True needs nms='hard' or 'diou', not {nms!r}")
         (_, _, height, width) = inputs[0].shape
         flat_feats = self._tower_feats(inputs)
         loc_logits = self._tower("loc_head", flat_feats).squeeze(2)
@@ -348,7 +355,8 @@ class ObjectDetection(nn.Module):
         if mode is None:
             mode = "dense" if loc_logits.dtype == torch.float32 else "candidate_first"
         return ops.dense_postprocess(loc_logits, cls_logits, box_raw, self._level_sizes(inputs), int(width), int(height),
-                                     score_threshold, iou_threshold, self.max_instances, mode=mode, nms=nms, sigma=sigma)
+                                     score_threshold, iou_threshold, self.max_instances, mode=mode, nms=nms, sigma=sigma,
+                                     box_voting=box_voting)
 
     # ------------------------------------------------------------------ training
     def _reduce_sums(self) -> Optional[callable]:

@@ -638,6 +638,22 @@ def nms_topk(cand: CandidateBuffers, batch: int, iou_thr: float, k: int, out: Op
     return out
 
 
+def box_vote_topk(cand: CandidateBuffers, batch: int, iou_thr: float, out: tuple, overlap: str = "iou"):
+    """Box voting (merge-NMS, YOLOv5's ``merge=True``) after :func:`nms_topk`: every kept box of ``out`` is replaced, in
+    place, by the score-weighted mean of the boxes of its image's list and class that its suppression test claims
+    (``overlap`` and ``iou_thr`` as in the NMS call, which must not have reset the counts).  Returns ``out``."""
+    infix = _overlap_infix(overlap)
+    num, _, classes, boxes = out
+    k = int(boxes.shape[1])
+    dev = cand.count.device
+    name = f"sihl_od_{infix}box_vote_topk"
+    with _on(dev):
+        rc = getattr(_lib(), name)(_p(cand.count), cand.capacity, _p(cand.key), _p(cand.box), _p(cand.cls), int(batch),
+                                   float(iou_thr), k, _p(num), _p(classes), _p(boxes), _stream(dev))
+    _native.check(rc, name)
+    return out
+
+
 SOFT_NMS_METHODS = {"linear": 1, "gaussian": 2}          # SIHL_OD_SOFT_NMS_LINEAR / _GAUSSIAN (sihl_od.h)
 NMS_KINDS = ("hard", "diou", "soft_linear", "soft_gaussian")
 
@@ -677,16 +693,20 @@ def soft_nms_topk(cand: CandidateBuffers, batch: int, method, iou_thr: float, si
 def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, levels, img_w: int, img_h: int,
                       score_thr: float = 0.05, iou_thr: float = 0.5, max_instances: int = 100,
                       cand: Optional[CandidateBuffers] = None, mode: str = "dense", split_nms: Optional[bool] = None,
-                      nms: str = "hard", sigma: float = 0.5):
+                      nms: str = "hard", sigma: float = 0.5, box_voting: bool = False):
     """Extension (no reference counterpart): dense decode of every location + class-aware NMS.
     Output format of ``ObjectDetection.forward`` (ref :122), zero padded past ``num_instances``.
     ``mode``: see :func:`dense_decode` (identical results).  ``split_nms``: class-split NMS (default: whenever the
     lists can hold more than ``SPLIT_NMS_FROM`` candidates).  ``nms``: ``"hard"`` (greedy, torchvision's semantics),
     ``"diou"`` (greedy DIoU-NMS with ``iou_thr`` as the DIoU threshold), ``"soft_linear"`` (Soft-NMS with ``iou_thr`` as
     Nt) or ``"soft_gaussian"`` (Soft-NMS with ``sigma``); the soft methods keep decaying scores down to ``score_thr``
-    and ignore ``split_nms``."""
+    and ignore ``split_nms``.  ``box_voting`` (``"hard"`` / ``"diou"`` only): each kept box becomes the score-weighted
+    mean of the boxes of its class that its suppression test claims (:func:`box_vote_topk`); the kept set, scores and
+    classes are those of the call without voting."""
     if nms not in NMS_KINDS:
         raise ValueError(f"nms={nms!r}: expected one of {NMS_KINDS}")
+    if box_voting and nms.startswith("soft_"):
+        raise ValueError(f"box_voting=True needs nms='hard' or 'diou', not {nms!r}")
     B, A = loc_logits.shape
     offsets, scales, _ = anchor_tables(levels, img_w, img_h, loc_logits.device)
     if cand is None:
@@ -701,7 +721,11 @@ def dense_postprocess(loc_logits: Tensor, cls_logits: Tensor, box_raw: Tensor, l
         # 3x cheaper than three launches (measured: profiles/r01_postprocess_sweep.json)
         n_sub = min(32, max(2, -(-cand.capacity // 2048)))
         split_nms = cand.capacity >= SPLIT_NMS_FROM and B * n_sub <= 296
-    return nms_topk(cand, B, iou_thr, max_instances, split=split_nms, overlap="diou" if nms == "diou" else "iou")
+    overlap = "diou" if nms == "diou" else "iou"
+    out = nms_topk(cand, B, iou_thr, max_instances, split=split_nms, overlap=overlap)
+    if box_voting:
+        box_vote_topk(cand, B, iou_thr, out, overlap=overlap)
+    return out
 
 
 def batched_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: float,
@@ -734,6 +758,42 @@ def batched_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: floa
     if single:
         return keep[: int(count.item())]
     return keep[:N], count
+
+
+def batched_box_vote(boxes: Tensor, scores: Tensor, idxs: Tensor, keep: Tensor, iou_threshold: float,
+                     keep_count: Optional[Tensor] = None, seg_offsets: Optional[Tensor] = None, overlap: str = "iou"):
+    """Box voting (merge-NMS) after :func:`batched_nms` with the same inputs, threshold and ``overlap``: the voted box
+    of every kept index, the score-weighted mean of the boxes of its segment and class that its suppression test
+    claims.  Without ``seg_offsets``: ``keep`` is the single segment's result and the return value is ``[len(keep), 4]``.
+    With ``seg_offsets``: ``keep`` and ``keep_count`` are :func:`batched_nms`'s and the return value is ``[N, 4]``,
+    aligned with ``keep`` (zero past ``keep_count`` in every segment).  No host synchronisation."""
+    infix = _overlap_infix(overlap)
+    boxes = _req(boxes, torch.float32, "boxes", 2)
+    scores = _req(scores, torch.float32, "scores", 1)
+    idxs = _req(idxs, torch.int64, "idxs", 1)
+    keep = _req(keep, torch.int64, "keep", 1)
+    dev = boxes.device
+    N = scores.numel()
+    if seg_offsets is None:
+        seg_offsets = torch.tensor([0, N], dtype=torch.int32, device=dev)
+        rows = keep.numel()
+        keep_count = torch.full((1,), rows, dtype=torch.int32, device=dev)
+    else:
+        if keep_count is None:
+            raise ValueError("batched_box_vote with seg_offsets needs batched_nms's keep_count")
+        seg_offsets = _req(seg_offsets, torch.int32, "seg_offsets", 1)
+        keep_count = _req(keep_count, torch.int32, "keep_count", 1)
+        rows = N
+    n_images = seg_offsets.numel() - 1
+    voted = torch.zeros((max(rows, 1), 4), dtype=torch.float32, device=dev)
+    if rows == 0:
+        return voted[:0]
+    name = f"sihl_od_batched_{infix}box_vote"
+    with _on(dev):
+        rc = getattr(_lib(), name)(_p(boxes), _p(scores), _p(idxs), _p(seg_offsets), n_images, N, float(iou_threshold),
+                                   _p(keep), _p(keep_count), _p(voted), _stream(dev))
+    _native.check(rc, name)
+    return voted[:rows]
 
 
 def batched_soft_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, max_output: int, method="gaussian",
