@@ -471,6 +471,32 @@ SIHL_OD_API int sihl_od_batched_diou_nms(const float *boxes, const float *scores
                         float diou_thr, int64_t *keep, int32_t *keep_count,
                         void *workspace, void *stream);
 
+/* Class-aware greedy NMS over quadrilaterals (text lines, documents, oriented objects; mmcv's nms_quadri) with the
+ * contract of sihl_od_batched_nms: quads [N, 4, 2] fp32 (four points (x, y) in pixels, finite), scores [N], classes
+ * int64 [N] in [0, 2^32), seg_offsets int32 [n_images+1] (device).  Per segment, visit by (score desc, index asc); a
+ * kept quad i suppresses every later quad j of its class with quad_iou(i, j) > iou_thr.  keep / keep_count as in
+ * sihl_od_batched_nms.  quad_iou is the IoU of the CONVEX HULLS of the two vertex sets, in fp32:
+ *   - for convex quads the polygon IoU, whatever the start vertex and orientation (CW or CCW); bit-identical under any
+ *     permutation of a quad's vertices; non-convex or self-intersecting vertex orders are taken by their hull;
+ *   - 0 when either hull has zero area (collinear or repeated points) and when the AABBs do not overlap (an overlap of
+ *     zero width counts as none);
+ *   - inter clamped to [0, min(area_i, area_j)], iou = inter / ((area_i + area_j) - inter), 0 unless the union > 0;
+ *   - quad_iou(i, j) and quad_iou(j, i) are the same bits.
+ * So a negative iou_thr also suppresses same-class quads that do not overlap.  At most 90 000 quads per call (the
+ * suppression mask takes up to N^2/64 words): larger n returns SIHL_OD_EINVAL.  Every n runs the whole-GPU bitmask
+ * path; many segments go in one call.  workspace: sihl_od_batched_quad_nms_workspace_bytes(n) bytes (0 for n = 0, when
+ * NULL is accepted; 0 as well for n outside [0, 90 000]).  No host synchronisation: the call can be captured in a
+ * CUDA graph. */
+SIHL_OD_API size_t sihl_od_batched_quad_nms_workspace_bytes(int64_t n);
+SIHL_OD_API int sihl_od_batched_quad_nms(const float *quads, const float *scores, const int64_t *classes,
+                        const int32_t *seg_offsets, int n_images, int64_t n,
+                        float iou_thr, int64_t *keep, int32_t *keep_count,
+                        void *workspace, void *stream);
+
+/* out[i * nb + j] = quad_iou(a_i, b_j) (the overlap above) for quads a [na, 4, 2] and b [nb, 4, 2], fp32 [na, nb]
+ * (device), one thread per pair; na * nb <= 2^38. */
+SIHL_OD_API int sihl_od_quad_iou(const float *a, int64_t na, const float *b, int64_t nb, float *out, void *stream);
+
 /* Class-aware box voting (merge-NMS; Gidaris & Komodakis, ICCV 2015; YOLOv5's non_max_suppression(merge=True)), one
  * pass after a greedy NMS (IoU or DIoU) that moves the coordinates of the kept boxes only.  For every emitted
  * detection k of class c, with the overlap and the threshold of the selection it follows (iou_thr / diou_thr):

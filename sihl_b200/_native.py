@@ -63,6 +63,9 @@ _SIGNATURES = {
     "sihl_od_diou_nms_topk": (I, [P, I64, P, P, P, I, F, I, P, P, P, P, P, I, P]),
     "sihl_od_diou_nms_topk_split": (I, [P, I64, P, P, P, I, F, I, P, P, P, P, P, I, P]),
     "sihl_od_batched_diou_nms": (I, [P, P, P, P, I, I64, F, P, P, P, P]),
+    "sihl_od_batched_quad_nms_workspace_bytes": (C.c_size_t, [I64]),
+    "sihl_od_batched_quad_nms": (I, [P, P, P, P, I, I64, F, P, P, P, P]),
+    "sihl_od_quad_iou": (I, [P, I64, P, I64, P, P]),
     "sihl_od_box_vote_topk": (I, [P, I64, P, P, P, I, F, I, P, P, P, P]),
     "sihl_od_diou_box_vote_topk": (I, [P, I64, P, P, P, I, F, I, P, P, P, P]),
     "sihl_od_batched_box_vote": (I, [P, P, P, P, I, I64, F, P, P, P, P]),

@@ -89,6 +89,150 @@ SIHL_HD float diou_pair(Box4 a, float area_a, Box4 b, float area_b)
     return iou - (cd / diag);
 }
 
+// ---- quadrilateral overlap (sihl_od_batched_quad_nms, sihl_od_quad_iou) -------------------------------------------------
+// A quad is 4 finite points (x, y) in pixels (finite is a precondition).  The overlap of two quads is the IoU of the
+// CONVEX HULLS of their vertex sets: for a convex quad that is the polygon IoU whatever its start vertex and orientation,
+// and a non-convex or self-intersecting ("bow-tie") vertex order still gets a defined value.
+//   - The hull is a function of the point SET (the points are sorted first), so the result is bit-identical under any
+//     permutation of a quad's vertices.
+//   - A hull of zero area (collinear or repeated points) has IoU 0 with everything.  Disjoint AABBs give exactly 0, and
+//     an AABB overlap of zero width counts as disjoint.
+//   - inter is clamped to [0, min(area_a, area_b)];  iou = inter / ((area_a + area_b) - inter), 0 unless the union > 0.
+//   - quad_iou(a, b) and quad_iou(b, a) are the same bits: the pair is put in a canonical order first.
+//   - fp32 throughout, with +,-,*,/, explicit fmaf and comparisons only: -fmad=false on the device and -ffp-contract=off
+//     on the host give the same bits.  Hull areas are taken about the hull's first vertex and the intersection about the lower corner of
+//     the AABB intersection, never about the image origin, where shoelace terms of a small quad at x ~ 4096 cancel.
+//   - The intersection clips hull A by the edges of hull B (Sutherland-Hodgman): every intermediate result is one closed
+//     polygon, so a shared or touching edge whose side tests come out as rounding noise changes the area by noise only.
+
+// Per-quad form, computed once per item: hull vertices CCW (3 of them repeat the third in slot 3; a zero-area hull has
+// area 0), the hull area and the AABB of the points.
+struct QuadHull {
+    float x[4], y[4];
+    float area;
+    float x1, y1, x2, y2;
+};
+
+// ax * by - ay * bx with Kahan's difference of products (two fmaf, within 1.5 ulp): the plain form loses all digits of a
+// thin slanted quad's area to cancellation.  fmaf is correctly rounded on the device and in the host's libm alike.
+SIHL_HD float cross2(float ax, float ay, float bx, float by)
+{
+    const float w = ay * bx;
+    const float e = fmaf(-ay, bx, w);
+    const float f = fmaf(ax, by, -w);
+    return f + e;
+}
+
+// compare-exchange on (x, y) lexicographic order
+SIHL_HD void pt_sort2(float &ax, float &ay, float &bx, float &by)
+{
+    if (bx < ax || (bx == ax && by < ay)) {
+        const float tx = ax, ty = ay;
+        ax = bx; ay = by; bx = tx; by = ty;
+    }
+}
+
+// p: x0, y0, x1, y1, x2, y2, x3, y3.  Andrew's monotone chain unrolled for four points.
+SIHL_HD QuadHull quad_hull(const float *p)
+{
+    float x0 = p[0] + 0.f, y0 = p[1] + 0.f, x1 = p[2] + 0.f, y1 = p[3] + 0.f;   // + 0: -0 becomes +0, one order of zeros
+    float x2 = p[4] + 0.f, y2 = p[5] + 0.f, x3 = p[6] + 0.f, y3 = p[7] + 0.f;
+    QuadHull h;
+    h.x1 = fminf(fminf(x0, x1), fminf(x2, x3)); h.x2 = fmaxf(fmaxf(x0, x1), fmaxf(x2, x3));
+    h.y1 = fminf(fminf(y0, y1), fminf(y2, y3)); h.y2 = fmaxf(fmaxf(y0, y1), fmaxf(y2, y3));
+    pt_sort2(x0, y0, x1, y1); pt_sort2(x2, y2, x3, y3);
+    pt_sort2(x0, y0, x2, y2); pt_sort2(x1, y1, x3, y3);
+    pt_sort2(x1, y1, x2, y2);
+    // p0 and p3 are hull vertices; p1 / p2 lie below (c < 0), above (c > 0) or on the chord p0 -> p3
+    const float dx = x3 - x0, dy = y3 - y0;
+    const float c1 = cross2(dx, dy, x1 - x0, y1 - y0), c2 = cross2(dx, dy, x2 - x0, y2 - y0);
+    bool k1 = c1 != 0.f, k2 = c2 != 0.f;
+    if (c1 < 0.f && c2 < 0.f) {                             // both on the lower chain p0, p1, p2, p3
+        k1 = cross2(x1 - x0, y1 - y0, x2 - x0, y2 - y0) > 0.f;
+        k2 = !k1 || cross2(x2 - x1, y2 - y1, x3 - x1, y3 - y1) > 0.f;
+    } else if (c1 > 0.f && c2 > 0.f) {                      // both on the upper chain p3, p2, p1, p0
+        k2 = cross2(x2 - x3, y2 - y3, x1 - x3, y1 - y3) > 0.f;
+        k1 = !k2 || cross2(x1 - x2, y1 - y2, x0 - x2, y0 - y2) > 0.f;
+    }
+    // CCW: p0, the kept lower points by x, p3, the kept upper points by decreasing x
+    float hx[4] = {x0, x0, x0, x0}, hy[4] = {y0, y0, y0, y0};
+    int m = 1;
+    if (k1 && c1 < 0.f) { hx[m] = x1; hy[m] = y1; ++m; }
+    if (k2 && c2 < 0.f) { hx[m] = x2; hy[m] = y2; ++m; }
+    hx[m] = x3; hy[m] = y3; ++m;
+    if (k2 && c2 > 0.f) { hx[m] = x2; hy[m] = y2; ++m; }
+    if (k1 && c1 > 0.f) { hx[m] = x1; hy[m] = y1; ++m; }
+    for (int i = m; i < 4; ++i) { hx[i] = hx[m - 1]; hy[i] = hy[m - 1]; }
+    for (int i = 0; i < 4; ++i) { h.x[i] = hx[i]; h.y[i] = hy[i]; }
+    const float t1 = cross2(hx[1] - hx[0], hy[1] - hy[0], hx[2] - hx[0], hy[2] - hy[0]);
+    const float t2 = cross2(hx[2] - hx[0], hy[2] - hy[0], hx[3] - hx[0], hy[3] - hy[0]);
+    h.area = m < 3 ? 0.f : (t1 + t2) * 0.5f;
+    return h;
+}
+
+// true when hull b comes before hull a in the canonical order of a pair (lexicographic on the vertex slots, which
+// determine the hull; no NaN and no -0 can occur there)
+SIHL_HD bool quad_hull_before(const QuadHull &b, const QuadHull &a)
+{
+    for (int i = 0; i < 4; ++i) {
+        if (b.x[i] != a.x[i]) return b.x[i] < a.x[i];
+        if (b.y[i] != a.y[i]) return b.y[i] < a.y[i];
+    }
+    return false;
+}
+
+constexpr int kQuadClipMax = 8;     // a convex 4-gon clipped by 4 half-planes has at most 8 vertices
+
+// IoU of two hulls.  Sutherland-Hodgman of the first hull of the canonical pair against the second's edges, about the
+// lower corner of the AABB intersection.  A vertex on an edge's line counts as inside; a crossing point is emitted only
+// for a strict sign change.  Rounding on nearly collinear chains could in principle emit more than kQuadClipMax points:
+// those past the cap are dropped, which keeps the result defined and changes the area by rounding noise only.
+SIHL_HD float quad_iou_hulls(const QuadHull &qa, const QuadHull &qb)
+{
+    const bool swap = quad_hull_before(qb, qa);
+    const QuadHull &a = swap ? qb : qa;
+    const QuadHull &b = swap ? qa : qb;
+    const float ox = fmaxf(a.x1, b.x1), oy = fmaxf(a.y1, b.y1);
+    if (!(fminf(a.x2, b.x2) > ox) || !(fminf(a.y2, b.y2) > oy)) return 0.f;
+    if (!(a.area > 0.f) || !(b.area > 0.f)) return 0.f;
+    float px[kQuadClipMax], py[kQuadClipMax], qx[kQuadClipMax], qy[kQuadClipMax];
+    int n = 4;
+    for (int i = 0; i < 4; ++i) { px[i] = a.x[i] - ox; py[i] = a.y[i] - oy; }
+    for (int e = 0; e < 4 && n > 0; ++e) {
+        const float ex = b.x[e] - ox, ey = b.y[e] - oy;
+        const float fx = b.x[(e + 1) & 3] - ox, fy = b.y[(e + 1) & 3] - oy;
+        const float dx = fx - ex, dy = fy - ey;
+        int m = 0;
+        float sc = cross2(dx, dy, px[0] - ex, py[0] - ey);
+        for (int i = 0; i < n; ++i) {
+            const int j = i + 1 < n ? i + 1 : 0;
+            const float sn = cross2(dx, dy, px[j] - ex, py[j] - ey);
+            if (sc >= 0.f) {
+                if (m < kQuadClipMax) { qx[m] = px[i]; qy[m] = py[i]; }
+                ++m;
+            }
+            if ((sc > 0.f && sn < 0.f) || (sc < 0.f && sn > 0.f)) {
+                const float t = sc / (sc - sn);
+                if (m < kQuadClipMax) { qx[m] = px[i] + t * (px[j] - px[i]); qy[m] = py[i] + t * (py[j] - py[i]); }
+                ++m;
+            }
+            sc = sn;
+        }
+        n = m < kQuadClipMax ? m : kQuadClipMax;
+        for (int i = 0; i < n; ++i) { px[i] = qx[i]; py[i] = qy[i]; }
+    }
+    float s = 0.f;                                          // fan about the first vertex: no cancelling terms
+    for (int i = 1; i + 1 < n; ++i) s = s + cross2(px[i] - px[0], py[i] - py[0], px[i + 1] - px[0], py[i + 1] - py[0]);
+    const float lim = fminf(a.area, b.area);
+    float inter = s * 0.5f;
+    inter = inter > 0.f ? (inter < lim ? inter : lim) : 0.f;
+    const float uni = (a.area + b.area) - inter;
+    return uni > 0.f ? inter / uni : 0.f;
+}
+
+// quad_iou of two quads given as 8 floats each
+SIHL_HD float quad_iou(const float *a, const float *b) { return quad_iou_hulls(quad_hull(a), quad_hull(b)); }
+
 // torchvision.ops.complete_box_iou_loss for one row — tv:ops/ciou_loss.py:47-64,
 // tv:ops/diou_loss.py:64-91, tv:ops/_utils.py:87-106.  If grad != nullptr it receives
 // dLoss/d(pred x1,y1,x2,y2) with alpha held constant (ciou_loss.py:61-62) and the

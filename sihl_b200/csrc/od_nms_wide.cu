@@ -20,6 +20,9 @@
 //
 // Memory: the mask needs sum_c n_c * (n_c / 64 + 2) words, bounded by N^2/64 + 3N for N items; the entry point
 // takes this path for 8192 <= N <= 90 000 (1 GiB of mask at most) and the one-CTA-per-segment kernel otherwise.
+//
+// The quadrilateral NMS (sihl_od_batched_quad_nms, end of this file) runs the same pipeline for every N up to 90 000,
+// with its own scatter (hulls) and mask (convex-hull IoU) kernels.
 #include "od_common.cuh"
 
 namespace sihl {
@@ -357,12 +360,124 @@ k_wide_emit(WideBuffers w, const int32_t *__restrict__ seg_offsets, int64_t *__r
     if (tid == 0) keep_count[seg] = running;
 }
 
+// ---- quadrilateral NMS (sihl_od_batched_quad_nms): the same pipeline, with the hull overlap of od_math.h ---------------
+// k_wide_scatter_quad writes the AABB into sbox, the hull area into sarea and the hull vertices into squad (two float4
+// per item, class-major); k_wide_mask_quad tests the AABBs first and clips the hulls only for pairs whose AABBs overlap.
+// Every other step is the box path's kernel.  The quad array is a separate argument: WideBuffers keeps its layout.
+constexpr int kWideQuad = 2;                  // launch_wide_batched_nms's kind for quads (kIoU / kDIoU are the boxes')
+constexpr int64_t kQuadNmsMax = 90000;        // the mask takes up to N^2/64 words: 1 GiB at this size
+
+static size_t quad_nms_workspace_bytes(int64_t n)
+{
+    return n == 0 ? 0 : carve_wide(nullptr, n).bytes + round_up_256((size_t)n * 2 * sizeof(float4));
+}
+
+__global__ void __launch_bounds__(256)
+k_wide_scatter_quad(const float *__restrict__ quads, const int *__restrict__ seg_of, const int32_t *__restrict__ seg_offsets,
+                    int n, WideBuffers w, float4 *__restrict__ squad)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int s0 = __ldg(seg_offsets + __ldg(seg_of + i));
+    const int q = s0 + w.cnt_q[i];
+    float p[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) p[k] = __ldg(quads + (size_t)8 * i + k);
+    const QuadHull h = quad_hull(p);
+    const int cs = s0 + w.cnt_cs[i];
+    w.sbox[q] = make_float4(h.x1, h.y1, h.x2, h.y2);
+    w.sarea[q] = h.area;
+    squad[2 * q] = make_float4(h.x[0], h.y[0], h.x[1], h.y[1]);
+    squad[2 * q + 1] = make_float4(h.x[2], h.y[2], h.x[3], h.y[3]);
+    w.scs[q] = cs;
+    w.sce[q] = cs + w.cnt_len[i];
+    w.sidx[q] = i;
+    w.sr[q] = s0 + w.cnt_r[i];
+    w.kept[q] = 0;
+}
+
+__device__ __forceinline__ QuadHull load_hull(float4 box, float area, float4 v0, float4 v1)
+{
+    QuadHull h;
+    h.x[0] = v0.x; h.y[0] = v0.y; h.x[1] = v0.z; h.y[1] = v0.w;
+    h.x[2] = v1.x; h.y[2] = v1.y; h.x[3] = v1.z; h.y[3] = v1.w;
+    h.area = area;
+    h.x1 = box.x; h.y1 = box.y; h.x2 = box.z; h.y2 = box.w;
+    return h;
+}
+
+// wide_mask's tiling and word layout; the test of a pair is quad_iou_hulls(q, later) > thr, where AABBs that do not
+// overlap (zero width included) give IoU 0 without a clip
+__global__ void __launch_bounds__(64) k_wide_mask_quad(WideBuffers w, const float4 *__restrict__ squad, int n, float thr)
+{
+    __shared__ float4 s_box[64], s_v0[64], s_v1[64];
+    __shared__ float s_area[64];
+    __shared__ int s_cs[64];
+    __shared__ int s_last;
+    const int t = threadIdx.x;
+    const int R = blockIdx.x;
+    const int q = R * 64 + t;
+    const bool have = q < n;
+    const bool apart_hits = 0.f > thr;
+    int cs = 0, ce = 0;
+    long long off = 0;
+    QuadHull hq = load_hull(make_float4(0.f, 0.f, 0.f, 0.f), 0.f, make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f));
+    if (have) {
+        cs = w.scs[q]; ce = w.sce[q]; off = w.rowoff[q];
+        hq = load_hull(w.sbox[q], w.sarea[q], squad[2 * q], squad[2 * q + 1]);
+    }
+    if (t == 0) s_last = 0;
+    __syncthreads();
+    if (have) atomicMax(&s_last, (ce - 1) >> 6);
+    __syncthreads();
+    const int c_first = R + (int)blockIdx.y * kWideColsPerCta;
+    const int c_end = min(s_last, c_first + kWideColsPerCta - 1);
+    for (int Cg = c_first; Cg <= c_end; ++Cg) {            // block-uniform bounds
+        const int qc = Cg * 64 + t;
+        __syncthreads();
+        if (qc < n) {
+            s_box[t] = w.sbox[qc]; s_area[t] = w.sarea[qc]; s_cs[t] = w.scs[qc];
+            s_v0[t] = squad[2 * qc]; s_v1[t] = squad[2 * qc + 1];
+        } else {
+            s_cs[t] = -1;
+        }
+        __syncthreads();
+        if (!have || Cg > ((ce - 1) >> 6)) continue;       // past this row's class segment
+        unsigned long long word = 0ull;
+        const int b0 = Cg == R ? t + 1 : 0;                // only later quads (q' > q)
+        for (int b = b0; b < 64; ++b) {
+            if (s_cs[b] != cs) continue;
+            const float4 bb = s_box[b];
+            const bool apart = !(fminf(hq.x2, bb.z) > fmaxf(hq.x1, bb.x)) || !(fminf(hq.y2, bb.w) > fmaxf(hq.y1, bb.y));
+            const bool hit = apart ? apart_hits : quad_iou_hulls(hq, load_hull(bb, s_area[b], s_v0[b], s_v1[b])) > thr;
+            if (hit) word |= 1ull << b;
+        }
+        w.mask[off + (Cg - (cs >> 6))] = word;
+    }
+}
+
+// sihl_od_quad_iou: one thread per pair
+__global__ void __launch_bounds__(256)
+k_quad_iou(const float *__restrict__ a, int64_t na, const float *__restrict__ b, int64_t nb, float *__restrict__ out)
+{
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= na * nb) return;
+    const int64_t i = k / nb, j = k - i * nb;
+    float pa[8], pb[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) { pa[c] = __ldg(a + 8 * i + c); pb[c] = __ldg(b + 8 * j + c); }
+    out[k] = quad_iou(pa, pb);
+}
+
+// kind: kIoU / kDIoU (boxes [N, 4]) or kWideQuad (quads [N, 8]: needs quad_nms_workspace_bytes(n), of which the first
+// carve_wide(n).bytes are the box path's buffers)
 int launch_wide_batched_nms(const float *boxes, const float *scores, const int64_t *classes, const int32_t *seg_offsets,
                             int n_images, int64_t n64, int kind, float iou_thr, int64_t *keep, int32_t *keep_count,
                             void *workspace, cudaStream_t st)
 {
     const int n = (int)n64;
     WideBuffers w = carve_wide(workspace, n64);
+    float4 *squad = reinterpret_cast<float4 *>(static_cast<unsigned char *>(workspace) + w.bytes);
     int rc = cuda_status(cudaMemsetAsync(w.cnt_q, 0, (size_t)4 * n * sizeof(int), st), "cudaMemsetAsync(wide counters)");
     if (rc) return rc;
     const int nb = (n + 255) / 256;
@@ -371,13 +486,15 @@ int launch_wide_batched_nms(const float *boxes, const float *scores, const int64
     const dim3 cgrid((unsigned)((n + kWideITile - 1) / kWideITile), (unsigned)((n + kWideJSlab - 1) / kWideJSlab));
     k_wide_count<<<cgrid, kWideITile, 0, st>>>(w.akey, w.seg_of, seg_offsets, n, w.cnt_q, w.cnt_r, w.cnt_cs, w.cnt_len);
     SIHL_CHECK_LAUNCH("k_wide_count");
-    k_wide_scatter<<<nb, 256, 0, st>>>(reinterpret_cast<const float4 *>(boxes), w.seg_of, seg_offsets, n, w);
+    if (kind == kWideQuad) k_wide_scatter_quad<<<nb, 256, 0, st>>>(boxes, w.seg_of, seg_offsets, n, w, squad);
+    else k_wide_scatter<<<nb, 256, 0, st>>>(reinterpret_cast<const float4 *>(boxes), w.seg_of, seg_offsets, n, w);
     SIHL_CHECK_LAUNCH("k_wide_scatter");
     k_wide_rowoff<<<1, 1024, 0, st>>>(w.scs, w.sce, n, w.rowoff);
     SIHL_CHECK_LAUNCH("k_wide_rowoff");
     const int tiles = (n + 63) / 64;
     const dim3 mgrid((unsigned)tiles, (unsigned)((tiles + kWideColsPerCta - 1) / kWideColsPerCta));
-    if (kind == kDIoU) k_wide_mask_diou<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
+    if (kind == kWideQuad) k_wide_mask_quad<<<mgrid, 64, 0, st>>>(w, squad, n, iou_thr);
+    else if (kind == kDIoU) k_wide_mask_diou<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
     else k_wide_mask<<<mgrid, 64, 0, st>>>(w, n, iou_thr);
     SIHL_CHECK_LAUNCH("k_wide_mask");
     k_wide_reduce<<<tiles, kReduceThreads, 0, st>>>(w, n);
@@ -390,3 +507,40 @@ int launch_wide_batched_nms(const float *boxes, const float *scores, const int64
 }
 
 }  // namespace sihl
+
+using namespace sihl;
+
+extern "C" size_t sihl_od_batched_quad_nms_workspace_bytes(int64_t n)
+{
+    return n >= 0 && n <= kQuadNmsMax ? quad_nms_workspace_bytes(n) : 0;
+}
+
+extern "C" int sihl_od_batched_quad_nms(const float *quads, const float *scores, const int64_t *classes,
+                                        const int32_t *seg_offsets, int n_images, int64_t n, float iou_thr, int64_t *keep,
+                                        int32_t *keep_count, void *workspace, void *stream)
+{
+    SIHL_CHECK_ARG(seg_offsets && keep_count, "NULL argument");
+    SIHL_CHECK_ARG(n >= 0 && n_images >= 0, "bad sizes");
+    SIHL_CHECK_ARG(n <= kQuadNmsMax, "n=%lld quads: sihl_od_batched_quad_nms takes at most %lld", (long long)n,
+                   (long long)kQuadNmsMax);
+    SIHL_CHECK_ARG(n == 0 || (quads && scores && classes && keep), "NULL argument");
+    SIHL_CHECK_ARG(workspace != nullptr || n == 0, "workspace needed for n=%lld", (long long)n);
+    if (n_images == 0) return SIHL_OD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n == 0)
+        return cuda_status(cudaMemsetAsync(keep_count, 0, (size_t)n_images * sizeof(int32_t), st), "cudaMemsetAsync(keep_count)");
+    return launch_wide_batched_nms(quads, scores, classes, seg_offsets, n_images, n, kWideQuad, iou_thr, keep, keep_count,
+                                   workspace, st);
+}
+
+extern "C" int sihl_od_quad_iou(const float *a, int64_t na, const float *b, int64_t nb, float *out, void *stream)
+{
+    SIHL_CHECK_ARG(na >= 0 && nb >= 0 && na < (1ll << 31) && nb < (1ll << 31), "bad sizes");
+    SIHL_CHECK_ARG(na * nb <= (1ll << 38), "na * nb = %lld pairs: at most 2^38", (long long)(na * nb));
+    if (na == 0 || nb == 0) return SIHL_OD_OK;
+    SIHL_CHECK_ARG(a && b && out, "NULL argument");
+    const int64_t blocks = (na * nb + 255) / 256;
+    k_quad_iou<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, na, b, nb, out);
+    SIHL_CHECK_LAUNCH("k_quad_iou");
+    return SIHL_OD_OK;
+}

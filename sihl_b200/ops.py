@@ -836,6 +836,66 @@ def batched_soft_nms(boxes: Tensor, scores: Tensor, idxs: Tensor, max_output: in
     return keep[:N], keep_scores[:N], count
 
 
+QUAD_NMS_MAX = 90000            # quads per batched_quad_nms call (sihl_od.h)
+
+
+def _req_quads(quads: Tensor, name: str) -> Tensor:
+    """``[N, 4, 2]`` or ``[N, 8]`` fp32 CUDA quads -> contiguous ``[N, 8]``."""
+    if isinstance(quads, Tensor) and not (quads.dim() == 2 and quads.shape[1] == 8) and \
+            not (quads.dim() == 3 and tuple(quads.shape[1:]) == (4, 2)):
+        raise ValueError(f"{name}: expected [N, 4, 2] or [N, 8], got shape {tuple(quads.shape)}")
+    return _req(quads, torch.float32, name).reshape(-1, 8)
+
+
+def batched_quad_nms(quads: Tensor, scores: Tensor, idxs: Tensor, iou_threshold: float,
+                     seg_offsets: Optional[Tensor] = None):
+    """Class-aware greedy NMS over quadrilaterals with :func:`batched_nms`'s contract: ``quads`` ``[N, 4, 2]`` or
+    ``[N, 8]`` (four points (x, y) in pixels), and the overlap is the IoU of the convex hulls of the two vertex sets
+    (``sihl_od.h``; see :func:`quad_iou`).  With ``seg_offsets`` (int32 ``[n_images+1]``) returns ``(keep [N] i64,
+    keep_count [n_images] i32)`` without a host synchronisation; without it, the kept indices of the single segment (one
+    deliberate sync to size the result).  At most ``QUAD_NMS_MAX`` quads per call."""
+    if isinstance(quads, Tensor) and quads.shape[0] > QUAD_NMS_MAX:
+        raise ValueError(f"batched_quad_nms takes at most {QUAD_NMS_MAX} quads per call, got {quads.shape[0]}")
+    quads = _req_quads(quads, "quads")
+    scores = _req(scores, torch.float32, "scores", 1)
+    idxs = _req(idxs, torch.int64, "idxs", 1)
+    dev = quads.device
+    N = scores.numel()
+    if quads.shape[0] != N or idxs.numel() != N:
+        raise ValueError(f"quads, scores and idxs disagree on N: {quads.shape[0]}, {N}, {idxs.numel()}")
+    single = seg_offsets is None
+    if single:
+        seg_offsets = torch.tensor([0, N], dtype=torch.int32, device=dev)
+    else:
+        seg_offsets = _req(seg_offsets, torch.int32, "seg_offsets", 1)
+    n_images = seg_offsets.numel() - 1
+    keep = torch.empty((max(N, 1),), dtype=torch.int64, device=dev)
+    count = torch.zeros((n_images,), dtype=torch.int32, device=dev)
+    ws_bytes = int(_lib().sihl_od_batched_quad_nms_workspace_bytes(N))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev) if ws_bytes else None
+    with _on(dev):
+        rc = _lib().sihl_od_batched_quad_nms(_p(quads), _p(scores), _p(idxs), _p(seg_offsets), n_images, N,
+                                             float(iou_threshold), _p(keep), _p(count), _p(ws), _stream(dev))
+    _native.check(rc, "sihl_od_batched_quad_nms")
+    if single:
+        return keep[: int(count.item())]
+    return keep[:N], count
+
+
+def quad_iou(a: Tensor, b: Tensor) -> Tensor:
+    """``[Na, Nb]`` fp32 IoU of the convex hulls of the quads ``a`` and ``b`` (``[N, 4, 2]`` or ``[N, 8]``): the polygon
+    IoU for convex quads whatever their start vertex and orientation, 0 for a zero-area hull or AABBs that do not
+    overlap, and the same bits for (a, b) and (b, a).  The overlap :func:`batched_quad_nms` compares with its threshold."""
+    a = _req_quads(a, "a")
+    b = _req_quads(b, "b")
+    dev = a.device
+    out = torch.empty((a.shape[0], b.shape[0]), dtype=torch.float32, device=dev)
+    with _on(dev):
+        rc = _lib().sihl_od_quad_iou(_p(a), a.shape[0], _p(b), b.shape[0], _p(out), _stream(dev))
+    _native.check(rc, "sihl_od_quad_iou")
+    return out
+
+
 # --------------------------------------------------------------------------- N3: matching for the validation mAP
 COCO_IOU_THRESHOLDS = tuple(0.5 + 0.05 * i for i in range(10))
 COCO_AREA_RANGES = ((0.0, 1e5 ** 2), (0.0, 32.0 ** 2), (32.0 ** 2, 96.0 ** 2), (96.0 ** 2, 1e5 ** 2))    # all, small, medium, large

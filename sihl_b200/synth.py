@@ -147,6 +147,39 @@ def nms_candidates_np(seed: int, n: int, size: int, num_classes: int = 80):
     return boxes, scores, classes
 
 
+def quad_candidates_np(seed: int, n: int, size: int, num_classes: int = 80):
+    """Quadrilateral NMS inputs: quads [n, 4, 2] f32 (four points (x, y) in [0, size]), scores U(0.05, 1) f32, classes
+    int64.  Rotated rectangles (sides U(4, 0.15*S) x U(2, 0.05*S), any angle) with vertex jitter, in clusters of up to
+    8 near-duplicates of one class (a detector's overlapping proposals) and, for a quarter of the clusters, a parallel
+    neighbour shifted across its short side (slanted text lines: high AABB IoU, little or no polygon overlap)."""
+    rng = np.random.RandomState(seed)
+    quads = np.empty((n, 4, 2), np.float64)
+    classes = np.empty(n, np.int64)
+    i = 0
+    while i < n:
+        m = min(n - i, int(rng.randint(1, 9)))
+        w, h = rng.uniform(4, 0.15 * size), rng.uniform(2, 0.05 * size)
+        th = rng.uniform(-np.pi, np.pi)
+        cx, cy = rng.uniform(0, size), rng.uniform(0, size)
+        c, s = np.cos(th), np.sin(th)
+        cls = rng.randint(0, num_classes)
+        for k in range(m):
+            if k == 1 and rng.rand() < 0.25:                      # parallel neighbour, one to two line heights away
+                off = h * rng.uniform(1.0, 2.0)
+                ccx, ccy, ww, hh = cx - s * off, cy + c * off, w, h
+            else:                                                 # near-duplicate
+                ccx, ccy = cx + rng.normal(0, 0.1 * h), cy + rng.normal(0, 0.1 * h)
+                ww, hh = w * rng.uniform(0.9, 1.1), h * rng.uniform(0.9, 1.1)
+            dx, dy = np.array([-ww, ww, ww, -ww]) / 2, np.array([-hh, -hh, hh, hh]) / 2
+            q = np.stack([ccx + c * dx - s * dy, ccy + s * dx + c * dy], 1)
+            quads[i] = q + rng.normal(0, 0.03 * hh, (4, 2))
+            classes[i] = cls
+            i += 1
+    quads = np.clip(quads, 0, size).astype(np.float32)
+    scores = rng.uniform(0.05, 1.0, n).astype(np.float32)
+    return quads, scores, classes
+
+
 # ----------------------------------------------------------------------------
 # device-side generator for bench.py (torch imported lazily: synth is also used
 # by numpy-only code)
