@@ -582,6 +582,25 @@ SIHL_OD_API int sihl_od_map_match(const float *det_boxes, const float *det_score
                       int32_t *det_order, int32_t *dt_match, uint8_t *dt_ignore, uint8_t *gt_ignore,
                       void *workspace, void *stream);
 
+/* The same matching for quadrilateral detections (the QuadrilateralDetection head): det_quads [B,K,8] and gt_quads
+ * [total_gt,8] are four points (x, y) in px each, everything else and every output as sihl_od_map_match, in the same
+ * layouts and under the same COCOeval.evaluateImg rule.  Two values change:
+ *   iou(d, g)  = the IoU of the convex hulls of the two vertex sets, the fp32 value of sihl_od_quad_iou (bit-identical
+ *                under any vertex order, 0 for disjoint AABBs or a zero-area hull), widened to double;
+ *   area(q)    = the hull's polygon area in fp32, widened to double, for gts and unmatched detections alike (not the
+ *                AABB's w * h: a thin slanted quad falls in the area range of its polygon).
+ * The hulls are built once per quad and the same-class IoUs of each image are filled into a [K, G_b] matrix over the
+ * whole GPU before the chains run.  K <= 1024, n_thresholds <= 16, n_areas <= 8.  workspace: at least
+ * sihl_od_quad_map_workspace_bytes(batch, k, total_gt, n_thresholds, n_areas) bytes (that query returns 0 for
+ * arguments out of range), passed in workspace_bytes; a shorter one is SIHL_OD_EINVAL.  batch = 0 reads and writes
+ * nothing (its empty arrays may be NULL).  No host synchronisation: the call can be captured in a CUDA graph. */
+SIHL_OD_API size_t sihl_od_quad_map_workspace_bytes(int batch, int k, int total_gt, int n_thresholds, int n_areas);
+SIHL_OD_API int sihl_od_quad_map_match(const float *det_quads, const float *det_scores, const int64_t *det_classes,
+                      int batch, int k, const float *gt_quads, const int64_t *gt_classes, const int32_t *gt_offsets,
+                      int total_gt, const double *iou_thresholds_host, int n_thresholds, const double *area_ranges_host,
+                      int n_areas, int32_t *det_order, int32_t *dt_match, uint8_t *dt_ignore, uint8_t *gt_ignore,
+                      void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---- N4 (SURVEY.md §8f): the per-location MLP towers in front of the hot path ----------------
  * ref object_detection.py:51-61 builds loc / cls / box / iou heads as torchvision ops.MLP(256 -> [256]*num_layers
  * + [out], norm_layer=LayerNorm, activation_layer=SiLU) and applies them to every location (:116, :121, :175).

@@ -56,13 +56,24 @@ __device__ __forceinline__ double box_iou_d(float4 d, float4 g)
     return i / u;
 }
 
-__global__ void __launch_bounds__(128) k_map_match(const __grid_constant__ MapParams p)
+// Where the chains of one image read their geometry: the box kernel computes IoU and area from the xyxy boxes, the quad
+// kernel reads IoU from its precomputed matrix and areas from the hulls.  D is what a chain keeps of its detection.
+struct MapBoxGeometry {
+    const float4 *db, *gb;
+    __device__ __forceinline__ float4 det(int d) const { return __ldg(db + d); }
+    __device__ __forceinline__ double det_area(float4 box) const { return box_area_d(box); }
+    __device__ __forceinline__ double gt_area(int g) const { return box_area_d(__ldg(gb + g)); }
+    __device__ __forceinline__ double iou(float4 box, int g) const { return box_iou_d(box, __ldg(gb + g)); }
+};
+
+// COCOeval.evaluateImg for image b (the rule above): rank the detections, flag the gts per area range, then one greedy
+// chain per (area range, threshold) on a thread.  Shared by k_map_match and k_quad_map_match; inlined into each.
+template <class Geo>
+__device__ __forceinline__ void map_match_image(const MapParams &p, const Geo &geo, int *s_order)
 {
-    __shared__ int s_order[kMapMaxK];
     const int b = blockIdx.x, tid = threadIdx.x, K = p.K;
     const float *sc = p.det_scores + (int64_t)b * K;
     const int64_t *dc = p.det_classes + (int64_t)b * K;
-    const float4 *db = p.det_boxes + (int64_t)b * K;
     const int g0 = __ldg(p.gt_offsets + b), g1 = __ldg(p.gt_offsets + b + 1);
 
     // detections by (score desc, input order): rank by counting (K <= 1024)
@@ -79,7 +90,7 @@ __global__ void __launch_bounds__(128) k_map_match(const __grid_constant__ MapPa
     // ignore flags of this image's gts per area range; clear the "taken" markers
     for (int i = tid; i < (g1 - g0) * p.n_area; i += blockDim.x) {
         const int a = i / (g1 - g0), g = g0 + i % (g1 - g0);
-        const double ar = box_area_d(__ldg(p.gt_boxes + g));
+        const double ar = geo.gt_area(g);
         p.gt_ignore[(int64_t)a * p.total_gt + g] = (ar < p.area_lo[a] || ar > p.area_hi[a]) ? 1 : 0;
     }
     for (int i = tid; i < (g1 - g0) * p.n_area * p.n_thr; i += blockDim.x)
@@ -97,13 +108,13 @@ __global__ void __launch_bounds__(128) k_map_match(const __grid_constant__ MapPa
         for (int r = 0; r < K; ++r) {
             const int d = s_order[r];
             const int64_t cls = __ldg(dc + d);
-            const float4 box = __ldg(db + d);
+            const auto det = geo.det(d);
             double best = thr;
             int m = -1;
             for (int pass = 0; pass < 2 && m < 0; ++pass) {        // regular gts first; ignored ones only while unmatched
                 for (int g = g0; g < g1; ++g) {
                     if (__ldg(p.gt_classes + g) != cls || gig[g] != pass || taken[g] != 0) continue;
-                    const double iou = box_iou_d(box, __ldg(p.gt_boxes + g));
+                    const double iou = geo.iou(det, g);
                     if (iou < best) continue;
                     best = iou;
                     m = g;
@@ -114,12 +125,99 @@ __global__ void __launch_bounds__(128) k_map_match(const __grid_constant__ MapPa
                 dti[r] = gig[m];
                 taken[m] = r + 1;
             } else {
-                const double ar = box_area_d(box);
+                const double ar = geo.det_area(det);
                 dtm[r] = -1;
                 dti[r] = (ar < p.area_lo[a] || ar > p.area_hi[a]) ? 1 : 0;
             }
         }
     }
+}
+
+__global__ void __launch_bounds__(128) k_map_match(const __grid_constant__ MapParams p)
+{
+    __shared__ int s_order[kMapMaxK];
+    const MapBoxGeometry geo{p.det_boxes + (int64_t)blockIdx.x * p.K, p.gt_boxes};
+    map_match_image(p, geo, s_order);
+}
+
+// ---- polygon IoU (sihl_od_quad_map_match): the same chains over quads ----------------------------------------------
+// The overlap is od_math.h's hull IoU, the one sihl_od_batched_quad_nms suppresses with, and the area of a quad is its
+// hull's polygon area.  A clip costs ~40x a box IoU, so it is not recomputed inside the chains (each chain would redo
+// every pair of its image, 40 times per image, on one SM): k_quad_map_hulls builds every hull once, k_quad_map_iou fills
+// the [K, G_b] fp32 IoU block of each image with the pairs spread over the whole GPU, and k_quad_map_match runs the
+// chains above on that matrix.  Image b's block starts at K * gt_offsets[b]: the matrix is K * total_gt floats.
+struct MapQuadGeometry {
+    const float *m;                   // image b's [K, G_b] IoU block
+    const QuadHull *dh, *gh;          // image b's detection hulls; every gt hull
+    int g0, gn;
+    __device__ __forceinline__ int det(int d) const { return d; }
+    __device__ __forceinline__ double det_area(int d) const { return (double)__ldg(&dh[d].area); }
+    __device__ __forceinline__ double gt_area(int g) const { return (double)__ldg(&gh[g].area); }
+    __device__ __forceinline__ double iou(int d, int g) const { return (double)__ldg(m + (int64_t)d * gn + (g - g0)); }
+};
+
+// hulls[i] = quad_hull of detection i (i < n_det = B * K), then of gt i - n_det
+__global__ void __launch_bounds__(256)
+k_quad_map_hulls(const float *__restrict__ det_quads, int64_t n_det, const float *__restrict__ gt_quads, int64_t n_gt,
+                 QuadHull *__restrict__ hulls)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_det + n_gt) return;
+    const float *q = i < n_det ? det_quads + 8 * i : gt_quads + 8 * (i - n_det);
+    float p[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) p[c] = __ldg(q + c);
+    hulls[i] = quad_hull(p);
+}
+
+// One thread per (detection, gt) pair of the same image, grid-stride over the K * total_gt matrix.  Pair k lies in image
+// b with K * g0 <= k < K * g1, i.e. gt_offsets[b] <= k / K < gt_offsets[b + 1].  Pairs of different classes are skipped
+// (the chains test the class first and never read them); every same-class pair is written, an exact 0 included.
+__global__ void __launch_bounds__(256)
+k_quad_map_iou(const QuadHull *__restrict__ hulls, const int64_t *__restrict__ det_classes,
+               const int64_t *__restrict__ gt_classes, const int32_t *__restrict__ gt_offsets, int batch, int K,
+               int total_gt, float *__restrict__ iou)
+{
+    const int64_t n = (int64_t)K * total_gt, n_det = (int64_t)batch * K;
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
+        const int row = (int)(k / K);                       // in [g0, g1) of the pair's image
+        int lo = 0, hi = batch - 1;                         // last b with gt_offsets[b] <= row
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (__ldg(gt_offsets + mid) <= row) lo = mid; else hi = mid - 1;
+        }
+        const int g0 = __ldg(gt_offsets + lo), gn = __ldg(gt_offsets + lo + 1) - g0;
+        const int64_t local = k - (int64_t)K * g0;
+        const int d = (int)(local / gn), g = g0 + (int)(local - (int64_t)d * gn);
+        const int64_t di = (int64_t)lo * K + d;
+        if (__ldg(det_classes + di) != __ldg(gt_classes + g)) continue;
+        iou[k] = quad_iou_hulls(hulls[di], hulls[n_det + g]);
+    }
+}
+
+__global__ void __launch_bounds__(128)
+k_quad_map_match(const __grid_constant__ MapParams p, const float *__restrict__ iou, const QuadHull *__restrict__ hulls)
+{
+    __shared__ int s_order[kMapMaxK];
+    const int b = blockIdx.x, g0 = __ldg(p.gt_offsets + b), g1 = __ldg(p.gt_offsets + b + 1);
+    const MapQuadGeometry geo{iou + (int64_t)p.K * g0, hulls + (int64_t)b * p.K, hulls + (int64_t)gridDim.x * p.K, g0,
+                              g1 - g0};
+    map_match_image(p, geo, s_order);
+}
+
+// workspace: the hulls of every detection and gt, the IoU matrix, the taken markers of the chains
+struct QuadMapWorkspace {
+    size_t hulls, iou, taken, bytes;
+};
+
+static QuadMapWorkspace quad_map_workspace(int batch, int k, int total_gt, int n_thresholds, int n_areas)
+{
+    QuadMapWorkspace w;
+    w.hulls = 0;
+    w.iou = round_up_256(((size_t)batch * k + total_gt) * sizeof(QuadHull));
+    w.taken = w.iou + round_up_256((size_t)k * total_gt * sizeof(float));
+    w.bytes = w.taken + (size_t)(total_gt > 0 ? total_gt : 1) * n_thresholds * n_areas * sizeof(int32_t);
+    return w;
 }
 
 }  // namespace sihl
@@ -156,5 +254,59 @@ extern "C" int sihl_od_map_match(const float *det_boxes, const float *det_scores
     p.gt_taken = reinterpret_cast<int32_t *>(workspace); p.total_gt = total_gt;
     k_map_match<<<batch, 128, 0, (cudaStream_t)stream>>>(p);
     SIHL_CHECK_LAUNCH("k_map_match");
+    return SIHL_OD_OK;
+}
+
+extern "C" size_t sihl_od_quad_map_workspace_bytes(int batch, int k, int total_gt, int n_thresholds, int n_areas)
+{
+    if (batch < 0 || k < 1 || k > kMapMaxK || total_gt < 0 || n_thresholds < 1 || n_thresholds > kMapMaxT ||
+        n_areas < 1 || n_areas > kMapMaxA)
+        return 0;
+    return quad_map_workspace(batch, k, total_gt, n_thresholds, n_areas).bytes;
+}
+
+extern "C" int sihl_od_quad_map_match(const float *det_quads, const float *det_scores, const int64_t *det_classes, int batch,
+                                      int k, const float *gt_quads, const int64_t *gt_classes, const int32_t *gt_offsets,
+                                      int total_gt, const double *iou_thresholds_host, int n_thresholds,
+                                      const double *area_ranges_host, int n_areas, int32_t *det_order, int32_t *dt_match,
+                                      uint8_t *dt_ignore, uint8_t *gt_ignore, void *workspace, size_t workspace_bytes,
+                                      void *stream)
+{
+    SIHL_CHECK_ARG(iou_thresholds_host && area_ranges_host, "NULL thresholds / area ranges");
+    SIHL_CHECK_ARG(batch >= 0 && k >= 1 && k <= kMapMaxK && total_gt >= 0, "bad sizes (k=%d, at most %d detections per image)", k,
+                   kMapMaxK);
+    SIHL_CHECK_ARG(n_thresholds >= 1 && n_thresholds <= kMapMaxT && n_areas >= 1 && n_areas <= kMapMaxA,
+                   "at most %d IoU thresholds and %d area ranges", kMapMaxT, kMapMaxA);
+    if (batch == 0) return SIHL_OD_OK;                  // nothing is read or written: empty tensors may be NULL
+    SIHL_CHECK_ARG(det_quads && det_scores && det_classes && gt_offsets, "NULL input");
+    SIHL_CHECK_ARG(det_order && dt_match && dt_ignore && workspace, "NULL output / workspace");
+    SIHL_CHECK_ARG(total_gt == 0 || (gt_quads && gt_classes && gt_ignore), "NULL ground truth");
+    const QuadMapWorkspace w = quad_map_workspace(batch, k, total_gt, n_thresholds, n_areas);
+    SIHL_CHECK_ARG(workspace_bytes >= w.bytes, "workspace of %zu bytes, %zu needed (sihl_od_quad_map_workspace_bytes)",
+                   workspace_bytes, w.bytes);
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char *ws = static_cast<unsigned char *>(workspace);
+    QuadHull *hulls = reinterpret_cast<QuadHull *>(ws + w.hulls);
+    float *iou = reinterpret_cast<float *>(ws + w.iou);
+    const int64_t n_det = (int64_t)batch * k;
+    k_quad_map_hulls<<<(unsigned)((n_det + total_gt + 255) / 256), 256, 0, st>>>(det_quads, n_det, gt_quads, total_gt, hulls);
+    SIHL_CHECK_LAUNCH("k_quad_map_hulls");
+    if (total_gt > 0) {
+        const int64_t pairs = (int64_t)k * total_gt;
+        const int64_t blocks = (pairs + 255) / 256;
+        k_quad_map_iou<<<(unsigned)(blocks < kNumSMs * 64 ? blocks : kNumSMs * 64), 256, 0, st>>>(
+            hulls, det_classes, gt_classes, gt_offsets, batch, k, total_gt, iou);
+        SIHL_CHECK_LAUNCH("k_quad_map_iou");
+    }
+    MapParams p;
+    p.det_boxes = nullptr; p.det_scores = det_scores; p.det_classes = det_classes; p.K = k;
+    p.gt_boxes = nullptr; p.gt_classes = gt_classes; p.gt_offsets = gt_offsets;
+    p.n_thr = n_thresholds; p.n_area = n_areas;
+    for (int i = 0; i < n_thresholds; ++i) p.thr[i] = iou_thresholds_host[i];
+    for (int i = 0; i < n_areas; ++i) { p.area_lo[i] = area_ranges_host[2 * i]; p.area_hi[i] = area_ranges_host[2 * i + 1]; }
+    p.det_order = det_order; p.dt_match = dt_match; p.dt_ignore = dt_ignore; p.gt_ignore = gt_ignore;
+    p.gt_taken = reinterpret_cast<int32_t *>(ws + w.taken); p.total_gt = total_gt;
+    k_quad_map_match<<<batch, 128, 0, st>>>(p, iou, hulls);
+    SIHL_CHECK_LAUNCH("k_quad_map_match");
     return SIHL_OD_OK;
 }

@@ -7,6 +7,10 @@ COCOeval on the CPU at epoch end.  ``DetectionMAP`` keeps the interface the head
 one greedy chain per IoU threshold x area range, fp64 box IoU) and keeps only the compact match tables; ``compute``
 does COCOeval.accumulate / summarize on them — a few cumulative sums per category on the host.
 
+``iou_type="quad"`` evaluates the QuadrilateralDetection head's four-vertex polygons instead of boxes: the matching is
+``sihl_od_quad_map_match`` (the IoU of the convex hulls of the vertex sets, the hull's polygon area for the area ranges)
+and everything after it is the same.
+
 Parity is UNPINNED: torchmetrics and faster_coco_eval are not installed where this was written; the algorithm is the
 published COCOeval one (see oracle/map_oracle.py, which restates it independently for the tests).
 """
@@ -24,10 +28,17 @@ RECALL_THRESHOLDS = np.linspace(0.0, 1.0, 101)
 
 
 class DetectionMAP:
-    """COCO box mAP / mAR over everything passed to :meth:`update` since construction (or :meth:`reset`)."""
+    """COCO mAP / mAR over everything passed to :meth:`update` since construction (or :meth:`reset`).  ``iou_type``:
+    ``"bbox"`` (xyxy boxes, box IoU) or ``"quad"`` (quads ``[K, 4, 2]`` or ``[K, 8]``, polygon IoU of their hulls)."""
+
+    IOU_TYPES = ("bbox", "quad")
 
     def __init__(self, max_detection_thresholds: Optional[Sequence[int]] = None,
-                 iou_thresholds: Sequence[float] = ops.COCO_IOU_THRESHOLDS, sync_dist: bool = True, **_ignored) -> None:
+                 iou_thresholds: Sequence[float] = ops.COCO_IOU_THRESHOLDS, sync_dist: bool = True,
+                 iou_type: str = "bbox", **_ignored) -> None:
+        if iou_type not in self.IOU_TYPES:
+            raise ValueError(f"iou_type must be one of {self.IOU_TYPES}, got {iou_type!r}")
+        self.iou_type = iou_type
         self.max_dets = sorted(int(m) for m in (max_detection_thresholds or (1, 10, 100)))
         self.iou_thresholds = tuple(float(t) for t in iou_thresholds)
         self.area_ranges = ops.COCO_AREA_RANGES
@@ -43,7 +54,11 @@ class DetectionMAP:
 
     def update(self, preds: List[Dict[str, Tensor]], target: List[Dict[str, Tensor]]) -> None:
         """torchmetrics' signature (ref :230-236): per-image dicts ``scores`` / ``labels`` / ``boxes`` (xyxy px) and
-        ``labels`` / ``boxes``.  Every image must carry the same number of detections (``forward`` returns K rows)."""
+        ``labels`` / ``boxes``.  Every image must carry the same number of detections (``forward`` returns K rows).
+        With ``iou_type="quad"`` both read ``quads`` ([n, 4, 2] or [n, 8] px) in place of ``boxes``."""
+        if self.iou_type == "quad":
+            self._update_quads(preds, target)
+            return
         scores = torch.stack([p["scores"] for p in preds])
         classes = torch.stack([p["labels"] for p in preds])
         boxes = torch.stack([p["boxes"] for p in preds])
@@ -55,16 +70,30 @@ class DetectionMAP:
         gt_classes = torch.cat(gc) if gc else torch.empty((0,), dtype=torch.int64, device=dev)
         self.update_batch(scores, classes, boxes, gt_boxes, gt_classes, counts)
 
+    def _update_quads(self, preds: List[Dict[str, Tensor]], target: List[Dict[str, Tensor]]) -> None:
+        scores = torch.stack([p["scores"] for p in preds])
+        classes = torch.stack([p["labels"] for p in preds])
+        quads = torch.stack([p["quads"].reshape(-1, 8) for p in preds])
+        dev = scores.device
+        counts = [int(t["quads"].shape[0]) for t in target]
+        gq = [t["quads"].as_subclass(Tensor).reshape(-1, 8).to(device=dev, dtype=torch.float32) for t in target]
+        gc = [t["labels"].as_subclass(Tensor).reshape(-1).to(device=dev, dtype=torch.int64) for t in target]
+        gt_quads = torch.cat(gq) if gq else torch.empty((0, 8), device=dev)
+        gt_classes = torch.cat(gc) if gc else torch.empty((0,), dtype=torch.int64, device=dev)
+        self.update_batch(scores, classes, quads, gt_quads, gt_classes, counts)
+
     def update_batch(self, scores: Tensor, classes: Tensor, boxes: Tensor, gt_boxes: Tensor, gt_classes: Tensor,
                      gt_counts: Sequence[int]) -> None:
         """The batched form the drop-in head calls: detections [B,K,...] as ``forward`` returns them, ground truth
-        concatenated with its per-image counts.  Enqueues one kernel; nothing is synchronised."""
+        concatenated with its per-image counts.  Enqueues the matching; nothing is synchronised.  With
+        ``iou_type="quad"``, ``boxes`` / ``gt_boxes`` are quads: [B,K,4,2] or [B,K,8] and [sumG,4,2] or [sumG,8]."""
         dev = scores.device
         off = np.zeros(len(gt_counts) + 1, dtype=np.int32)
         off[1:] = np.cumsum(gt_counts)
         gt_offsets = torch.from_numpy(off).to(dev)
-        res = ops.map_match(boxes.float(), scores, classes, gt_boxes, gt_classes, gt_offsets, self.iou_thresholds,
-                            self.area_ranges)
+        match = ops.quad_map_match if self.iou_type == "quad" else ops.map_match
+        res = match(boxes.float(), scores, classes, gt_boxes, gt_classes, gt_offsets, self.iou_thresholds,
+                    self.area_ranges)
         order = res["det_order"].long()
         self._batches.append(dict(
             scores=torch.gather(scores.float(), 1, order), classes=torch.gather(classes, 1, order),   # by rank

@@ -931,6 +931,59 @@ def map_match(det_boxes: Tensor, det_scores: Tensor, det_classes: Tensor, gt_box
     return dict(det_order=order, dt_match=dtm, dt_ignore=dti, gt_ignore=gti[:, :G])
 
 
+MAP_MAX_K, MAP_MAX_THRESHOLDS, MAP_MAX_AREAS = 1024, 16, 8     # sihl_od_map_match / sihl_od_quad_map_match (sihl_od.h)
+
+
+def quad_map_match(det_quads: Tensor, det_scores: Tensor, det_classes: Tensor, gt_quads: Tensor, gt_classes: Tensor,
+                   gt_offsets: Tensor, iou_thresholds: Sequence[float] = COCO_IOU_THRESHOLDS,
+                   area_ranges: Sequence[Tuple[float, float]] = COCO_AREA_RANGES) -> Dict[str, Tensor]:
+    """:func:`map_match` for quadrilaterals: ``det_quads`` ``[B,K,4,2]`` or ``[B,K,8]``, ``gt_quads`` ``[sumG,4,2]`` or
+    ``[sumG,8]`` (four points (x, y) in px).  The IoU is :func:`quad_iou`'s (convex hulls of the vertex sets) and the area
+    that places a quad in an area range is its hull's polygon area.  Returns the same dict as :func:`map_match`.  Shapes
+    and limits (K <= 1024, at most 16 thresholds and 8 area ranges) are checked before any CUDA call."""
+    if isinstance(det_quads, Tensor) and not (det_quads.dim() == 3 and det_quads.shape[2] == 8) and \
+            not (det_quads.dim() == 4 and tuple(det_quads.shape[2:]) == (4, 2)):
+        raise ValueError(f"det_quads: expected [B, K, 4, 2] or [B, K, 8], got shape {tuple(det_quads.shape)}")
+    if isinstance(det_scores, Tensor) and det_scores.dim() != 2:
+        raise ValueError(f"det_scores: expected [B, K], got shape {tuple(det_scores.shape)}")
+    B, K = (int(v) for v in det_scores.shape)
+    if tuple(det_quads.shape[:2]) != (B, K) or tuple(det_classes.shape) != (B, K):
+        raise ValueError(f"det_quads {tuple(det_quads.shape)}, det_scores {(B, K)} and det_classes "
+                         f"{tuple(det_classes.shape)} disagree on [B, K]")
+    if not 1 <= K <= MAP_MAX_K:
+        raise ValueError(f"quad_map_match takes 1 to {MAP_MAX_K} detections per image, got K={K}")
+    thr = np.ascontiguousarray(np.asarray(iou_thresholds, dtype=np.float64).reshape(-1))
+    areas = np.ascontiguousarray(np.asarray(area_ranges, dtype=np.float64).reshape(-1, 2))
+    T, NA = len(thr), len(areas)
+    if not (1 <= T <= MAP_MAX_THRESHOLDS and 1 <= NA <= MAP_MAX_AREAS):
+        raise ValueError(f"quad_map_match takes 1 to {MAP_MAX_THRESHOLDS} IoU thresholds and 1 to {MAP_MAX_AREAS} area "
+                         f"ranges, got {T} and {NA}")
+    det_quads = _req(det_quads, torch.float32, "det_quads").reshape(B, K, 8)
+    det_scores = _req(det_scores.float() if det_scores.dtype != torch.float32 else det_scores, torch.float32, "det_scores", 2)
+    det_classes = _req(det_classes, torch.int64, "det_classes", 2)
+    gt_quads = _req_quads(gt_quads, "gt_quads")
+    G = int(gt_quads.shape[0])
+    gt_classes = _req(gt_classes, torch.int64, "gt_classes", 1)
+    gt_offsets = _req(gt_offsets, torch.int32, "gt_offsets", 1)
+    if gt_classes.numel() != G or gt_offsets.numel() != B + 1:
+        raise ValueError(f"gt_quads [{G}], gt_classes [{gt_classes.numel()}] and gt_offsets [{gt_offsets.numel()}] "
+                         f"do not describe {B} images")
+    dev = det_quads.device
+    ws_bytes = int(_lib().sihl_od_quad_map_workspace_bytes(B, K, G, T, NA))
+    with _on(dev):
+        order = torch.empty((B, K), dtype=torch.int32, device=dev)
+        dtm = torch.empty((B, NA, T, K), dtype=torch.int32, device=dev)
+        dti = torch.empty((B, NA, T, K), dtype=torch.uint8, device=dev)
+        gti = torch.empty((NA, max(G, 1)), dtype=torch.uint8, device=dev)
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+        rc = _lib().sihl_od_quad_map_match(
+            _p(det_quads), _p(det_scores), _p(det_classes), B, K, _p(gt_quads) if G else None,
+            _p(gt_classes) if G else None, _p(gt_offsets), G, thr.ctypes.data, T, areas.ctypes.data, NA,
+            _p(order), _p(dtm), _p(dti), _p(gti), _p(ws), ws_bytes, _stream(dev))
+    _native.check(rc, "sihl_od_quad_map_match")
+    return dict(det_order=order, dt_match=dtm, dt_ignore=dti, gt_ignore=gti[:, :G])
+
+
 # ---- N4 (SURVEY.md §8f): the per-location MLP towers on the tensor cores -------------------------------------------------
 MLP_CHANNELS = 256                      # the reference's num_channels default; the kernels are built for it
 _MLP_OUT_PADS = (16, 32, 64, 96, 128, 256)

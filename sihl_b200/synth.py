@@ -180,6 +180,63 @@ def quad_candidates_np(seed: int, n: int, size: int, num_classes: int = 80):
     return quads, scores, classes
 
 
+def _rect_corners(cx, cy, w, h, th):
+    """[..., 4, 2] corners of w x h rectangles centred at (cx, cy), rotated by th."""
+    c, s = np.cos(th)[..., None], np.sin(th)[..., None]
+    dx = np.array([-0.5, 0.5, 0.5, -0.5]) * w[..., None]
+    dy = np.array([-0.5, -0.5, 0.5, 0.5]) * h[..., None]
+    return np.stack([cx[..., None] + c * dx - s * dy, cy[..., None] + s * dx + c * dy], -1)
+
+
+def quad_map_batch_np(seed: int, batch: int, k: int, gt_per_image: int, num_classes: int = 80, size: int = 1024,
+                      counts=None):
+    """Quad mAP inputs in the layout of ops.quad_map_match: ground truth = ``counts[b]`` (default ``gt_per_image``)
+    rotated rectangles per image (long side log-uniform in [6, 0.2*S], aspect down to 1:20, any angle); detections
+    [B, K] = jittered copies of a gt of the image (60%: centre, size, angle and vertices perturbed; 90% of them with the
+    gt's class), parallel-line decoys (20%: a copy shifted across its short side by one to two line heights, so its
+    AABB overlaps the gt's and its polygon barely or not) and random rectangles.  Scores are U(0, 1) rounded to two
+    decimals (exact ties).  Returns det_quads [B,K,4,2] f32, det_scores [B,K] f32, det_classes [B,K] i64, gt_quads
+    [sumG,4,2] f32, gt_classes [sumG] i64, gt_offsets [B+1] i32."""
+    rng = np.random.RandomState(seed)
+    counts = np.full(batch, gt_per_image, np.int64) if counts is None else np.asarray(counts, np.int64)
+    offsets = np.zeros(batch + 1, np.int32)
+    offsets[1:] = np.cumsum(counts)
+    G = int(offsets[-1])
+    gw = np.exp(rng.uniform(np.log(6.0), np.log(0.2 * size), G))
+    gh = np.maximum(gw * rng.uniform(0.05, 1.0, G), 3.0)
+    gth = rng.uniform(-np.pi, np.pi, G)
+    gcx, gcy = rng.uniform(0.1 * size, 0.9 * size, G), rng.uniform(0.1 * size, 0.9 * size, G)
+    gt_classes = rng.randint(0, num_classes, G).astype(np.int64)
+    gt_quads = _rect_corners(gcx, gcy, gw, gh, gth)
+    # detections: pick a gt of the image for each row (images without gt get random rectangles only)
+    u = rng.uniform(0, 1, (batch, k))
+    pick = offsets[:-1, None] + np.floor(rng.uniform(0, 1, (batch, k)) * np.maximum(counts, 1)[:, None]).astype(np.int64)
+    has = (counts > 0)[:, None] & np.ones((batch, k), bool)
+    pick = np.where(has, np.minimum(pick, max(G - 1, 0)), 0)
+    copy, decoy = has & (u < 0.6), has & (u >= 0.6) & (u < 0.8)
+    src = lambda a, fill: np.where(has, a[pick] if G else fill, fill)
+    w, h, th = src(gw, 1.0), src(gh, 1.0), src(gth, 0.0)
+    cx, cy = src(gcx, 0.0), src(gcy, 0.0)
+    jw, jh = rng.uniform(0.9, 1.1, (batch, k)), rng.uniform(0.9, 1.1, (batch, k))
+    w, h, th = w * jw, h * jh, th + rng.normal(0, 0.05, (batch, k))
+    cx, cy = cx + rng.normal(0, 0.1, (batch, k)) * h, cy + rng.normal(0, 0.1, (batch, k)) * h
+    off = h * rng.uniform(1.0, 2.0, (batch, k))
+    cx, cy = np.where(decoy, cx - np.sin(th) * off, cx), np.where(decoy, cy + np.cos(th) * off, cy)
+    rand = ~(copy | decoy)
+    rw = np.exp(rng.uniform(np.log(6.0), np.log(0.2 * size), (batch, k)))
+    w = np.where(rand, rw, w)
+    h = np.where(rand, np.maximum(rw * rng.uniform(0.05, 1.0, (batch, k)), 3.0), h)
+    th = np.where(rand, rng.uniform(-np.pi, np.pi, (batch, k)), th)
+    cx = np.where(rand, rng.uniform(0.1 * size, 0.9 * size, (batch, k)), cx)
+    cy = np.where(rand, rng.uniform(0.1 * size, 0.9 * size, (batch, k)), cy)
+    det_quads = _rect_corners(cx, cy, w, h, th)
+    det_quads = det_quads + rng.normal(0, 0.03, (batch, k, 4, 2)) * h[..., None, None] * copy[..., None, None]
+    keep_cls = copy & (rng.uniform(0, 1, (batch, k)) < 0.9) | decoy
+    det_classes = np.where(keep_cls, src(gt_classes, 0), rng.randint(0, num_classes, (batch, k))).astype(np.int64)
+    det_scores = np.round(rng.uniform(0, 1, (batch, k)), 2).astype(np.float32)
+    return (det_quads.astype(np.float32), det_scores, det_classes, gt_quads.astype(np.float32), gt_classes, offsets)
+
+
 # ----------------------------------------------------------------------------
 # device-side generator for bench.py (torch imported lazily: synth is also used
 # by numpy-only code)
