@@ -601,6 +601,38 @@ SIHL_OD_API int sihl_od_quad_map_match(const float *det_quads, const float *det_
                       int n_areas, int32_t *det_order, int32_t *dt_match, uint8_t *dt_ignore, uint8_t *gt_ignore,
                       void *workspace, size_t workspace_bytes, void *stream);
 
+/* The two matchings above with COCO's optional ground-truth annotations (COCOeval's iscrowd and area; computeIoU's
+ * maskUtils.iou(d, g, iscrowd) and evaluateImg).  Arguments, limits, workspace query, argument checks and outputs are
+ * those of the sibling entry, plus two DEVICE arrays [total_gt], either of which may be NULL (none: all zero):
+ *   gt_crowd uint8  nonzero marks a crowd region ("don't care" in text datasets)
+ *   gt_area  double the annotated area of the gt
+ * Rules:
+ *   1. a gt's area for the range test is gt_area[g] when gt_area[g] > 0; otherwise (<= 0, NaN, NULL) the sibling's
+ *      (box: fp32 w and h multiplied in double; quad: the hull area widened).  Detections always use their own area.
+ *   2. a crowd gt is ignored in every area range: gt_ignore[a, g] = crowd[g] || area outside range a.
+ *   3. the overlap of a detection with a crowd gt is the intersection over the DETECTION's area (IoA): for boxes
+ *      bbIou with u = the detection's w * h in fp64, with the IoU's early-outs; for quads the clamped hull intersection
+ *      over the detection's hull area in fp32, widened, 0 for disjoint AABBs or a zero-area hull.  Non-crowd pairs get
+ *      the sibling's IoU, bit for bit.
+ *   4. a crowd gt is never taken: later detections may match it again at the same threshold.  Everything else in the
+ *      chain is the sibling's (regular gts first, ignored ones only while nothing matched; the later of equal overlaps
+ *      wins; the start min(t, 1 - 1e-10)).
+ *   5. a detection matched to a crowd gt has dt_match = that gt's global index and dt_ignore = 1.
+ * So crowd gts leave the recall denominator through gt_ignore and their detections the precision through dt_ignore.
+ * With both pointers NULL the call computes exactly its sibling's tables.  batch = 0 reads and writes nothing (its empty
+ * arrays may be NULL), for boxes as well.  No host synchronisation: the call can be captured in a CUDA graph.  torchmetrics / pycocotools are absent here: parity UNPINNED. */
+SIHL_OD_API int sihl_od_map_match_crowd(const float *det_boxes, const float *det_scores, const int64_t *det_classes,
+                      int batch, int k, const float *gt_boxes, const int64_t *gt_classes, const int32_t *gt_offsets,
+                      int total_gt, const uint8_t *gt_crowd, const double *gt_area, const double *iou_thresholds_host,
+                      int n_thresholds, const double *area_ranges_host, int n_areas, int32_t *det_order,
+                      int32_t *dt_match, uint8_t *dt_ignore, uint8_t *gt_ignore, void *workspace, void *stream);
+SIHL_OD_API int sihl_od_quad_map_match_crowd(const float *det_quads, const float *det_scores, const int64_t *det_classes,
+                      int batch, int k, const float *gt_quads, const int64_t *gt_classes, const int32_t *gt_offsets,
+                      int total_gt, const uint8_t *gt_crowd, const double *gt_area, const double *iou_thresholds_host,
+                      int n_thresholds, const double *area_ranges_host, int n_areas, int32_t *det_order,
+                      int32_t *dt_match, uint8_t *dt_ignore, uint8_t *gt_ignore, void *workspace,
+                      size_t workspace_bytes, void *stream);
+
 /* ---- N4 (SURVEY.md §8f): the per-location MLP towers in front of the hot path ----------------
  * ref object_detection.py:51-61 builds loc / cls / box / iou heads as torchvision ops.MLP(256 -> [256]*num_layers
  * + [out], norm_layer=LayerNorm, activation_layer=SiLU) and applies them to every location (:116, :121, :175).

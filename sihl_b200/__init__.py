@@ -3,4 +3,4 @@
 top-k decode and (extension) dense decode + class-aware NMS, behind the C ABI of
 ``include/sihl_od.h``.  ``sihl_b200.heads.ObjectDetection`` is the drop-in head."""
 
-__version__ = "0.1.6"
+__version__ = "0.1.7"

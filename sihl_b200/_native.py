@@ -49,6 +49,8 @@ _SIGNATURES = {
     "sihl_od_map_match": (I, [P, P, P, I, I, P, P, P, I, P, I, P, I, P, P, P, P, P, P]),
     "sihl_od_quad_map_workspace_bytes": (C.c_size_t, [I, I, I, I, I]),
     "sihl_od_quad_map_match": (I, [P, P, P, I, I, P, P, P, I, P, I, P, I, P, P, P, P, P, C.c_size_t, P]),
+    "sihl_od_map_match_crowd": (I, [P, P, P, I, I, P, P, P, I, P, P, P, I, P, I, P, P, P, P, P, P]),
+    "sihl_od_quad_map_match_crowd": (I, [P, P, P, I, I, P, P, P, I, P, P, P, I, P, I, P, P, P, P, P, C.c_size_t, P]),
     "sihl_od_topk": (I, [P, I, I64, I, P, P, P]),
     "sihl_od_decode_rows": (I, [P, P, I, I, P, I, P, P, P, I, I, P, P, P, P, P]),
     "sihl_od_topk_t": (I, [P, I, I, I64, I, P, P, P]),

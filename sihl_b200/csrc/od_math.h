@@ -183,11 +183,15 @@ SIHL_HD bool quad_hull_before(const QuadHull &b, const QuadHull &a)
 
 constexpr int kQuadClipMax = 8;     // a convex 4-gon clipped by 4 half-planes has at most 8 vertices
 
-// IoU of two hulls.  Sutherland-Hodgman of the first hull of the canonical pair against the second's edges, about the
-// lower corner of the AABB intersection.  A vertex on an edge's line counts as inside; a crossing point is emitted only
-// for a strict sign change.  Rounding on nearly collinear chains could in principle emit more than kQuadClipMax points:
-// those past the cap are dropped, which keeps the result defined and changes the area by rounding noise only.
-SIHL_HD float quad_iou_hulls(const QuadHull &qa, const QuadHull &qb)
+// Overlap of two hulls: the intersection, clamped to [0, min(area_a, area_b)], over the union (kIoA = false, the IoU) or
+// over qa's area alone (kIoA = true, the IoA: COCOeval's overlap of a detection qa with a crowd region qb).  Both are 0
+// for disjoint AABBs or a zero-area hull.  Sutherland-Hodgman of the first hull of the canonical pair against the
+// second's edges, about the lower corner of the AABB intersection.  A vertex on an edge's line counts as inside; a
+// crossing point is emitted only for a strict sign change.  Rounding on nearly collinear chains could in principle emit
+// more than kQuadClipMax points: those past the cap are dropped, which keeps the result defined and changes the area by
+// rounding noise only.  One body for both forms, so that the intersection they divide is the same bits.
+template <bool kIoA>
+SIHL_HD float quad_overlap_hulls(const QuadHull &qa, const QuadHull &qb)
 {
     const bool swap = quad_hull_before(qb, qa);
     const QuadHull &a = swap ? qb : qa;
@@ -226,9 +230,16 @@ SIHL_HD float quad_iou_hulls(const QuadHull &qa, const QuadHull &qb)
     const float lim = fminf(a.area, b.area);
     float inter = s * 0.5f;
     inter = inter > 0.f ? (inter < lim ? inter : lim) : 0.f;
+    if (kIoA) return inter / qa.area;                       // qa.area > 0 here, and inter <= qa.area
     const float uni = (a.area + b.area) - inter;
     return uni > 0.f ? inter / uni : 0.f;
 }
+
+// IoU of two hulls
+SIHL_HD float quad_iou_hulls(const QuadHull &qa, const QuadHull &qb) { return quad_overlap_hulls<false>(qa, qb); }
+
+// intersection of two hulls over the area of the first
+SIHL_HD float quad_ioa_hulls(const QuadHull &qa, const QuadHull &qb) { return quad_overlap_hulls<true>(qa, qb); }
 
 // quad_iou of two quads given as 8 floats each
 SIHL_HD float quad_iou(const float *a, const float *b) { return quad_iou_hulls(quad_hull(a), quad_hull(b)); }

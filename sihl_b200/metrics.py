@@ -11,6 +11,10 @@ does COCOeval.accumulate / summarize on them — a few cumulative sums per categ
 ``sihl_od_quad_map_match`` (the IoU of the convex hulls of the vertex sets, the hull's polygon area for the area ranges)
 and everything after it is the same.
 
+Targets may carry COCO's optional ``iscrowd`` and ``area`` keys, as torchmetrics and pycocotools read them; the matching
+then runs through the ``_crowd`` entries (crowd regions and text datasets' "don't care" regions are ignored, and so are
+the detections that land on them; an annotated area > 0 places a gt in the small / medium / large ranges).
+
 Parity is UNPINNED: torchmetrics and faster_coco_eval are not installed where this was written; the algorithm is the
 published COCOeval one (see oracle/map_oracle.py, which restates it independently for the tests).
 """
@@ -55,7 +59,9 @@ class DetectionMAP:
     def update(self, preds: List[Dict[str, Tensor]], target: List[Dict[str, Tensor]]) -> None:
         """torchmetrics' signature (ref :230-236): per-image dicts ``scores`` / ``labels`` / ``boxes`` (xyxy px) and
         ``labels`` / ``boxes``.  Every image must carry the same number of detections (``forward`` returns K rows).
-        With ``iou_type="quad"`` both read ``quads`` ([n, 4, 2] or [n, 8] px) in place of ``boxes``."""
+        With ``iou_type="quad"`` both read ``quads`` ([n, 4, 2] or [n, 8] px) in place of ``boxes``.  A target may also
+        carry ``iscrowd`` (bool / integer) and ``area`` ([n] each, one value per ``labels`` entry); a missing key means
+        zeros for that image, i.e. no crowd region and the computed area."""
         if self.iou_type == "quad":
             self._update_quads(preds, target)
             return
@@ -68,7 +74,7 @@ class DetectionMAP:
         gc = [t["labels"].as_subclass(Tensor).reshape(-1).to(device=dev, dtype=torch.int64) for t in target]
         gt_boxes = torch.cat(gb) if gb else torch.empty((0, 4), device=dev)
         gt_classes = torch.cat(gc) if gc else torch.empty((0,), dtype=torch.int64, device=dev)
-        self.update_batch(scores, classes, boxes, gt_boxes, gt_classes, counts)
+        self.update_batch(scores, classes, boxes, gt_boxes, gt_classes, counts, **self._annotations(target, dev))
 
     def _update_quads(self, preds: List[Dict[str, Tensor]], target: List[Dict[str, Tensor]]) -> None:
         scores = torch.stack([p["scores"] for p in preds])
@@ -80,20 +86,44 @@ class DetectionMAP:
         gc = [t["labels"].as_subclass(Tensor).reshape(-1).to(device=dev, dtype=torch.int64) for t in target]
         gt_quads = torch.cat(gq) if gq else torch.empty((0, 8), device=dev)
         gt_classes = torch.cat(gc) if gc else torch.empty((0,), dtype=torch.int64, device=dev)
-        self.update_batch(scores, classes, quads, gt_quads, gt_classes, counts)
+        self.update_batch(scores, classes, quads, gt_quads, gt_classes, counts, **self._annotations(target, dev))
+
+    @staticmethod
+    def _annotations(target: List[Dict[str, Tensor]], dev) -> Dict[str, Optional[Tensor]]:
+        """``gt_crowd`` / ``gt_area`` for :meth:`update_batch` from the targets' optional ``iscrowd`` / ``area``:
+        None where no image has the key, otherwise concatenated with zeros for the images without it."""
+        out: Dict[str, Optional[Tensor]] = {}
+        for key, arg, dtype in (("iscrowd", "gt_crowd", torch.uint8), ("area", "gt_area", torch.float64)):
+            if not any(key in t for t in target):
+                out[arg] = None
+                continue
+            parts = []
+            for i, t in enumerate(target):
+                n = int(t["labels"].numel())
+                if key not in t:
+                    parts.append(torch.zeros(n, dtype=dtype, device=dev))
+                    continue
+                v = t[key].as_subclass(Tensor)
+                if tuple(v.shape) != (n,):
+                    raise ValueError(f"target {i}: {key!r} has shape {tuple(v.shape)}, labels has {n} entries")
+                parts.append((v != 0).to(device=dev, dtype=dtype) if key == "iscrowd" else v.to(device=dev, dtype=dtype))
+            out[arg] = torch.cat(parts) if parts else torch.empty((0,), dtype=dtype, device=dev)
+        return out
 
     def update_batch(self, scores: Tensor, classes: Tensor, boxes: Tensor, gt_boxes: Tensor, gt_classes: Tensor,
-                     gt_counts: Sequence[int]) -> None:
+                     gt_counts: Sequence[int], gt_crowd: Optional[Tensor] = None,
+                     gt_area: Optional[Tensor] = None) -> None:
         """The batched form the drop-in head calls: detections [B,K,...] as ``forward`` returns them, ground truth
         concatenated with its per-image counts.  Enqueues the matching; nothing is synchronised.  With
-        ``iou_type="quad"``, ``boxes`` / ``gt_boxes`` are quads: [B,K,4,2] or [B,K,8] and [sumG,4,2] or [sumG,8]."""
+        ``iou_type="quad"``, ``boxes`` / ``gt_boxes`` are quads: [B,K,4,2] or [B,K,8] and [sumG,4,2] or [sumG,8].
+        ``gt_crowd`` / ``gt_area`` ([sumG], optional) are the ``iscrowd`` / ``area`` annotations (see ``ops.map_match``)."""
         dev = scores.device
         off = np.zeros(len(gt_counts) + 1, dtype=np.int32)
         off[1:] = np.cumsum(gt_counts)
         gt_offsets = torch.from_numpy(off).to(dev)
         match = ops.quad_map_match if self.iou_type == "quad" else ops.map_match
         res = match(boxes.float(), scores, classes, gt_boxes, gt_classes, gt_offsets, self.iou_thresholds,
-                    self.area_ranges)
+                    self.area_ranges, gt_crowd=gt_crowd, gt_area=gt_area)
         order = res["det_order"].long()
         self._batches.append(dict(
             scores=torch.gather(scores.float(), 1, order), classes=torch.gather(classes, 1, order),   # by rank

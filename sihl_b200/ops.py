@@ -901,12 +901,41 @@ COCO_IOU_THRESHOLDS = tuple(0.5 + 0.05 * i for i in range(10))
 COCO_AREA_RANGES = ((0.0, 1e5 ** 2), (0.0, 32.0 ** 2), (32.0 ** 2, 96.0 ** 2), (96.0 ** 2, 1e5 ** 2))    # all, small, medium, large
 
 
+def _gt_annotations(gt_crowd: Optional[Tensor], gt_area: Optional[Tensor], G: int):
+    """COCO's optional per-gt annotations for the ``_crowd`` matching entries: ``gt_crowd`` (bool or integer, nonzero
+    marks a crowd region) -> uint8 0 / 1, ``gt_area`` (any real dtype) -> float64, both ``[G]`` CUDA tensors or None.
+    Shapes and dtypes are checked before anything runs on the device."""
+    for name, t in (("gt_crowd", gt_crowd), ("gt_area", gt_area)):
+        if t is None:
+            continue
+        if not isinstance(t, Tensor):
+            raise TypeError(f"{name}: expected a torch.Tensor or None, got {type(t).__name__}")
+        if tuple(t.shape) != (G,):
+            raise ValueError(f"{name}: expected shape [{G}] (one value per ground truth), got {tuple(t.shape)}")
+        if t.is_complex() or (name == "gt_crowd" and t.is_floating_point()):
+            raise TypeError(f"{name}: expected {'bool or integer' if name == 'gt_crowd' else 'real'} values, got {t.dtype}")
+        if not t.is_cuda:
+            raise RuntimeError(f"{name}: sihl_b200 kernels run on CUDA tensors only (got {t.device}); there is no CPU path")
+    if gt_crowd is not None:
+        gt_crowd = (gt_crowd != 0).to(torch.uint8).contiguous()
+    if gt_area is not None:
+        gt_area = gt_area.to(torch.float64).contiguous()
+    return gt_crowd, gt_area
+
+
 def map_match(det_boxes: Tensor, det_scores: Tensor, det_classes: Tensor, gt_boxes: Tensor, gt_classes: Tensor,
               gt_offsets: Tensor, iou_thresholds: Sequence[float] = COCO_IOU_THRESHOLDS,
-              area_ranges: Sequence[Tuple[float, float]] = COCO_AREA_RANGES) -> Dict[str, Tensor]:
+              area_ranges: Sequence[Tuple[float, float]] = COCO_AREA_RANGES, gt_crowd: Optional[Tensor] = None,
+              gt_area: Optional[Tensor] = None) -> Dict[str, Tensor]:
     """COCOeval.evaluateImg for a whole batch on the GPU (ref object_detection.py:230-237 feeds this to torchmetrics,
     which matches on the CPU at epoch end).  ``det_*`` [B,K,...] as ``forward`` returns them, ground truth in CSR form.
-    Returns dict(det_order i32 [B,K], dt_match i32 [B,NA,T,K], dt_ignore u8 [B,NA,T,K], gt_ignore u8 [NA,sumG])."""
+    Returns dict(det_order i32 [B,K], dt_match i32 [B,NA,T,K], dt_ignore u8 [B,NA,T,K], gt_ignore u8 [NA,sumG]).
+
+    ``gt_crowd`` / ``gt_area`` (``[sumG]`` CUDA tensors, optional) are COCO's ``iscrowd`` and ``area`` annotations
+    (``sihl_od_map_match_crowd``): a crowd gt is ignored in every area range, overlaps a detection by intersection over
+    the detection's area and may be matched by any number of detections, which are then ignored; an area > 0 replaces
+    the box area in the area-range test.  Without either, the tables are those of the plain matching."""
+    crowd, area = _gt_annotations(gt_crowd, gt_area, int(gt_boxes.shape[0]))
     det_boxes = _req(det_boxes, torch.float32, "det_boxes", 3)
     det_scores = _req(det_scores.float() if det_scores.dtype != torch.float32 else det_scores, torch.float32, "det_scores", 2)
     det_classes = _req(det_classes, torch.int64, "det_classes", 2)
@@ -922,12 +951,18 @@ def map_match(det_boxes: Tensor, det_scores: Tensor, det_classes: Tensor, gt_box
         dti = torch.empty((B, NA, T, K), dtype=torch.uint8, device=dev)
         gti = torch.empty((NA, max(G, 1)), dtype=torch.uint8, device=dev)
         ws = torch.empty((int(_lib().sihl_od_map_workspace_bytes(G, T, NA)),), dtype=torch.uint8, device=dev)
-        rc = _lib().sihl_od_map_match(
-            _p(det_boxes), _p(det_scores), _p(det_classes), B, K,
-            _p(_req(gt_boxes, torch.float32, "gt_boxes", 2)) if G else None, _p(_req(gt_classes, torch.int64, "gt_classes", 1)) if G else None,
-            _p(_req(gt_offsets, torch.int32, "gt_offsets", 1)), G, thr.ctypes.data, T, areas.ctypes.data, NA,
-            _p(order), _p(dtm), _p(dti), _p(gti), _p(ws), _stream(dev))
-    _native.check(rc, "sihl_od_map_match")
+        gt = (_p(_req(gt_boxes, torch.float32, "gt_boxes", 2)) if G else None,
+              _p(_req(gt_classes, torch.int64, "gt_classes", 1)) if G else None,
+              _p(_req(gt_offsets, torch.int32, "gt_offsets", 1)), G)
+        rest = (thr.ctypes.data, T, areas.ctypes.data, NA, _p(order), _p(dtm), _p(dti), _p(gti), _p(ws), _stream(dev))
+        if crowd is None and area is None:
+            name = "sihl_od_map_match"
+            rc = _lib().sihl_od_map_match(_p(det_boxes), _p(det_scores), _p(det_classes), B, K, *gt, *rest)
+        else:
+            name = "sihl_od_map_match_crowd"
+            rc = _lib().sihl_od_map_match_crowd(_p(det_boxes), _p(det_scores), _p(det_classes), B, K, *gt,
+                                                _p(crowd) if G else None, _p(area) if G else None, *rest)
+    _native.check(rc, name)
     return dict(det_order=order, dt_match=dtm, dt_ignore=dti, gt_ignore=gti[:, :G])
 
 
@@ -936,11 +971,14 @@ MAP_MAX_K, MAP_MAX_THRESHOLDS, MAP_MAX_AREAS = 1024, 16, 8     # sihl_od_map_mat
 
 def quad_map_match(det_quads: Tensor, det_scores: Tensor, det_classes: Tensor, gt_quads: Tensor, gt_classes: Tensor,
                    gt_offsets: Tensor, iou_thresholds: Sequence[float] = COCO_IOU_THRESHOLDS,
-                   area_ranges: Sequence[Tuple[float, float]] = COCO_AREA_RANGES) -> Dict[str, Tensor]:
+                   area_ranges: Sequence[Tuple[float, float]] = COCO_AREA_RANGES, gt_crowd: Optional[Tensor] = None,
+                   gt_area: Optional[Tensor] = None) -> Dict[str, Tensor]:
     """:func:`map_match` for quadrilaterals: ``det_quads`` ``[B,K,4,2]`` or ``[B,K,8]``, ``gt_quads`` ``[sumG,4,2]`` or
     ``[sumG,8]`` (four points (x, y) in px).  The IoU is :func:`quad_iou`'s (convex hulls of the vertex sets) and the area
     that places a quad in an area range is its hull's polygon area.  Returns the same dict as :func:`map_match`.  Shapes
-    and limits (K <= 1024, at most 16 thresholds and 8 area ranges) are checked before any CUDA call."""
+    and limits (K <= 1024, at most 16 thresholds and 8 area ranges) are checked before any CUDA call.  ``gt_crowd`` /
+    ``gt_area`` as in :func:`map_match` (``sihl_od_quad_map_match_crowd``): a crowd quad ("don't care" region) overlaps
+    a detection by the hulls' intersection over the detection's hull area, and an area > 0 replaces the hull area."""
     if isinstance(det_quads, Tensor) and not (det_quads.dim() == 3 and det_quads.shape[2] == 8) and \
             not (det_quads.dim() == 4 and tuple(det_quads.shape[2:]) == (4, 2)):
         raise ValueError(f"det_quads: expected [B, K, 4, 2] or [B, K, 8], got shape {tuple(det_quads.shape)}")
@@ -958,6 +996,7 @@ def quad_map_match(det_quads: Tensor, det_scores: Tensor, det_classes: Tensor, g
     if not (1 <= T <= MAP_MAX_THRESHOLDS and 1 <= NA <= MAP_MAX_AREAS):
         raise ValueError(f"quad_map_match takes 1 to {MAP_MAX_THRESHOLDS} IoU thresholds and 1 to {MAP_MAX_AREAS} area "
                          f"ranges, got {T} and {NA}")
+    crowd, area = _gt_annotations(gt_crowd, gt_area, int(gt_quads.shape[0]))
     det_quads = _req(det_quads, torch.float32, "det_quads").reshape(B, K, 8)
     det_scores = _req(det_scores.float() if det_scores.dtype != torch.float32 else det_scores, torch.float32, "det_scores", 2)
     det_classes = _req(det_classes, torch.int64, "det_classes", 2)
@@ -976,11 +1015,17 @@ def quad_map_match(det_quads: Tensor, det_scores: Tensor, det_classes: Tensor, g
         dti = torch.empty((B, NA, T, K), dtype=torch.uint8, device=dev)
         gti = torch.empty((NA, max(G, 1)), dtype=torch.uint8, device=dev)
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-        rc = _lib().sihl_od_quad_map_match(
-            _p(det_quads), _p(det_scores), _p(det_classes), B, K, _p(gt_quads) if G else None,
-            _p(gt_classes) if G else None, _p(gt_offsets), G, thr.ctypes.data, T, areas.ctypes.data, NA,
-            _p(order), _p(dtm), _p(dti), _p(gti), _p(ws), ws_bytes, _stream(dev))
-    _native.check(rc, "sihl_od_quad_map_match")
+        gt = (_p(gt_quads) if G else None, _p(gt_classes) if G else None, _p(gt_offsets), G)
+        rest = (thr.ctypes.data, T, areas.ctypes.data, NA, _p(order), _p(dtm), _p(dti), _p(gti), _p(ws), ws_bytes,
+                _stream(dev))
+        if crowd is None and area is None:
+            name = "sihl_od_quad_map_match"
+            rc = _lib().sihl_od_quad_map_match(_p(det_quads), _p(det_scores), _p(det_classes), B, K, *gt, *rest)
+        else:
+            name = "sihl_od_quad_map_match_crowd"
+            rc = _lib().sihl_od_quad_map_match_crowd(_p(det_quads), _p(det_scores), _p(det_classes), B, K, *gt,
+                                                     _p(crowd) if G else None, _p(area) if G else None, *rest)
+    _native.check(rc, name)
     return dict(det_order=order, dt_match=dtm, dt_ignore=dti, gt_ignore=gti[:, :G])
 
 

@@ -237,6 +237,49 @@ def quad_map_batch_np(seed: int, batch: int, k: int, gt_per_image: int, num_clas
     return (det_quads.astype(np.float32), det_scores, det_classes, gt_quads.astype(np.float32), gt_classes, offsets)
 
 
+def map_crowd_batch_np(seed: int, batch: int, k: int, gt_per_image: int, num_classes: int = 80, geometry: str = "box",
+                       size: int = 1024, counts=None, crowd_frac: float = 0.1):
+    """mAP inputs with COCO's ``iscrowd`` / ``area`` annotations for ops.map_match (``geometry="box"``: the AABBs) or
+    ops.quad_map_match (``"quad"``), built on :func:`quad_map_batch_np`.  About ``crowd_frac`` of the gts become crowd
+    ("don't care") regions: large rectangles of 0.2 to 0.45 S a side, each with a cluster of up to 6 small same-class
+    detections inside it.  ``gt_area``: 30% zeros and 5% negative (the computed area is used), 30% the gt's own
+    area scaled by U(0.3, 3), the rest drawn near the 32^2 and 96^2 range boundaries (so gts move between small, medium and
+    large).  Returns det [B,K,4] xyxy or [B,K,4,2], det_scores, det_classes, gt [sumG,4] or [sumG,4,2], gt_classes,
+    gt_offsets, gt_crowd uint8 [sumG], gt_area float64 [sumG]."""
+    if geometry not in ("box", "quad"):
+        raise ValueError(f"geometry must be 'box' or 'quad', got {geometry!r}")
+    dq, ds, dc, gq, gc, go = quad_map_batch_np(seed, batch, k, gt_per_image, num_classes, size, counts)
+    rng = np.random.RandomState(seed + 7919)
+    G = int(go[-1])
+    crowd = (rng.uniform(0, 1, G) < crowd_frac).astype(np.uint8)
+    for g in np.nonzero(crowd)[0]:
+        b = int(np.searchsorted(go, g, side="right") - 1)
+        cw, ch = rng.uniform(0.2, 0.45, 2) * size
+        cx, cy = rng.uniform(0.25 * size, 0.75 * size, 2)
+        th = rng.uniform(-np.pi, np.pi) if geometry == "quad" else 0.0
+        gq[g] = _rect_corners(np.array(cx), np.array(cy), np.array(cw), np.array(ch), np.array(th))
+        rows = rng.choice(k, size=min(6, k), replace=False)
+        u, v = rng.uniform(-0.35, 0.35, (2, len(rows)))
+        px, py = cx + np.cos(th) * u * cw - np.sin(th) * v * ch, cy + np.sin(th) * u * cw + np.cos(th) * v * ch
+        w = rng.uniform(0.05, 0.2, len(rows)) * cw
+        h = w * rng.uniform(0.3, 1.0, len(rows))
+        dq[b, rows] = _rect_corners(px, py, w, h, th + rng.normal(0, 0.05, len(rows)))
+        dc[b, rows] = gc[g]
+    hull = np.abs(np.array([_shoelace(q) for q in gq.reshape(-1, 4, 2)])) if G else np.zeros(0)
+    pick = rng.uniform(0, 1, G)
+    near = np.where(rng.uniform(0, 1, G) < 0.5, 32.0, 96.0) ** 2 * rng.uniform(0.9, 1.1, G)
+    gt_area = np.where(pick < 0.3, 0.0, np.where(pick < 0.35, -1.0, np.where(pick < 0.65, hull * rng.uniform(0.3, 3, G), near)))
+    if geometry == "box":
+        aabb = lambda q: np.concatenate([q.min(-2), q.max(-2)], -1).astype(np.float32)
+        return aabb(dq), ds, dc, aabb(gq), gc, go, crowd, gt_area.astype(np.float64)
+    return dq.astype(np.float32), ds, dc, gq.astype(np.float32), gc, go, crowd, gt_area.astype(np.float64)
+
+
+def _shoelace(q) -> float:
+    x, y = q[:, 0].astype(np.float64), q[:, 1].astype(np.float64)
+    return 0.5 * float(np.dot(x, np.roll(y, -1)) - np.dot(y, np.roll(x, -1)))
+
+
 # ----------------------------------------------------------------------------
 # device-side generator for bench.py (torch imported lazily: synth is also used
 # by numpy-only code)
